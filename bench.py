@@ -10,6 +10,7 @@ sequential s.list=1..20  => one step = one full bessCpp call = 220 PDAS fits (20
   torchrun ... bench.py --gpus N ...                        our arm, N ranks: REPEATED 10-fold CV, one repetition per
                                                             rank (weak scaling, see below)
   python bench.py --impl reference ...                      the reference's own CPU code (oracle/_ref) on host cores
+  python bench.py ... --dump-outputs DIR                    also write the last timed call's results as DIR/*.npy
 
 N > 1.  A single C5 call is 2.3 ms of which only the 0.6 ms screening sweep is p-sized; the 220 fits behind it run on a
 40 MB screened design as ONE resident launch whose length is the per-chain dependency chain, so one call cannot be made
@@ -598,7 +599,25 @@ def run_ours(args):
         }
     if world > 1:
         dist.destroy_process_group()
+    if rank == 0 and args.dump_outputs:
+        dump_outputs(out, args.dump_outputs)
     return line if rank == 0 else None
+
+
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(out, dirname):
+    """Writes what the last timed call returned to its caller -- every array and number of the result, not the run
+    statistics -- as <dirname>/<name>.npy in float64 (the index arrays are exact there).  The inputs are fixed by their
+    seeds, so two builds of the library can be compared output for output."""
+    arrays = {name: np.atleast_1d(np.asarray(v, dtype=np.float64)) for name, v in out.items() if name != "stats" and v is not None}
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_LIMIT_BYTES:
+        raise ValueError(f"--dump-outputs: {total} bytes of outputs exceed the {DUMP_LIMIT_BYTES}-byte limit")
+    os.makedirs(dirname, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(dirname, name + ".npy"), a)
 
 
 class StdoutToStderr:
@@ -629,7 +648,11 @@ def main():
     ap.add_argument("--torch-cv-reduce", action="store_true",
                     help="N > 1: average the CV curves with torch.distributed in the bench instead of inside the library")
     ap.add_argument("--torch-design", action="store_true", help="draw the design with torch.randn instead of the library's generator")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last timed call returned as DIR/<name>.npy (float64)")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
     if args.impl == "reference":
         run_reference(args)
     else:

@@ -6,6 +6,10 @@ import os
 import subprocess
 import sys
 
+import pytest
+
+from oracle import ref
+
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 BASE_KEYS = {"metric", "value", "unit", "n_gpus", "steps", "warmup", "ms_per_step", "higher_is_better", "scaling", "vs_baseline",
@@ -54,6 +58,8 @@ def test_our_bench_lines_multi_gpu_are_weak_scaling_on_unique_fits():
         assert j["e2e"]["h2d_bytes_per_step"] < 8 * 1000 * 500000  # every rank uploads only its column shard
 
 
+@pytest.mark.skipif(not ref.available(), reason="the reference's own library (oracle/_ref, built by oracle/Makefile from the "
+                                               "original project's sources, which are not part of this repository) is not built")
 def test_reference_arm_runs_here_and_keeps_the_contract():
     r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--steps", "1", "--warmup", "0"],
                        capture_output=True, text=True, timeout=600, cwd=ROOT,

@@ -364,17 +364,20 @@ def test_errors_are_loud():
         cbess.fit(x, y, 1, w, True, 1, 1, 20, 2, 1, True, 3, True, 40, [1, 2], 1, 2, False, 1)  # K too large
 
 
-@pytest.mark.skipif(not refso.available(), reason="prebuilt oracle/_ref/libbess_ref.so did not travel")
 def test_config1_against_the_real_reference():
-    """BASELINE config 1 at full size (n=500, p=1000, s.list=1..20, GIC) and its 10-fold-CV variant, against the
-    reference binary itself on the same arrays and the same CV seed."""
+    """BASELINE config 1 at full size (n=500, p=1000, s.list=1..20, GIC) and its 10-fold-CV variant with the folds the
+    library draws itself (CV seed 123), against what the reference returned for the same arrays and the same CV seed
+    (tests/golden/full/c1.npz, c1cv.npz)."""
     from bess_b200 import cbess
     from bess_b200.gen_data import gen_data
     d = gen_data(500, 1000, "gaussian", 10, seed=1)
     w = np.ones(500)
     seq = np.arange(1, 21)
-    for is_cv, ic in [(False, 3), (True, 1)]:
-        r = refso.pywrap_bess(d.x, d.y, 1, w, True, 1, 1, 20, 2, 1, True, ic, is_cv, 10, seq, 1, 20, False, 1, cv_seed=123)
+    for cfg, is_cv, ic in [("c1", False, 3), ("c1cv", True, 1)]:
+        g = load_full_golden(cfg)
+        assert np.array_equal(full_checksum(d), g["checksum"]), "regenerated inputs differ from the ones the golden was made on"
+        r = dict(beta=np.zeros(1000), coef0=float(g["coef0"]), train_loss=float(g["train_loss"]), ic=float(g["ic"]))
+        r["beta"][g["support"]] = g["beta_support"]
         out = cbess.fit(d.x, d.y, 1, w, True, 1, 1, 20, 2, 1, True, ic, is_cv, 10, seq, 1, 20, False, 1, cv_seed=123)
         _check_final(out, r)
 
