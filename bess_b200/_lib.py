@@ -19,13 +19,19 @@ class BessB200Error(RuntimeError):
     pass
 
 
+class Csc(C.Structure):
+    """struct bess_b200_csc (include/bess_b200.h): a sparse design in compressed sparse column form"""
+    _fields_ = [("colptr", C.c_void_p), ("rowidx", C.c_void_p), ("values", C.c_void_p), ("nnz", C.c_longlong)]
+
+
 class Ext(C.Structure):
     """struct bess_b200_ext (include/bess_b200.h)"""
     _fields_ = [("fold_of_row", ip), ("cv_seed", C.c_uint), ("x_on_device", C.c_int), ("device", C.c_int),
                 ("screening_A_out", ip), ("chosen_s_out", ip), ("stats_out", dp), ("profile", C.c_int),
                 ("world", C.c_int), ("rank", C.c_int), ("col_lo", C.c_longlong), ("p_total", C.c_longlong),
                 ("nccl_unique_id", C.c_void_p), ("chosen_lambda_out", dp), ("beta_out_zeroed", C.c_int), ("cv_reduce_over_ranks", C.c_int),
-                ("cv_seed_set", C.c_int), ("tie_exact_out", ip), ("resident_out", dp), ("fold_shard", C.c_int)]
+                ("cv_seed_set", C.c_int), ("tie_exact_out", ip), ("resident_out", dp), ("fold_shard", C.c_int),
+                ("x_csc", C.POINTER(Csc))]
 
 
 _PYWRAP_ARGS = [dp, C.c_int, C.c_int, dp, C.c_int, C.c_int, dp, C.c_int, C.c_bool, C.c_int, C.c_int, C.c_int, C.c_int,
@@ -55,6 +61,8 @@ def load():
     lib.bessgpu_create.argtypes = [C.POINTER(C.c_void_p), C.c_int]
     lib.bessgpu_destroy.argtypes = [C.c_void_p]
     lib.bessgpu_load.argtypes = [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, dp, dp, C.c_int]
+    lib.bessgpu_load_csc.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_longlong, C.c_int,
+                                     dp, dp, C.c_int]
     lib.bessgpu_screen.argtypes = [C.c_void_p, C.c_int, ip, C.c_int, ip]
     lib.bessgpu_screen_local.argtypes = [C.c_void_p, C.c_int, ip, C.c_int, dp, ip, ip]
     lib.bessgpu_gather_columns.argtypes = [C.c_void_p, ip, ip, C.c_int, C.c_void_p, C.c_longlong]

@@ -33,6 +33,60 @@ def _i(a):
     return a.ctypes.data_as(ip)
 
 
+def is_sparse(x):
+    """A scipy.sparse matrix or array (scipy is only imported by the caller that made one)."""
+    return type(x).__module__.startswith("scipy.sparse")
+
+
+def _is_raw_csc(x):
+    """An ``(indptr, indices, data, shape)`` tuple: three arrays (numpy or torch) and a shape tuple.  Nested sequences of
+    numbers stay a dense design."""
+    return (isinstance(x, tuple) and len(x) == 4 and isinstance(x[3], tuple) and len(x[3]) == 2
+            and all(hasattr(a, "ndim") for a in x[:3]))
+
+
+def canonical_csc(x):
+    """A scipy.sparse matrix in any format -> a new CSC matrix with float64 values, int64 indptr, int32 row indices sorted
+    inside every column and duplicates summed (the form bess_b200_csc requires).  The caller's matrix is not modified."""
+    import scipy.sparse as sp
+    if x.ndim != 2:
+        raise ValueError("x must be 2-D")
+    m = sp.csc_matrix(x, dtype=np.float64, copy=True)
+    m.sum_duplicates()
+    m.sort_indices()
+    m.indptr = m.indptr.astype(np.int64, copy=False)
+    m.indices = m.indices.astype(np.int32, copy=False)
+    return m
+
+
+def csc_arrays(x):
+    """The three CSC arrays of a sparse design, passed to the library as (colptr, rowidx, values, nnz, (n, p), on_device,
+    keep-alive).  ``x`` is a scipy.sparse matrix (canonicalised by canonical_csc) or a raw ``(indptr, indices, data, shape)``
+    tuple taken as given -- host arrays (converted to int64 / int32 / float64) or torch CUDA tensors of exactly those
+    dtypes (device-resident, read in place)."""
+    if is_sparse(x):
+        m = canonical_csc(x)
+        arrs, shape = (m.indptr, m.indices, m.data), m.shape
+    else:
+        if not _is_raw_csc(x):
+            raise TypeError("a sparse x is a scipy.sparse matrix or an (indptr, indices, data, shape) tuple")
+        arrs, shape = tuple(x[:3]), tuple(x[3])
+    n, p = int(shape[0]), int(shape[1])
+    if all(getattr(a, "is_cuda", False) for a in arrs):
+        want = ("torch.int64", "torch.int32", "torch.float64")
+        for a, dt in zip(arrs, want):
+            if str(a.dtype) != dt or not a.is_contiguous():
+                raise TypeError(f"device CSC arrays must be contiguous {want} tensors")
+        ptrs = [C.c_void_p(a.data_ptr()) for a in arrs]
+        return ptrs[0], ptrs[1], ptrs[2], int(arrs[2].numel()), (n, p), True, arrs
+    host = (np.ascontiguousarray(arrs[0], dtype=np.int64).ravel(), np.ascontiguousarray(arrs[1], dtype=np.int32).ravel(),
+            np.ascontiguousarray(arrs[2], dtype=np.float64).ravel())
+    if host[0].size != p + 1 or host[1].size != host[2].size:
+        raise ValueError("CSC arrays: indptr needs p + 1 entries and indices / data the same length")
+    ptrs = [a.ctypes.data_as(C.c_void_p) for a in host]
+    return ptrs[0], ptrs[1], ptrs[2], int(host[2].size), (n, p), False, host
+
+
 def _prep(x, y, weight, g_index, state, sequence, lambda_sequence, always_select):
     x = np.ascontiguousarray(x, dtype=np.float64)
     if x.ndim != 2:
@@ -84,6 +138,9 @@ def fit(x, y, data_type, weight, is_normal, algorithm_type, model_type, max_iter
         n_lambda=None, powell_path=1, want_curve=False, g_index=None, cv_reduce_over_ranks=False, fold_shard=False):
     """``bess_b200_fit``: pywrap_bess + status code + extensions.  Returns a dict.
     ``x`` is a host ndarray, or pass ``x_device_ptr`` (int, row-major n x p fp64 in HBM) with ``n``/``p``.
+    A sparse ``x`` -- a scipy.sparse matrix in any format, or a raw ``(indptr, indices, data, shape)`` tuple of host arrays
+    or of torch CUDA tensors (device-resident) -- goes to the library as a CSC design (``bess_b200_csc``); see
+    ``csc_arrays``.
     ``world > 1``: column-sharded multi-GPU call -- ``x`` is this rank's column shard ``[col_lo, col_lo + p)`` of a
     ``p_total``-column design, ``nccl_id`` the job's 128-byte NCCL unique id (``bess_b200.dist.nccl_unique_id``); beta
     and always_select use global column numbers.
@@ -91,7 +148,12 @@ def fit(x, y, data_type, weight, is_normal, algorithm_type, model_type, max_iter
     ``[s_min, s_max] x [lambda_min, lambda_max]`` (pgs_path, path.cpp:1138); ``powell_path`` 1 = golden-section line
     searches, 2 = walks on an ``n_lambda``-point log grid."""
     lib = _lib.load()
-    if x_device_ptr is None:
+    csc = None
+    if is_sparse(x) or _is_raw_csc(x):
+        cp, ri, cv, nnz, (n, p), csc_on_device, _csc_arrays_alive = csc_arrays(x)
+        csc = _lib.Csc(cp, ri, cv, nnz)
+        xptr = None if x_device_ptr is None else C.cast(C.c_void_p(int(x_device_ptr)), dp)  # both: the library refuses
+    elif x_device_ptr is None:
         x = np.ascontiguousarray(x, dtype=np.float64)
         n, p = x.shape
         xptr = _d(x)
@@ -132,6 +194,9 @@ def fit(x, y, data_type, weight, is_normal, algorithm_type, model_type, max_iter
     ext.cv_seed = int(cv_seed) if cv_seed is not None else 0  # None: $BESS_CV_SEED or 123
     ext.cv_seed_set = 1 if cv_seed is not None else 0
     ext.x_on_device = 1 if x_device_ptr is not None else 0
+    if csc is not None:
+        ext.x_csc = C.pointer(csc)
+        ext.x_on_device = 1 if csc_on_device else 0
     ext.device = int(device)
     scrA = np.zeros(max(int(screening_size), 1), dtype=np.int32)
     ext.screening_A_out = _i(scrA)

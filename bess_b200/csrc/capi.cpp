@@ -88,6 +88,13 @@ int bess_b200_fit_impl(double *x, int x_row, int x_col, double *y, int y_len, in
             a.x_on_device = ext->x_on_device != 0;
             a.device = ext->device;
             a.profile = ext->profile != 0;
+            if (ext->x_csc) {
+                a.csc = true;
+                a.csc_colptr = ext->x_csc->colptr;
+                a.csc_rowidx = ext->x_csc->rowidx;
+                a.csc_values = ext->x_csc->values;
+                a.csc_nnz = ext->x_csc->nnz;
+            }
             if (shard) {
                 a.world = ext->world;
                 a.rank = ext->rank;
@@ -327,6 +334,11 @@ int bessgpu_load(bessgpu_handle *h, const double *x, int n, int p, int x_on_devi
                  const double *weight, int model_type)
 {
     return guarded([&] { h->eng->load(x, n, p, x_on_device != 0, y, weight, model_type); });
+}
+int bessgpu_load_csc(bessgpu_handle *h, const long long *colptr, const int *rowidx, const double *values, int n, int p,
+                     long long nnz, int on_device, const double *y, const double *weight, int model_type)
+{
+    return guarded([&] { h->eng->load_csc(colptr, rowidx, values, n, p, nnz, on_device != 0, y, weight, model_type); });
 }
 int bessgpu_screen(bessgpu_handle *h, int size, const int *always, int n_always, int *out)
 {

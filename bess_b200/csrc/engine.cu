@@ -14,6 +14,7 @@
 #include <mutex>
 #include <numeric>
 #include <thread>
+#include <utility>
 
 namespace bess {
 
@@ -340,6 +341,23 @@ struct Engine::Impl {
     // design
     double *X = nullptr;
     long long ldx = 0;
+    // sparse design (Engine::load_csc) until screening or densify() makes it dense; csc_owned: the arrays are ours
+    bool csc = false, csc_owned = false;
+    long long *cp = nullptr;
+    int *ri = nullptr;
+    double *cv = nullptr;
+    long long nnz = 0;
+    void free_csc()
+    {
+        if (csc_owned) {
+            dfree(st, cp);
+            dfree(st, ri);
+            dfree(st, cv);
+        }
+        cp = nullptr; ri = nullptr; cv = nullptr;
+        csc = csc_owned = false;
+        nnz = 0;
+    }
     int n = 0, p = 0, npad = 0;
     double *y = nullptr, *w = nullptr;  // [npad] device
     std::vector<double> hy, hw;          // host copies (current, i.e. after normalisation)
@@ -612,6 +630,7 @@ Engine::~Engine()
     m.free_chain_buffers();
     m.free_sweep_buffers();
     if (m.x_owned) dfree(m.st, m.X);
+    m.free_csc();
     dfree(m.st, m.gidx); dfree(m.st, m.gsz); dfree(m.st, m.glist);
     cudaStreamSynchronize(m.st);
     m.ctx->ar.reset();
@@ -717,12 +736,11 @@ void Engine::profile(double *ms_out, long long *n_out) const
 // own pageable path stages through one thread's memcpy (measured 11 GB/s: 183 of the 357 ms of a config-3 call).  Here a
 // few host threads fill a two-buffer pinned ring in parallel while the previous buffer's DMA runs: the copy approaches
 // the PCIe rate of a pinned source.  Row chunks keep the 2-D pitch conversion (p -> ldx columns) inside the DMA.
-static void upload_pageable(DeviceContext *c, cudaStream_t st, double *dX, size_t ldx, const double *x, int n, int p)
+// The ring itself: chunk(k) gives the host bytes of chunk k (at most buf_bytes), dma(k, stage, bytes) enqueues the copy of
+// the staged chunk.
+template <class Chunk, class Dma>
+static void staged_upload(DeviceContext *c, cudaStream_t st, size_t buf_bytes, int nchunks, Chunk chunk, Dma dma)
 {
-    const size_t row_bytes = (size_t)p * 8;
-    const size_t buf_bytes = std::max<size_t>((size_t)32 << 20, row_bytes);
-    const size_t rows_per = std::max<size_t>(1, buf_bytes / row_bytes);
-    const int nchunks = (int)(((size_t)n + rows_per - 1) / rows_per);
     c->reserve_stage(buf_bytes);
     static const int T = [] {
         const char *e = std::getenv("BESS_B200_UPLOAD_THREADS");
@@ -735,10 +753,9 @@ static void upload_pageable(DeviceContext *c, cudaStream_t st, double *dX, size_
     auto worker = [&](int t) {
         for (int k = 0; k < nchunks; k++) {
             while (go.load(std::memory_order_acquire) < k) std::this_thread::yield();
-            const size_t r0 = (size_t)k * rows_per, rows = std::min(rows_per, (size_t)n - r0);
-            const size_t bytes = rows * row_bytes;
-            const size_t b0 = bytes * (size_t)t / (size_t)T, b1 = bytes * (size_t)(t + 1) / (size_t)T;
-            std::memcpy(c->h_stage[k & 1] + b0, reinterpret_cast<const char *>(x) + r0 * row_bytes + b0, b1 - b0);
+            const std::pair<const char *, size_t> ck = chunk(k);
+            const size_t b0 = ck.second * (size_t)t / (size_t)T, b1 = ck.second * (size_t)(t + 1) / (size_t)T;
+            std::memcpy(c->h_stage[k & 1] + b0, ck.first + b0, b1 - b0);
             done.fetch_add(1, std::memory_order_release);
         }
     };
@@ -748,16 +765,11 @@ static void upload_pageable(DeviceContext *c, cudaStream_t st, double *dX, size_
         for (int k = 0; k < nchunks; k++) {
             if (k >= 2) CUDA_CHECK(cudaEventSynchronize(c->ev_stage[k & 1]));  // the DMA that read this buffer last
             go.store(k, std::memory_order_release);
-            {   // the calling thread is worker 0
-                const size_t r0 = (size_t)k * rows_per, rows = std::min(rows_per, (size_t)n - r0);
-                const size_t bytes = rows * row_bytes;
-                std::memcpy(c->h_stage[k & 1], reinterpret_cast<const char *>(x) + r0 * row_bytes, bytes / (size_t)T);
-                done.fetch_add(1, std::memory_order_release);
-            }
+            const std::pair<const char *, size_t> ck = chunk(k);
+            std::memcpy(c->h_stage[k & 1], ck.first, ck.second / (size_t)T);  // the calling thread is worker 0
+            done.fetch_add(1, std::memory_order_release);
             while (done.load(std::memory_order_acquire) < (long long)T * (k + 1)) std::this_thread::yield();
-            const size_t r0 = (size_t)k * rows_per, rows = std::min(rows_per, (size_t)n - r0);
-            CUDA_CHECK(cudaMemcpy2DAsync(dX + r0 * ldx, ldx * 8, c->h_stage[k & 1], row_bytes, row_bytes, rows,
-                                         cudaMemcpyHostToDevice, st));
+            dma(k, c->h_stage[k & 1], ck.second);
             CUDA_CHECK(cudaEventRecord(c->ev_stage[k & 1], st));
         }
     } catch (...) {
@@ -772,29 +784,57 @@ static void upload_pageable(DeviceContext *c, cudaStream_t st, double *dX, size_
     if (nchunks > 1) CUDA_CHECK(cudaEventSynchronize(c->ev_stage[(nchunks - 2) & 1]));
 }
 
+static void upload_pageable(DeviceContext *c, cudaStream_t st, double *dX, size_t ldx, const double *x, int n, int p)
+{
+    const size_t row_bytes = (size_t)p * 8;
+    const size_t buf_bytes = std::max<size_t>((size_t)32 << 20, row_bytes);
+    const size_t rows_per = std::max<size_t>(1, buf_bytes / row_bytes);
+    const int nchunks = (int)(((size_t)n + rows_per - 1) / rows_per);
+    auto chunk = [&](int k) {
+        const size_t r0 = (size_t)k * rows_per, rows = std::min(rows_per, (size_t)n - r0);
+        return std::make_pair(reinterpret_cast<const char *>(x) + r0 * row_bytes, rows * row_bytes);
+    };
+    auto dma = [&](int k, const char *stage, size_t bytes) {
+        const size_t r0 = (size_t)k * rows_per;
+        CUDA_CHECK(cudaMemcpy2DAsync(dX + r0 * ldx, ldx * 8, stage, row_bytes, row_bytes, bytes / row_bytes,
+                                     cudaMemcpyHostToDevice, st));
+    };
+    staged_upload(c, st, buf_bytes, nchunks, chunk, dma);
+}
+
+// Host -> device copy of a 1-D host array (the CSC arrays of load_csc): pageable memory of 64 MB or more goes through the
+// same ring in 32 MB chunks, pinned memory (and small arrays) with one direct copy.
+static void upload_1d(DeviceContext *c, cudaStream_t st, void *dst, const void *src, size_t bytes)
+{
+    if (bytes == 0) return;
+    bool pageable = false;
+    if (bytes >= ((size_t)64 << 20)) {
+        cudaPointerAttributes pa;
+        const cudaError_t e = cudaPointerGetAttributes(&pa, src);
+        if (e != cudaSuccess) cudaGetLastError();
+        pageable = e != cudaSuccess || pa.type == cudaMemoryTypeUnregistered;
+    }
+    if (!pageable) {
+        CUDA_CHECK(cudaMemcpyAsync(dst, src, bytes, cudaMemcpyHostToDevice, st));
+        return;
+    }
+    const size_t buf_bytes = (size_t)32 << 20;
+    const int nchunks = (int)((bytes + buf_bytes - 1) / buf_bytes);
+    auto chunk = [&](int k) {
+        const size_t b0 = (size_t)k * buf_bytes;
+        return std::make_pair(reinterpret_cast<const char *>(src) + b0, std::min(buf_bytes, bytes - b0));
+    };
+    auto dma = [&](int k, const char *stage, size_t nb) {
+        CUDA_CHECK(cudaMemcpyAsync(reinterpret_cast<char *>(dst) + (size_t)k * buf_bytes, stage, nb, cudaMemcpyHostToDevice, st));
+    };
+    staged_upload(c, st, buf_bytes, nchunks, chunk, dma);
+}
+
 void Engine::load(const double *x, int n, int p, bool x_on_device, const double *y, const double *weight, int family,
                   bool borrow)
 {
     Impl &m = *d_;
-    if (n < 2 || p < 1) throw EngineError{"load: need n >= 2 and p >= 1"};
-    if (family < 1 || family > 4) throw EngineError{"load: model_type must be 1..4"};
-    if (sharded_) {
-        long long lo, hi;
-        shard_range(p_total_, world_, rank_, &lo, &hi);
-        if (hi - lo != p) throw EngineError{"load: the shard must hold exactly the columns of bess_b200_shard_range"};
-    }
-    m.free_chain_buffers();
-    m.free_sweep_buffers();
-    if (m.x_owned) dfree(m.st, m.X);
-    // a new problem: every arena block of the previous one is dead once the stream has drained
-    CUDA_CHECK(cudaStreamSynchronize(m.st));
-    m.ctx->ar.reset();
-    m.ctx->mir.reset();
-    m.ctx->rb.reset();
-    m.sel_pending = m.stats_pending = false;
-    n_ = n; p_ = p; family_ = family;
-    m.n = n; m.p = p; m.npad = (n + 1) & ~1;
-    m.ldx = (p + 1) & ~1LL;
+    begin_load(n, p, family);
     // A device-resident design with an even column count can be used in place while it is only READ (screening
     // replaces it by the gathered columns); normalize() takes a private copy otherwise.
     if (borrow && x_on_device && (p % 2 == 0) && ((uintptr_t)x % 16 == 0)) {
@@ -819,6 +859,42 @@ void Engine::load(const double *x, int n, int p, bool x_on_device, const double 
                                          x_on_device ? cudaMemcpyDeviceToDevice : cudaMemcpyHostToDevice, m.st));
         m.span_end(sp);
     }
+    end_load(y, weight, family);
+}
+
+// what every load shares: the previous problem's buffers go, the shapes are set
+void Engine::begin_load(int n, int p, int family)
+{
+    Impl &m = *d_;
+    if (n < 2 || p < 1) throw EngineError{"load: need n >= 2 and p >= 1"};
+    if (family < 1 || family > 4) throw EngineError{"load: model_type must be 1..4"};
+    if (sharded_) {
+        long long lo, hi;
+        shard_range(p_total_, world_, rank_, &lo, &hi);
+        if (hi - lo != p) throw EngineError{"load: the shard must hold exactly the columns of bess_b200_shard_range"};
+    }
+    m.free_chain_buffers();
+    m.free_sweep_buffers();
+    if (m.x_owned) dfree(m.st, m.X);
+    m.free_csc();
+    m.X = nullptr;
+    m.x_owned = true;
+    // a new problem: every arena block of the previous one is dead once the stream has drained
+    CUDA_CHECK(cudaStreamSynchronize(m.st));
+    m.ctx->ar.reset();
+    m.ctx->mir.reset();
+    m.ctx->rb.reset();
+    m.sel_pending = m.stats_pending = false;
+    n_ = n; p_ = p; family_ = family;
+    m.n = n; m.p = p; m.npad = (n + 1) & ~1;
+    m.ldx = (p + 1) & ~1LL;
+}
+
+// the response and weights, and the kernel descriptor of the new problem
+void Engine::end_load(const double *y, const double *weight, int family)
+{
+    Impl &m = *d_;
+    const int n = m.n;
     m.hy.assign(y, y + n);
     m.hw.assign(weight, weight + n);
     m.y = m.stage_vec(y, (size_t)n, (size_t)m.npad);
@@ -834,6 +910,87 @@ void Engine::load(const double *x, int n, int p, bool x_on_device, const double 
     h_xmean_.clear();
     h_xnorm_.clear();
     y_mean_ = 0.0;
+}
+
+void Engine::load_csc(const long long *colptr, const int *rowidx, const double *values, int n, int p, long long nnz,
+                      bool on_device, const double *y, const double *weight, int family)
+{
+    Impl &m = *d_;
+    if (n < 2 || p < 1) throw EngineError{"load_csc: need n >= 2 and p >= 1"};
+    if (family < 1 || family > 4) throw EngineError{"load_csc: model_type must be 1..4"};
+    if (sharded_) throw EngineError{"load_csc: a sparse design is single-GPU only"};
+    if (nnz < 0 || !colptr || (nnz > 0 && (!rowidx || !values))) throw EngineError{"x_csc: colptr, rowidx and values must be given"};
+    if (!on_device) {  // O(p) on the host; device arrays are checked by csc_check_kernel
+        if (colptr[0] != 0) throw EngineError{"x_csc: colptr[0] must be 0"};
+        for (long long j = 0; j < p; j++)
+            if (colptr[j + 1] < colptr[j])
+                throw EngineError{"x_csc: colptr must be non-decreasing (colptr[" + std::to_string(j + 1) + "] < colptr[" +
+                                  std::to_string(j) + "])"};
+        if (colptr[p] != nnz) throw EngineError{"x_csc: colptr[p] must equal nnz"};
+    }
+    begin_load(n, p, family);
+    const int sp = m.span_begin(7);
+    if (on_device) {  // only ever read: used in place
+        m.cp = const_cast<long long *>(colptr);
+        m.ri = const_cast<int *>(rowidx);
+        m.cv = const_cast<double *>(values);
+        m.csc_owned = false;
+    } else {
+        m.csc_owned = true;
+        m.cp = dalloc<long long>(m.st, (size_t)p + 1);
+        m.ri = dalloc<int>(m.st, (size_t)nnz);
+        m.cv = dalloc<double>(m.st, (size_t)nnz);
+        upload_1d(m.ctx, m.st, m.cp, colptr, ((size_t)p + 1) * 8);
+        upload_1d(m.ctx, m.st, m.ri, rowidx, (size_t)nnz * 4);
+        upload_1d(m.ctx, m.st, m.cv, values, (size_t)nnz * 8);
+    }
+    m.span_end(sp);
+    m.csc = true;
+    m.nnz = nnz;
+    end_load(y, weight, family);
+    int *h_flag = m.ctx->rb.alloc<int>(1);
+    int *d_flag = m.ctx->ar.alloc<int>(1);
+    CUDA_CHECK(cudaMemsetAsync(d_flag, 0, 4, m.st));
+    launch_csc_check(m.cp, m.ri, n, p, nnz, d_flag, m.st);
+    CUDA_CHECK(cudaMemcpyAsync(h_flag, d_flag, 4, cudaMemcpyDeviceToHost, m.st));
+    CUDA_CHECK(cudaStreamSynchronize(m.st));
+    stats_.kernel_launches += 1;
+    m.mk_load = m.ctx->ar.mark();
+    const int bad = *h_flag;
+    if (bad) {
+        m.free_csc();
+        std::string why;
+        if (bad & CSC_BAD_COLPTR) why += " colptr must start at 0, be non-decreasing and end at nnz;";
+        if (bad & CSC_BAD_ROW) why += " a row index is outside [0, n);";
+        if (bad & CSC_UNSORTED) why += " row indices must be strictly increasing inside every column (unsorted or duplicate);";
+        why.pop_back();
+        throw EngineError{"x_csc:" + why};
+    }
+}
+
+bool Engine::sparse() const { return d_->csc; }
+
+void Engine::densify()
+{
+    Impl &m = *d_;
+    if (!m.csc) return;
+    const long long ldx = ((long long)m.p + 1) & ~1LL;
+    const size_t bytes = (size_t)m.n * (size_t)ldx * 8;
+    size_t free_b = 0, total_b = 0;
+    CUDA_CHECK(cudaMemGetInfo(&free_b, &total_b));
+    if (bytes > free_b)
+        throw EngineError{"sparse design without screening: its dense form (" + std::to_string(bytes >> 20) + " MB) does not fit "
+                          "the device (" + std::to_string(free_b >> 20) + " MB free); screen it (is_screening) instead"};
+    double *X = dalloc<double>(m.st, (size_t)m.n * ldx);
+    CUDA_CHECK(cudaMemsetAsync(X, 0, bytes, m.st));
+    const int sp = m.span_begin(5);
+    launch_csc_densify(m.cp, m.ri, m.cv, nullptr, m.p, X, ldx, m.st);
+    m.span_end(sp);
+    stats_.kernel_launches += 1;
+    m.free_csc();  // stream-ordered: the arrays live until the densify kernel is done
+    m.X = X;
+    m.x_owned = true;
+    m.ldx = ldx;
 }
 
 static int *screen_select(Engine::Impl &m, EngineStats &st, int family, int size, const std::vector<int> &always_select,
@@ -864,7 +1021,7 @@ void Engine::screen_enqueue(int size, const std::vector<int> &always_select)
     if (size < 1 || size > p_model()) throw EngineError{"screening_size must be in [1, p]"};
     const long long ldn = (size + 1) & ~1LL;
     double *Xn = dalloc<double>(m.st, (size_t)m.n * ldn);
-    if (ldn != size) CUDA_CHECK(cudaMemsetAsync(Xn, 0, (size_t)m.n * ldn * 8, m.st));
+    if (ldn != size || m.csc) CUDA_CHECK(cudaMemsetAsync(Xn, 0, (size_t)m.n * ldn * 8, m.st));
     m.h_sel = m.ctx->rb.alloc<int>((size_t)size);
     m.h_sel_tie = m.ctx->rb.alloc<int>(1);
     *m.h_sel_tie = 0;
@@ -873,7 +1030,8 @@ void Engine::screen_enqueue(int size, const std::vector<int> &always_select)
         const int *d_sel = screen_select(m, stats_, family_, size, always_select, nullptr, nullptr, /*to_pinned=*/true);
         // X <- X[:, sel]  (screening.cpp:83-88)
         const int spk = m.span_begin(5);
-        launch_gather_cols(m.X, m.ldx, m.n, d_sel, size, Xn, ldn, m.st);
+        if (m.csc) launch_csc_densify(m.cp, m.ri, m.cv, d_sel, size, Xn, ldn, m.st);
+        else launch_gather_cols(m.X, m.ldx, m.n, d_sel, size, Xn, ldn, m.st);
         m.span_end(spk);
         stats_.kernel_launches += 1;
         m.sel_pending = true;  // the index list and the tie flag are on their way to the pinned block
@@ -914,6 +1072,7 @@ void Engine::screen_enqueue(int size, const std::vector<int> &always_select)
         col_lo_ = 0;
     }
     if (m.x_owned) dfree(m.st, m.X);  // stream-ordered: the gather above has the old design until it is done
+    m.free_csc();
     m.x_owned = true;
     m.X = Xn;
     m.ldx = ldn;
@@ -941,6 +1100,7 @@ void Engine::screen_local(int size, const std::vector<int> &always_select, std::
 void Engine::gather_columns(const int *cols, const int *pos, int mcols, double *dst_dev, long long ld)
 {
     Impl &m = *d_;
+    if (m.csc) throw EngineError{"gather_columns: the design is sparse"};
     if (mcols <= 0) return;
     int *d_cols = dalloc<int>(m.st, mcols), *d_pos = dalloc<int>(m.st, mcols);
     CUDA_CHECK(cudaMemcpyAsync(d_cols, cols, (size_t)mcols * 4, cudaMemcpyHostToDevice, m.st));
@@ -965,7 +1125,16 @@ static int *screen_select(Engine::Impl &m, EngineStats &stats_, int family_, int
     BatchDesc b{};
     b.nch = 1;
     b.chain[0] = 0;
-    if (family_ == FAM_LM) {
+    if (m.csc) {
+        // the same utilities over the stored entries of a sparse design; algorithmic bytes: the three CSC arrays and the
+        // n-vectors the kernel reads (y; y and w for the GLM families)
+        const int sp = m.span_begin(0);
+        if (family_ == FAM_LM) launch_screen_csc_lm(m.cp, m.ri, m.cv, m.p, m.nnz, m.y, m.d.bd, m.st);
+        else launch_screen_glm_csc(m.cp, m.ri, m.cv, m.n, m.p, m.y, m.w, family_, m.d.bd, m.st);
+        m.span_end(sp);
+        stats_.big_sweep_bytes += 12.0 * (double)m.nnz + 8.0 * ((double)m.p + 1) + (family_ == FAM_LM ? 8.0 : 16.0) * m.n;
+        stats_.kernel_launches += 1;
+    } else if (family_ == FAM_LM) {
         // one-column least squares on RAW x (screening.cpp:46): (x_j.y / x_j.x_j)^2
         std::vector<double> ones(m.n, 1.0);
         m.put_vec(m.d.G, 0, m.hy);
@@ -1042,6 +1211,7 @@ static int *screen_select(Engine::Impl &m, EngineStats &stats_, int family_, int
 void Engine::normalize(int data_type, bool is_normal)
 {
     Impl &m = *d_;
+    if (m.csc) throw EngineError{"normalize: a sparse design must be screened or densified first"};
     const int n = m.n, p = m.p;
     if (!m.x_owned) {  // normalisation is in place: take a private copy of a borrowed design
         double *Xc = dalloc<double>(m.st, (size_t)n * m.ldx);

@@ -102,6 +102,14 @@ public:
     // borrow: a device-resident x may be used in place (no copy) until something needs to write to it.
     void load(const double *x, int n, int p, bool x_on_device, const double *y, const double *weight, int family,
               bool borrow = false);
+    // ---- sparse design in CSC form (include/bess_b200.h, bess_b200_csc): the three arrays are copied to the device
+    // (device arrays are read in place) and checked; a malformed input throws.  The design stays sparse until screening
+    // keeps its columns (screen / screen_enqueue densify them) or densify() expands all of it; screen_local reads it as is.
+    void load_csc(const long long *colptr, const int *rowidx, const double *values, int n, int p, long long nnz,
+                  bool on_device, const double *y, const double *weight, int family);
+    // the whole CSC design -> the dense row-major n x ldx design a load() of the same matrix holds
+    void densify();
+    bool sparse() const;
     // per-category device time (CUDA events on the engine's stream): 0 screening sweep (the pass over the raw design),
     // 1 PDAS dual sweeps, 2 finish, 3 top-k, 4 chain kernels, 5 other, 6 normalisation / x_j.x_j passes, 7 host->device upload
     void set_profiling(bool on);
@@ -194,6 +202,8 @@ public:
 
     struct Impl;
 private:
+    void begin_load(int n, int p, int family);
+    void end_load(const double *y, const double *weight, int family);
     Impl *d_ = nullptr;
     int n_ = 0, p_ = 0, family_ = 0;
     int S_ = 1;

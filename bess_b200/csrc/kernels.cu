@@ -18,6 +18,7 @@
 #include "kernels.cuh"
 #include "device_utils.cuh"
 
+#include <algorithm>
 #include <cfloat>
 #include <cmath>
 #include <cstdio>
@@ -1087,9 +1088,61 @@ __device__ __forceinline__ void solve2(double a, double b, double c, double r0, 
     x1 = (a * r1 - b * r0) / det;
 }
 
-__global__ void __launch_bounds__(128) screen_glm_kernel(const double *__restrict__ X, long long ldx, int n, int p,
-                                                         const double *__restrict__ y, const double *__restrict__ w,
-                                                         int family, double *util)
+// Column readers of screen_glm_kernel.  start(rev) begins a pass over the rows (ascending, or descending when rev); at(i)
+// then returns x[i][j] for the rows of that pass in order.  The dense reader is the strided load of a row-major design;
+// the CSC reader walks the column's stored entries with a cursor and returns 0.0 for absent rows, so both feed the same
+// arithmetic the same values in the same order.
+struct DenseColumn {
+    const double *__restrict__ xc;
+    long long ldx;
+    static __device__ __forceinline__ DenseColumn make(const double *X, long long ldx, const long long *, const int *, int j)
+    {
+        return DenseColumn{X + j, ldx};
+    }
+    __device__ __forceinline__ void start(bool) {}
+    __device__ __forceinline__ double at(int i) { return __ldg(xc + (size_t)i * ldx); }
+};
+struct CscColumn {
+    const int *ri;
+    const double *v;
+    long long b, e, k;
+    int next;  // row of entry k, -1 once the pass has used every entry
+    int step;
+    // values = the CSC value array (passed where the dense reader takes X)
+    static __device__ __forceinline__ CscColumn make(const double *values, long long, const long long *colptr,
+                                                     const int *rowidx, int j)
+    {
+        CscColumn c;
+        c.ri = rowidx;
+        c.v = values;
+        c.b = __ldg(colptr + j);
+        c.e = __ldg(colptr + j + 1);
+        c.k = c.b;
+        c.next = -1;
+        c.step = 1;
+        return c;
+    }
+    __device__ __forceinline__ void start(bool rev)
+    {
+        step = rev ? -1 : 1;
+        k = rev ? e - 1 : b;
+        next = (k >= b && k < e) ? __ldg(ri + k) : -1;
+    }
+    __device__ __forceinline__ double at(int i)
+    {
+        if (i != next) return 0.0;
+        const double x = __ldg(v + k);
+        k += step;
+        next = (k >= b && k < e) ? __ldg(ri + k) : -1;
+        return x;
+    }
+};
+
+template <class Column>
+__global__ void __launch_bounds__(128) screen_glm_kernel(const double *__restrict__ X, long long ldx,
+                                                         const long long *__restrict__ colptr, const int *__restrict__ rowidx,
+                                                         int n, int p, const double *__restrict__ y,
+                                                         const double *__restrict__ w, int family, double *util)
 {
     extern __shared__ __align__(128) unsigned char smem_raw[];
     double *ys = reinterpret_cast<double *>(smem_raw);
@@ -1101,14 +1154,15 @@ __global__ void __launch_bounds__(128) screen_glm_kernel(const double *__restric
     __syncthreads();
     const int j = blockIdx.x * blockDim.x + threadIdx.x;
     if (j >= p) return;
-    const double *xc = X + j;
+    Column xc = Column::make(X, ldx, colptr, rowidx, j);
     if (family == FAM_LOGIT) {
         double b00 = 0.0, b01 = 0.0;  // beta0
         double b10, b11;              // beta1
         // step 0 at beta0 = 0: Pi = 0.5
         double ll0 = 0.0, s00 = 0, s01 = 0, s11 = 0, r0 = 0, r1 = 0;
+        xc.start(false);
         for (int i = 0; i < n; i++) {
-            const double x = __ldg(xc + (size_t)i * ldx);
+            const double x = xc.at(i);
             const double pi = 0.5;
             ll0 += (ys[i] * log(pi) + (1.0 - ys[i]) * log(1.0 - pi)) * ws[i];
             const double W = pi * (1.0 - pi);
@@ -1120,8 +1174,9 @@ __global__ void __launch_bounds__(128) screen_glm_kernel(const double *__restric
         for (int it = 0; it < 30; it++) {
             double ll1 = 0.0;
             s00 = s01 = s11 = r0 = r1 = 0.0;
+            xc.start(false);
             for (int i = 0; i < n; i++) {
-                const double x = __ldg(xc + (size_t)i * ldx);
+                const double x = xc.at(i);
                 const double eu = b10 + b11 * x;
                 const double e = exp(clampd(eu, 30.0));
                 const double pi = e / (1.0 + e);
@@ -1141,8 +1196,9 @@ __global__ void __launch_bounds__(128) screen_glm_kernel(const double *__restric
         double b0 = 0.0, b1 = 0.0;
         for (int it = 0; it < 100; it++) {
             double g0 = 0, g1 = 0, h00 = 0, h01 = 0, h11 = 0, ll0 = 0, ew0 = 0;
+            xc.start(false);
             for (int i = 0; i < n; i++) {
-                const double x = __ldg(xc + (size_t)i * ldx);
+                const double x = xc.at(i);
                 const double eta = clampd(b0 + b1 * x, 30.0);
                 const double e = exp(eta);
                 if (i == 0) ew0 = e * ws[0];
@@ -1159,8 +1215,9 @@ __global__ void __launch_bounds__(128) screen_glm_kernel(const double *__restric
             double n0 = b0 - d0, n1 = b1 - d1, ll1 = 0.0;
             for (;;) {
                 ll1 = 0.0;
+                xc.start(false);
                 for (int i = 0; i < n; i++) {
-                    const double x = __ldg(xc + (size_t)i * ldx);
+                    const double x = xc.at(i);
                     const double eta = clampd(n0 + n1 * x, 30.0);
                     ll1 += (ys[i] * eta - exp(eta)) * ws[i];
                 }
@@ -1179,8 +1236,9 @@ __global__ void __launch_bounds__(128) screen_glm_kernel(const double *__restric
         for (int l = 1; l <= 30; l++) {
             // one backward pass: S0, S1, S2 running suffix sums
             double S0 = 0, S1 = 0, S2 = 0, g = 0, hneg = 0;
+            xc.start(true);
             for (int i = n - 1; i >= 0; i--) {
-                const double x = __ldg(xc + (size_t)i * ldx);
+                const double x = xc.at(i);
                 const double th = exp(clampd(b0 * x, 50.0));
                 S0 += th; S1 += th * x; S2 += th * x * x;
                 const double e = ws[i] * ys[i];
@@ -1194,8 +1252,9 @@ __global__ void __launch_bounds__(128) screen_glm_kernel(const double *__restric
             double b1 = b0 - step * d, ll1;
             for (;;) {
                 double S = 0, acc = 0;
+                xc.start(true);
                 for (int i = n - 1; i >= 0; i--) {
-                    const double x = __ldg(xc + (size_t)i * ldx);
+                    const double x = xc.at(i);
                     const double th = exp(clampd(b1 * x, 30.0));
                     S += th;
                     acc += log(th / S) * ys[i] * ws[i];
@@ -1217,8 +1276,123 @@ void launch_screen_glm(const double *X, long long ldx, int n, int p, const doubl
                        double *util, cudaStream_t st)
 {
     const size_t smem = (size_t)2 * n * sizeof(double);
-    CUDA_CHECK(cudaFuncSetAttribute(screen_glm_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    screen_glm_kernel<<<(p + 127) / 128, 128, smem, st>>>(X, ldx, n, p, y, w, family, util);
+    CUDA_CHECK(cudaFuncSetAttribute(screen_glm_kernel<DenseColumn>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    screen_glm_kernel<DenseColumn><<<(p + 127) / 128, 128, smem, st>>>(X, ldx, nullptr, nullptr, n, p, y, w, family, util);
+    CUDA_CHECK(cudaGetLastError());
+}
+void launch_screen_glm_csc(const long long *colptr, const int *rowidx, const double *values, int n, int p, const double *y,
+                           const double *w, int family, double *util, cudaStream_t st)
+{
+    const size_t smem = (size_t)2 * n * sizeof(double);
+    CUDA_CHECK(cudaFuncSetAttribute(screen_glm_kernel<CscColumn>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    screen_glm_kernel<CscColumn><<<(p + 127) / 128, 128, smem, st>>>(values, 0, colptr, rowidx, n, p, y, w, family, util);
+    CUDA_CHECK(cudaGetLastError());
+}
+
+// ---- sparse (CSC) designs.  A warp (or, for the gaussian utility, a sub-warp sized to the mean column length) owns a
+// column and walks its stored entries; offsets into rowidx / values are 64-bit.
+static unsigned csc_grid(long long items_per_block, long long count)
+{
+    return (unsigned)std::max<long long>(1, std::min<long long>((count + items_per_block - 1) / items_per_block, 148LL * 64));
+}
+
+// Validation of the caller's arrays: colptr[0] == 0, non-decreasing, colptr[p] == nnz; rows in [0, n) and strictly
+// increasing inside every column.  A column whose offsets are out of range is flagged and not read.
+__global__ void __launch_bounds__(256) csc_check_kernel(const long long *__restrict__ colptr, const int *__restrict__ rowidx,
+                                                        int n, int p, long long nnz, int *flag)
+{
+    const int lane = threadIdx.x & 31;
+    const long long nw = ((long long)gridDim.x * blockDim.x) >> 5;
+    int bad = 0;
+    for (long long j = ((long long)blockIdx.x * blockDim.x + threadIdx.x) >> 5; j < p; j += nw) {
+        const long long b = __ldg(colptr + j), e = __ldg(colptr + j + 1);
+        if (b < 0 || e < b || e > nnz || (j == 0 && b != 0) || (j == p - 1 && e != nnz)) {
+            bad |= CSC_BAD_COLPTR;
+            continue;
+        }
+        for (long long k = b + lane; k < e; k += 32) {
+            const int r = __ldg(rowidx + k);
+            if (r < 0 || r >= n) bad |= CSC_BAD_ROW;
+            if (k > b && __ldg(rowidx + k - 1) >= r) bad |= CSC_UNSORTED;
+        }
+    }
+    bad = __reduce_or_sync(0xffffffffu, bad);
+    if (lane == 0 && bad) atomicOr(flag, bad);
+}
+void launch_csc_check(const long long *colptr, const int *rowidx, int n, int p, long long nnz, int *flag, cudaStream_t st)
+{
+    csc_check_kernel<<<csc_grid(8, p), 256, 0, st>>>(colptr, rowidx, n, p, nnz, flag);
+    CUDA_CHECK(cudaGetLastError());
+}
+
+// Xn[rowidx[k]][q] = values[k] over the entries of column cols[q] (the columns screening keeps, or all of them)
+__global__ void __launch_bounds__(256) csc_densify_kernel(const long long *__restrict__ colptr, const int *__restrict__ rowidx,
+                                                          const double *__restrict__ values, const int *__restrict__ cols,
+                                                          int m, double *Xn, long long ldn)
+{
+    const int lane = threadIdx.x & 31;
+    const long long nw = ((long long)gridDim.x * blockDim.x) >> 5;
+    for (long long q = ((long long)blockIdx.x * blockDim.x + threadIdx.x) >> 5; q < m; q += nw) {
+        const int j = cols ? __ldg(cols + q) : (int)q;
+        const long long b = __ldg(colptr + j), e = __ldg(colptr + j + 1);
+        for (long long k = b + lane; k < e; k += 32) Xn[(size_t)__ldg(rowidx + k) * ldn + q] = __ldg(values + k);
+    }
+}
+void launch_csc_densify(const long long *colptr, const int *rowidx, const double *values, const int *cols, int m, double *Xn,
+                        long long ldn, cudaStream_t st)
+{
+    if (m <= 0) return;
+    csc_densify_kernel<<<csc_grid(8, m), 256, 0, st>>>(colptr, rowidx, values, cols, m, Xn, ldn);
+    CUDA_CHECK(cudaGetLastError());
+}
+
+// One-column least squares on the raw column (screening.cpp:46), (x_j.y / x_j.x_j)^2, over the non-zeros only: G lanes per
+// column, G the power of two nearest below the mean column length.  An all-zero column gives 0 / 0 as in the dense sweep.
+template <int G>
+__global__ void __launch_bounds__(256) screen_csc_lm_kernel(const long long *__restrict__ colptr,
+                                                            const int *__restrict__ rowidx,
+                                                            const double *__restrict__ values, int p,
+                                                            const double *__restrict__ y, double *util)
+{
+    const int lane = threadIdx.x % G;
+    const long long per_pass = ((long long)gridDim.x * blockDim.x) / G;
+    for (long long j0 = ((long long)blockIdx.x * blockDim.x) / G; j0 < p; j0 += per_pass) {
+        const long long j = j0 + threadIdx.x / G;
+        double ds = 0.0, hs = 0.0;
+        if (j < p) {
+            const long long b = __ldg(colptr + j), e = __ldg(colptr + j + 1);
+            for (long long k = b + lane; k < e; k += G) {
+                const double x = __ldg(values + k);
+                ds = fma(x, __ldg(y + __ldg(rowidx + k)), ds);
+                hs = fma(x, x, hs);
+            }
+        }
+#pragma unroll
+        for (int o = G / 2; o > 0; o >>= 1) {
+            ds += __shfl_xor_sync(0xffffffffu, ds, o, G);
+            hs += __shfl_xor_sync(0xffffffffu, hs, o, G);
+        }
+        if (j < p && lane == 0) {
+            const double bq = ds / hs;
+            util[j] = bq * bq;
+        }
+    }
+}
+void launch_screen_csc_lm(const long long *colptr, const int *rowidx, const double *values, int p, long long nnz,
+                          const double *y, double *util, cudaStream_t st)
+{
+    const double mean = (double)nnz / (double)p;
+    int g = 1;
+    while (g < 32 && 2 * g <= mean) g *= 2;
+    const unsigned grid = csc_grid(256 / g, p);
+    switch (g) {
+        case 1: screen_csc_lm_kernel<1><<<grid, 256, 0, st>>>(colptr, rowidx, values, p, y, util); break;
+        case 2: screen_csc_lm_kernel<2><<<grid, 256, 0, st>>>(colptr, rowidx, values, p, y, util); break;
+        case 4: screen_csc_lm_kernel<4><<<grid, 256, 0, st>>>(colptr, rowidx, values, p, y, util); break;
+        case 8: screen_csc_lm_kernel<8><<<grid, 256, 0, st>>>(colptr, rowidx, values, p, y, util); break;
+        case 16: screen_csc_lm_kernel<16><<<grid, 256, 0, st>>>(colptr, rowidx, values, p, y, util); break;
+        default: screen_csc_lm_kernel<32><<<grid, 256, 0, st>>>(colptr, rowidx, values, p, y, util); break;
+    }
     CUDA_CHECK(cudaGetLastError());
 }
 

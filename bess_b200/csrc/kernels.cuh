@@ -177,6 +177,19 @@ void launch_gather_cols_pos(const double *X, long long ldx, int n, const int *co
                             long long ld, cudaStream_t st);
 void launch_screen_glm(const double *X, long long ldx, int n, int p, const double *y, const double *w, int family,
                        double *util, cudaStream_t st);
+// ---- sparse (CSC) designs: colptr [p + 1] 64-bit offsets, rowidx / values [nnz]
+// flag |= CSC_BAD_COLPTR / CSC_BAD_ROW / CSC_UNSORTED (one O(nnz) pass; a column whose offsets are bad is not read)
+enum { CSC_BAD_COLPTR = 1, CSC_BAD_ROW = 2, CSC_UNSORTED = 4 };
+void launch_csc_check(const long long *colptr, const int *rowidx, int n, int p, long long nnz, int *flag, cudaStream_t st);
+// Xn[rowidx[k]][q] = values[k] for the entries of column cols[q] (cols == nullptr: column q), q < m; Xn zero-filled
+void launch_csc_densify(const long long *colptr, const int *rowidx, const double *values, const int *cols, int m, double *Xn,
+                        long long ldn, cudaStream_t st);
+// gaussian screening utility (x_j.y / x_j.x_j)^2 of every column over its non-zeros
+void launch_screen_csc_lm(const long long *colptr, const int *rowidx, const double *values, int p, long long nnz,
+                          const double *y, double *util, cudaStream_t st);
+// screen_glm_kernel with a CSC column reader (absent rows read as 0.0): the same arithmetic in the same order
+void launch_screen_glm_csc(const long long *colptr, const int *rowidx, const double *values, int n, int p, const double *y,
+                           const double *w, int family, double *util, cudaStream_t st);
 // device-side gen.data design (gen_design.cu): X[i][j], row-major n x p with leading dimension ld
 void launch_gen_design(double *X, long long ld, int n, long long p, double rho, unsigned long long seed, cudaStream_t st);
 void launch_gen_design_cortype(double *X, long long ld, int n, long long p, double rho, unsigned long long seed, int cortype,

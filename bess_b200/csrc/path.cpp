@@ -770,7 +770,9 @@ static void bess_run_once(const BessArgs &a, BessResult &out, bool tie_exact)
 {
     // ---- argument validation (the reference validates in its R/Python front-ends and dereferences null otherwise,
     // SURVEY Q19; here bad arguments are reported)
-    if (!a.x || !a.y || !a.weight) throw EngineError{"x, y and weight must be non-null"};
+    if ((!a.x && !a.csc) || !a.y || !a.weight) throw EngineError{"x, y and weight must be non-null"};
+    if (a.csc && a.x) throw EngineError{"x and x_csc are both given: pass the design one way"};
+    if (a.csc && a.world > 1) throw EngineError{"a sparse design (x_csc) is single-GPU only (world must be <= 1)"};
     if (a.n < 2 || a.p < 1) throw EngineError{"need n >= 2 and p >= 1"};
     if (!(a.algorithm_type == 1 || a.algorithm_type == 2 || a.algorithm_type == 3 || a.algorithm_type == 5))
         throw EngineError{"algorithm_type must be 1 (PDAS), 2, 3 or 5 (bess.cpp:93)"};
@@ -821,7 +823,12 @@ static void bess_run_once(const BessArgs &a, BessResult &out, bool tie_exact)
     eng.set_profiling(a.profile);
     if (shard) eng.init_shard(a.world, a.rank, a.nccl_id, a.col_lo, a.p_total);
     else if (a.fold_shard && a.world > 1 && a.is_cv) eng.init_comm(a.world, a.rank, a.nccl_id);
-    eng.load(a.x, a.n, a.p, a.x_on_device, a.y, a.weight, a.model_type, /*borrow=*/a.is_screening);
+    if (a.csc) {
+        eng.load_csc(a.csc_colptr, a.csc_rowidx, a.csc_values, a.n, a.p, a.csc_nnz, a.x_on_device, a.y, a.weight, a.model_type);
+        if (!a.is_screening) eng.densify();  // screening densifies only the columns it keeps
+    } else {
+        eng.load(a.x, a.n, a.p, a.x_on_device, a.y, a.weight, a.model_type, /*borrow=*/a.is_screening);
+    }
 
     lap(0);
     std::vector<int> always = a.always_select;

@@ -56,6 +56,12 @@ struct BessArgs {
     // chain, and only the per-fold test losses are reduced (one NCCL all-reduce of K numbers per evaluated level; the
     // sequential path reduces its whole levels x K matrix once).  world / rank / nccl_id as above, col_lo / p_total unused.
     bool fold_shard = false;
+    // sparse design (bess_b200_csc): x is then null and the three arrays (device pointers when x_on_device) give n x p
+    bool csc = false;
+    const long long *csc_colptr = nullptr;
+    const int *csc_rowidx = nullptr;
+    const double *csc_values = nullptr;
+    long long csc_nnz = 0;
 };
 
 struct BessResult {

@@ -51,6 +51,18 @@ class GpuEngine:
         _lib.check(self._lib.bessgpu_load(self._h, ptr, n, p, on_dev, _d(y), _d(w), model_type))
         self.n, self.p = n, p
 
+    def load_csc(self, x, y, weight, model_type):
+        """``load`` for a sparse design: a scipy.sparse matrix (canonicalised) or a raw ``(indptr, indices, data, shape)``
+        tuple of host arrays or torch CUDA tensors (see ``cbess.csc_arrays``).  Returns self."""
+        from .cbess import csc_arrays
+        y = np.ascontiguousarray(y, dtype=np.float64)
+        w = np.ascontiguousarray(weight, dtype=np.float64)
+        cp, ri, cv, nnz, (n, p), on_dev, keep = csc_arrays(x)
+        _lib.check(self._lib.bessgpu_load_csc(self._h, cp, ri, cv, n, p, nnz, int(on_dev), _d(y), _d(w), model_type))
+        self._csc_arrays = keep  # device tensors are read in place until screening
+        self.n, self.p = n, p
+        return self
+
     def screen(self, size, always_select=()):
         alw = np.ascontiguousarray(list(always_select), dtype=np.int32)
         out = np.zeros(size, dtype=np.int32)

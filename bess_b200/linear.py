@@ -13,6 +13,7 @@ import math
 
 import numpy as np
 
+from . import cbess
 from .cbess import pywrap_bess
 
 _ALG = {"Pdas": 1, "GroupPdas": 2, "L0L2": 5}
@@ -55,9 +56,12 @@ class bess_base:
         self.ic_type_int = _IC[self.ic_type]
 
     def fit(self, X, y, is_weight=False, is_normal=True, weight=None, state=None, group=None):
-        X = np.asarray(X, dtype=np.float64)
+        """X: an n x p array, or a scipy.sparse matrix in any format (sent to the library in CSC form; the fit sees the
+        same values as on X.toarray())."""
+        sparse = cbess.is_sparse(X)
+        X = cbess.canonical_csc(X) if sparse else np.asarray(X, dtype=np.float64)
         y = np.asarray(y, dtype=np.float64)
-        if np.isnan(X).any():
+        if np.isnan(X.data if sparse else X).any():
             raise ValueError("There is NAN value in X")
         if np.isnan(y).any():
             raise ValueError("There is NAN value in y")
@@ -76,7 +80,7 @@ class bess_base:
             g_index = np.arange(p, dtype=np.int32)
         if self.model_type_int == 4:
             order = y[:, 0].argsort()  # linear.py:257-263: rows sorted by time, y <- status
-            X = X[order]
+            X = cbess.canonical_csc(X.tocsr()[order]) if sparse else X[order]
             y = y[order][:, 1].reshape(-1)
         if n != y.size:
             raise ValueError("X.shape(0) should be equal to y.size")
@@ -121,6 +125,15 @@ class bess_base:
             screening_size = min(self.screening_size, p)
         else:
             self.screening_size = screening_size = 1
+        if sparse:  # the extended entry takes the CSC design; the arguments pywrap_bess ignores are left out
+            out = cbess.fit(X, y, self.data_type, weight, is_normal, self.algorithm_type_int, self.model_type_int,
+                            self.max_iter, self.exchange_num, self.path_type_int, self.is_warm_start, self.ic_type_int,
+                            self.is_cv, self.K, self.sequence, self.s_min, self.s_max, self.is_screening, screening_size,
+                            always_select=self.always_select, want_trace=False, lambda_seq=self.lambda_sequence,
+                            lambda_min=self.lambda_min or 0, lambda_max=self.lambda_max or 0, n_lambda=self.n_lambda,
+                            powell_path=self.powell_path, g_index=g_index if self.algorithm_type_int == 2 else None)
+            self.beta, self.coef0, self.train_loss, self.ic = out["beta"], out["coef0"], out["train_loss"], out["ic"]
+            return self
         result = pywrap_bess(X, y, self.data_type, weight, is_normal, self.algorithm_type_int, self.model_type_int,
                              self.max_iter, self.exchange_num, self.path_type_int, self.is_warm_start, self.ic_type_int,
                              self.is_cv, self.K, g_index, state, self.sequence, self.lambda_sequence, self.s_min,
@@ -131,10 +144,11 @@ class bess_base:
         return self
 
     def predict(self, X):
-        X = np.asarray(X, dtype=np.float64)
+        """X: an array or a scipy.sparse matrix."""
+        X = cbess.canonical_csc(X) if cbess.is_sparse(X) else np.asarray(X, dtype=np.float64)
         if X.shape[1] != self.p:
             raise ValueError("X.shape[1] should be " + str(self.p))
-        eta = X @ self.beta + self.coef0
+        eta = np.asarray(X @ self.beta).ravel() + self.coef0
         if self.model_type_int == 1:
             return eta
         if self.model_type_int == 2:

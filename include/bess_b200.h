@@ -53,6 +53,19 @@ void pywrap_bess(double *x, int x_row, int x_col, double *y, int y_len, int data
                  double *aic_out, int aic_out_len, double *bic_out, int bic_out_len, double *gic_out, int gic_out_len,
                  int *A_out, int A_out_len, int *l_out);
 
+/* A sparse design in compressed sparse column (CSC) form: column j holds the rows rowidx[colptr[j] .. colptr[j+1]) with
+ * the values values[colptr[j] .. colptr[j+1]); every other entry is 0.  Offsets are 64-bit, so nnz may exceed 2^31.
+ * bess_b200_fit checks the input and returns 1 with a message rather than repairing it:
+ *   colptr[0] == 0, colptr non-decreasing, colptr[p] == nnz  (O(p), on the host; on the device for device arrays);
+ *   0 <= rowidx[k] < n and rowidx strictly increasing inside every column (no duplicates)  (one O(nnz) device pass).
+ * The values are used as given (fp64, lossless): the fit sees exactly the matrix a dense call with the same entries sees. */
+typedef struct bess_b200_csc {
+    const long long *colptr;  /* [p + 1] column offsets                                                                  */
+    const int *rowidx;        /* [nnz] row of every stored entry                                                          */
+    const double *values;     /* [nnz] value of every stored entry (explicit zeros allowed)                               */
+    long long nnz;
+} bess_b200_csc;
+
 /* Extensions for bess_b200_fit (all optional; zero-initialise the struct for defaults). */
 typedef struct bess_b200_ext {
     const int *fold_of_row;   /* explicit CV fold of every row (length n, values 0..K-1); NULL = draw from cv_seed   */
@@ -65,7 +78,8 @@ typedef struct bess_b200_ext {
                               /*  5 PDAS dual-sweep algorithmic bytes, 6 kernel_launches, 7 trace_len,                */
                               /*  8..15 device ms per kernel category (profile != 0): screening sweep, PDAS dual      */
                               /*  sweeps, finish, top-k, chain kernels, other, normalisation passes, H2D upload;      */
-                              /*  16..23 launches per category; 24 algorithmic bytes of the screening sweep (8np);    */
+                              /*  16..23 launches per category; 24 algorithmic bytes of the screening sweep (8np;     */
+                              /*  sparse design: 12 nnz + 8 (p + 1) + the n-vectors it reads); 7 covers a CSC copy;   */
                               /*  25 sweep row splits; 26 algorithmic bytes of the normalisation / x_j.x_j passes;    */
                               /*  27..31 host wall-clock ms by phase: load, screening, normalisation, fold / chain    */
                               /*  set-up, path                                                                        */
@@ -100,6 +114,11 @@ typedef struct bess_b200_ext {
                                 /* c % world, bess_b200_chain_owner), every rank runs the full-data chain, and only the       */
                                 /* per-fold test losses are all-reduced -- SURVEY 8e axis A inside ONE call; every rank       */
                                 /* returns the same model, bit-identical to the single-GPU call                               */
+    const bess_b200_csc *x_csc; /* non-NULL: the design is sparse (see bess_b200_csc); x must then be NULL, x_row / x_col give */
+                                /* n and p, and x_on_device = 1 means the three arrays are device pointers (read in place,   */
+                                /* never written).  Screening densifies only the kept columns; without screening the whole    */
+                                /* design is densified on the device (n * p * 8 bytes must fit).  Single GPU only (world <= 1); */
+                                /* screening together with groups is refused as for dense designs                             */
 } bess_b200_ext;
 
 /* Same arguments and outputs as pywrap_bess, returns 0 on success.  The per-level trace of the call (what the reference's
@@ -152,6 +171,9 @@ int bessgpu_destroy(bessgpu_handle *h);
 /* upload (or device-to-device copy) the design; replaces the by-value copies of bess.cpp:233/61 and Algorithm.h:58 */
 int bessgpu_load(bessgpu_handle *h, const double *x, int n, int p, int x_on_device, const double *y,
                  const double *weight, int model_type);
+/* the same for a CSC design (bess_b200_csc, same validation); it stays sparse until bessgpu_screen keeps its columns */
+int bessgpu_load_csc(bessgpu_handle *h, const long long *colptr, const int *rowidx, const double *values, int n, int p,
+                     long long nnz, int on_device, const double *y, const double *weight, int model_type);
 /* screening.cpp:26-105; out: screening_size kept columns, ascending */
 int bessgpu_screen(bessgpu_handle *h, int screening_size, const int *always_select, int n_always, int *screening_A_out);
 /* column-sharded screening (multi-GPU): the local top-`size` candidates of this handle's columns as (utility, local
