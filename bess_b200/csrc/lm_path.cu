@@ -10,13 +10,14 @@
 //
 //   * SWEEPER CTAs (all but one CTA per chain) each own a slice of ~p/137 adjacent columns for the whole launch.  Per
 //     iteration a sweeper stages the residual vectors of all chains ([n][FT], one bulk-TMA copy into shared memory), walks
-//     all n rows of its slice once (16-byte loads of X from L2, 2*FT fp64 FMAs per load), reduces its row phases in a
+//     all n rows of its slice once (the leading rows from a copy it keeps in the shared memory the owners' budget leaves
+//     it, the others as 16-byte loads of X from L2; 2*FT fp64 FMAs per 16 bytes), reduces its row phases in a
 //     fixed order, applies the splicing sacrifice (Algorithm.h:1112-1123) and writes bd; values above the chain's
 //     published threshold are appended to a short candidate list.  No row splits, no partial vectors in memory.
 //   * one OWNER CTA per chain keeps the chain's state in shared memory for the whole launch: the active columns X_A (all
 //     n rows, column-major, in reusable slots), their Gram matrix and X_A^T y (cached per slot pair -- a PDAS iteration
 //     typically exchanges 0-3 columns, only those rows of the Gram are recomputed), the response, the fold mask and
-//     A_list.  Per iteration it ranks the candidates (exact top-k: larger value first, lower index first; falls back to a
+//     A_list.  Per iteration it ranks the best candidates (exact top-k: larger value first, lower index first; falls back to a
 //     radix select over the whole bd vector when the list is short or overflows), loads the new columns, solves the
 //     bordered normal equations by Cholesky, publishes the residual of the next sweep and runs the cycle test
 //     (Algorithm.h:164-170).  A chain that has met the stopping rule writes its result (support, coefficients, l, train /
@@ -217,6 +218,16 @@ __host__ __device__ inline size_t sweeper_smem_doubles(int npad, int FT)
     return (r > scr ? r : scr) + 16 + 16 + 2 + 2;
 }
 
+// Slice width in column pairs, rounded to even: a row segment of an even number of pairs is a whole number of 32-byte
+// sectors (measured: 18-pair slices stream 15 % faster than 17- or 19-pair ones)
+__host__ __device__ inline int sweeper_pairs(int p, int nsweep)
+{
+    const int P2 = (p + 1) >> 1;
+    int WpA = (P2 + nsweep - 1) / nsweep;
+    if (WpA > 1 && (WpA & 1) && WpA < LP_WPMAX) WpA++;
+    return WpA;
+}
+
 template <int FT>
 __device__ void sweeper_main(const Dev &d, const LpDesc &L, unsigned char *raw)
 {
@@ -238,10 +249,7 @@ __device__ void sweeper_main(const Dev &d, const LpDesc &L, unsigned char *raw)
     const int n = d.n, npad = (n + 1) & ~1;
     const int sidx = (int)blockIdx.x - L.nch;
     const int P2 = (d.p + 1) >> 1;
-    // slice width in column pairs, rounded to even: a row segment of an even number of pairs is a whole number of 32-byte
-    // sectors (measured: 18-pair slices stream 15 % faster than 17- or 19-pair ones)
-    int WpA = (P2 + L.nsweep - 1) / L.nsweep;
-    if (WpA > 1 && (WpA & 1) && WpA < LP_WPMAX) WpA++;
+    const int WpA = sweeper_pairs(d.p, L.nsweep);
     const int q0 = min(P2, sidx * WpA), q1 = min(P2, q0 + WpA);
     const int Wp = q1 - q0;
     const int RP = Wp > 0 ? min(LP_NT / Wp, LP_RPMAX) : 0;
@@ -249,6 +257,22 @@ __device__ void sweeper_main(const Dev &d, const LpDesc &L, unsigned char *raw)
     const bool active = Wp > 0 && rp < RP;
     const int W2 = 2 * Wp, nout = W2 * FT;
     const uint32_t rbytes = (uint32_t)((size_t)npad * FT * sizeof(double));
+    // The launch sizes its shared memory for the owners; what the residual stage leaves free keeps the first nres rows of
+    // the slice on chip for the whole launch, [nres][W2] (a warp's double2 reads are consecutive: conflict-free).  Each sweep
+    // reads those rows from shared memory and streams only rows nres.. from L2.
+    double2 *Xs = reinterpret_cast<double2 *>(raw + sweeper_smem_doubles(npad, FT) * sizeof(double));
+    int nres = 0;
+    if (Wp > 0) {
+        unsigned dyn;
+        asm("mov.u32 %0, %%dynamic_smem_size;" : "=r"(dyn));
+        const size_t used = sweeper_smem_doubles(npad, FT) * sizeof(double);
+        if (dyn > used) nres = (int)min((size_t)n, (dyn - used) / (sizeof(double2) * Wp));
+    }
+#pragma unroll 4
+    for (int e = tid; e < nres * Wp; e += LP_NT) {
+        const int i = e / Wp, q = e - i * Wp;
+        Xs[e] = ldg_stream_v2(d.X + (size_t)i * d.ldx + 2 * (size_t)(q0 + q));
+    }
     if (tid == 0) {
         lp_mbar_init(sm.mbar, 1);
         asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
@@ -293,17 +317,39 @@ __device__ void sweeper_main(const Dev &d, const LpDesc &L, unsigned char *raw)
 #pragma unroll
             for (int f = 0; f < FT; f++) a0[f] = a1[f] = 0.0;
             if (active) {
-                // software pipeline: the x loads of row group g + 1 are in flight while group g is multiplied
+                // row i of this thread's column pair into the sums; every thread adds its rows in ascending order
+                auto row_fma = [&](const double2 xv, int i) {
+                    const double *r = sm.R + (size_t)i * FT;
+                    if constexpr (FT == 1) {
+                        const double g = r[0];
+                        a0[0] = fma(xv.x, g, a0[0]);
+                        a1[0] = fma(xv.y, g, a1[0]);
+                    } else {
+#pragma unroll
+                        for (int f = 0; f < FT; f += 2) {
+                            const double2 g = *reinterpret_cast<const double2 *>(r + f);
+                            a0[f] = fma(xv.x, g.x, a0[f]);
+                            a1[f] = fma(xv.y, g.x, a1[f]);
+                            a0[f + 1] = fma(xv.x, g.y, a0[f + 1]);
+                            a1[f + 1] = fma(xv.y, g.y, a1[f + 1]);
+                        }
+                    }
+                };
+                // software pipeline: the x loads of row group g + 1 are in flight while group g is multiplied; the first
+                // streamed group is in flight while the on-chip rows are multiplied
                 constexpr int U = 4;
                 const double *xp = d.X + 2 * (size_t)(q0 + cp);
+                const int is = rp + (nres > rp ? (nres - rp + RP - 1) / RP : 0) * RP;  // first row of this thread from L2
                 double2 xn[U];
 #pragma unroll
                 for (int u = 0; u < U; u++) {
-                    const int i = rp + u * RP;
+                    const int i = is + u * RP;
                     xn[u] = i < n ? ldg_stream_v2(xp + (size_t)i * d.ldx) : make_double2(0.0, 0.0);
                 }
                 lp_mbar_wait(sm.mbar, parity);
-                for (int i0 = rp; i0 < n; i0 += RP * U) {
+#pragma unroll 4
+                for (int i = rp; i < nres; i += RP) row_fma(Xs[(size_t)i * Wp + cp], i);
+                for (int i0 = is; i0 < n; i0 += RP * U) {
                     double2 xv[U];
 #pragma unroll
                     for (int u = 0; u < U; u++) xv[u] = xn[u];
@@ -315,23 +361,7 @@ __device__ void sweeper_main(const Dev &d, const LpDesc &L, unsigned char *raw)
 #pragma unroll
                     for (int u = 0; u < U; u++) {
                         const int i = i0 + u * RP;
-                        if (i < n) {
-                            const double *r = sm.R + (size_t)i * FT;
-                            if constexpr (FT == 1) {
-                                const double g = r[0];
-                                a0[0] = fma(xv[u].x, g, a0[0]);
-                                a1[0] = fma(xv[u].y, g, a1[0]);
-                            } else {
-#pragma unroll
-                                for (int f = 0; f < FT; f += 2) {
-                                    const double2 g = *reinterpret_cast<const double2 *>(r + f);
-                                    a0[f] = fma(xv[u].x, g.x, a0[f]);
-                                    a1[f] = fma(xv[u].y, g.x, a1[f]);
-                                    a0[f + 1] = fma(xv[u].x, g.y, a0[f + 1]);
-                                    a1[f + 1] = fma(xv[u].y, g.y, a1[f + 1]);
-                                }
-                            }
-                        }
+                        if (i < n) row_fma(xv[u], i);
                     }
                 }
             } else {
@@ -411,7 +441,7 @@ struct OwnSm {
     int *misc;     // [16]
     int ldS;
 };
-enum { MI_FLAG = 0, MI_CNT = 1, MI_NNEW = 2, MI_SEEN = 3, MI_TIE = 4, MI_KREM = 5, MI_NEQ = 6, MI_COUNT = 7, MI_Q = 8 };
+enum { MI_FLAG = 0, MI_CNT = 1, MI_NNEW = 2, MI_SEEN = 3, MI_TIE = 4, MI_KREM = 5, MI_NEQ = 6, MI_COUNT = 7, MI_Q = 8, MI_RANKN = 9 };
 
 __host__ __device__ inline size_t owner_smem_bytes(int npad, int kcap, int ns, int hist_rows)
 {
@@ -628,9 +658,89 @@ __device__ void fallback_select(const double *bd, int p, int kk, OwnSm &s, int *
 // non-negative doubles, so their bit patterns order like the values and the comparisons stay off the FP64 pipe) and file
 // the best 2 * kcap + 8 of them by rank: every select of this phase (the closing cycle test of a fit, then the first
 // iteration of the next path step) reads its winners, its boundary and its next threshold from that table.
+constexpr int RANK_DIRECT = 128;  // lists up to this size are ranked by direct comparison alone (P = 4)
 __device__ void rank_candidates(OwnSm &s, int count, int rmax)
 {
     const int tid = threadIdx.x;
+    if (count > RANK_DIRECT && count > rmax) {
+        // Only ranks below rmax are read.  Narrow the list to the keys that can hold one: MSB-first radix digits of the bit
+        // patterns, from the highest bit in which the keys differ, until the keys above the boundary digit plus that
+        // digit's whole bin are at most RANK_DIRECT (or every bit is decided: exact ties).  Every dropped key ranks below
+        // every kept one, so the kept keys ranked among themselves get their ranks in the whole list.
+        const int lane = tid & 31, wid = tid >> 5;
+        const bool have = tid < count;
+        const unsigned long long key = have ? (unsigned long long)__double_as_longlong(s.cv[tid]) : 0ull;
+        const int idx = have ? s.ci[tid] : 0;
+        const unsigned long long dx = have ? key ^ (unsigned long long)__double_as_longlong(s.cv[0]) : 0ull;
+        const unsigned ohi = __reduce_or_sync(0xffffffffu, (unsigned)(dx >> 32)), olo = __reduce_or_sync(0xffffffffu, (unsigned)dx);
+        if (lane == 0) {
+            s.hbin[2 * wid] = (int)ohi;
+            s.hbin[2 * wid + 1] = (int)olo;
+        }
+        if (tid == 0) s.misc[MI_RANKN] = 0;
+        __syncthreads();
+        unsigned long long dall = 0ull;
+        for (int w = 0; w < LP_NT / 32; w++)
+            dall |= ((unsigned long long)(unsigned)s.hbin[2 * w] << 32) | (unsigned)s.hbin[2 * w + 1];
+        unsigned long long *pre_sh = reinterpret_cast<unsigned long long *>(s.red);
+        if (dall != 0ull) {
+            int hb = 63 - __clzll((long long)dall), lb = max(hb - 7, 0);
+            unsigned long long mask = hb == 63 ? 0ull : ~0ull << (hb + 1);  // the bits above hb are equal in all keys
+            unsigned long long prefix;
+            if (tid == 0) *pre_sh = (unsigned long long)__double_as_longlong(s.cv[0]) & mask;
+            int krem = rmax;
+            for (;;) {
+                __syncthreads();
+                prefix = *pre_sh;
+                if (tid < 256) s.hbin[tid] = 0;
+                __syncthreads();
+                const unsigned long long dmask = (2ull << (hb - lb)) - 1ull;
+                if (have && (key & mask) == prefix) atomicAdd(&s.hbin[(int)((key >> lb) & dmask)], 1);
+                __syncthreads();
+                if (tid < 32) {
+                    int loc[8], tot = 0;
+#pragma unroll
+                    for (int q = 0; q < 8; q++) {
+                        loc[q] = s.hbin[tid * 8 + q];
+                        tot += loc[q];
+                    }
+                    int suf = tot;
+#pragma unroll
+                    for (int o = 1; o < 32; o <<= 1) {
+                        const int t = __shfl_down_sync(0xffffffffu, suf, o);
+                        if (tid + o < 32) suf += t;
+                    }
+                    const int above = suf - tot;
+                    if (above < krem && suf >= krem) {
+                        int acc = above;
+                        for (int q = 7; q >= 0; q--) {
+                            if (acc + loc[q] >= krem) {
+                                *pre_sh = prefix | ((unsigned long long)(tid * 8 + q) << lb);
+                                s.misc[MI_KREM] = krem - acc;
+                                s.misc[MI_NEQ] = loc[q];
+                                break;
+                            }
+                            acc += loc[q];
+                        }
+                    }
+                }
+                __syncthreads();
+                prefix = *pre_sh;
+                krem = s.misc[MI_KREM];
+                mask |= dmask << lb;
+                if ((rmax - krem) + s.misc[MI_NEQ] <= RANK_DIRECT || lb == 0) break;
+                hb = lb - 1;
+                lb = max(hb - 7, 0);
+            }
+            if (have && (key & mask) >= prefix) {
+                const int pos = atomicAdd(&s.misc[MI_RANKN], 1);
+                s.cv[pos] = __longlong_as_double((long long)key);
+                s.ci[pos] = idx;
+            }
+            __syncthreads();
+            count = s.misc[MI_RANKN];
+        }
+    }
     // P threads per candidate split the comparison loop (P = 4 while 4 * count fits the CTA): the loop is a chain of
     // shared-memory loads and integer compares that a thread cannot overlap with anything, so its length is the cost
     const int P = count * 4 <= LP_NT ? 4 : (count * 2 <= LP_NT ? 2 : 1);
@@ -1431,7 +1541,11 @@ bool lm_path_eligible(const Dev &d, int max_iter, int sm_count, std::string *why
 
 void launch_lm_path(const Dev &d, const LpDesc &desc, int sm_count, int max_iter, cudaStream_t st)
 {
-    const size_t smem = lm_path_smem_bytes(d, max_iter, sm_count);
+    // CTAs run one per SM whatever they request: when the owners need less than the whole budget, ask for enough to keep
+    // each sweeper's whole slice on chip (sweeper_main), up to the budget
+    const size_t slice = (size_t)d.n * sweeper_pairs(d.p, desc.nsweep) * 2 * sizeof(double);
+    const size_t want = std::min(sweeper_smem_doubles((d.n + 1) & ~1, desc.fh) * sizeof(double) + slice, (size_t)(232448 - 2048));
+    const size_t smem = std::max(lm_path_smem_bytes(d, max_iter, sm_count), (want + 127) & ~(size_t)127);
     void (*fn)(const Dev, const LpDesc) = nullptr;
     switch (desc.fh) {
         case 1: fn = lm_path_kernel<1>; break;
