@@ -443,7 +443,8 @@ int bessgpu_stats(bessgpu_handle *h, double *o)
     return guarded([&] {
         const EngineStats &s = h->eng->stats();
         o[0] = (double)s.n_fits; o[1] = (double)s.n_pdas_iters; o[2] = (double)s.n_sweeps; o[3] = (double)s.n_batches;
-        o[4] = (double)s.n_boundary_ties; o[5] = s.sweep_bytes; o[6] = (double)s.kernel_launches; o[7] = 0.0;
+        o[4] = (double)s.n_boundary_ties; o[5] = s.sweep_bytes; o[6] = (double)s.kernel_launches;
+        o[7] = (double)s.max_cluster;
     });
 }
 int bessgpu_topk(const double *vals, int n, int k, int *idx_out, int *tie_out)
@@ -489,6 +490,17 @@ int bess_b200_debug_gram(const double *V, int ldv, int nrows, int mm, const doub
 int bess_b200_debug_solve(const double *S, int lds, int mm, double *x_out, int impl, int reps, double *ticks_out)
 {
     return guarded([&] { debug_solve(S, lds, mm, x_out, impl, reps, ticks_out); });
+}
+// S: (mm + 1) x lds bordered system, placed and solved as a fit with support cap kcap would; path_out: int[3]
+int bess_b200_debug_solve_path(const double *S, int lds, int mm, int kcap, double *x_out, int *path_out)
+{
+    return guarded([&] { debug_solve_path(S, lds, mm, kcap, x_out, path_out); });
+}
+// Gram of rows [r0, r1) of V; S_io: ldo x ldo (ldo = 64 when mm <= 64, else ldv), initial contents in, result out
+int bess_b200_debug_gram_rows(const double *V, int ldv, int r0, int r1, int mm, const double *wt, double *S_io, int kcap,
+                              int impl)
+{
+    return guarded([&] { debug_gram_rows(V, ldv, r0, r1, mm, wt, S_io, kcap, impl); });
 }
 
 // ---- multi-GPU host helpers ------------------------------------------------------------------------------------------

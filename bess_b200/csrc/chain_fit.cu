@@ -505,7 +505,9 @@ __device__ __noinline__ void block_syrk_dmma(const double *V, int ldv, int r0, i
 #pragma unroll
                     for (int w = 0; w < 2; w++) {
                         const int a = ti[u] * 16 + mt * 8 + g, b = tj[u] * 16 + nt * 8 + t4 * 2 + w;
-                        if (a < mm && b < mm) {
+                        // lower triangle only: a diagonal tile holds (a, b) and (b, a), rounded differently (the weight
+                        // scales the B operand), and both would be stored to both places
+                        if (a < mm && b < mm && a >= b) {
                             S[(size_t)a * lds + b] = acc[u][mt][nt][w];
                             S[(size_t)b * lds + a] = acc[u][mt][nt][w];
                         }
@@ -572,6 +574,8 @@ __device__ __forceinline__ void gram(const double *V, int ldv, int r0, int r1, i
 // A pivot at or below PIVOT_TOL times the column's own diagonal entry (its squared norm) is a numerically dependent column.
 constexpr double PIVOT_TOL = 1e-13;
 __device__ unsigned long long g_rankdef_count = 0ull;  // truncated (rank-deficient) solves since the last debug_take_rankdef()
+// singular systems of more than FIT_SMEM_MS unknowns (chol_panel_major: x <- NaN) since the last take_wide_singular()
+__device__ unsigned long long g_wide_singular_count = 0ull;
 // S0: pristine copy of the system (same layout).  Returns false -- S is then garbage -- when a pivot fails the test above.
 __device__ bool block_chol_solve_small(double *S, int lds, int mm, double *x, double *dg, const double *S0)
 {
@@ -1199,7 +1203,10 @@ __device__ void pm_backsub(const double *L, const int *poff, int mm, int c0, int
     }
 }
 // Sg: bordered system in global memory (row-major, lower triangle + border row mm); multi-stage runs overwrite it.
-// x (shared memory) <- solution.
+// x (shared memory) <- solution.  There is no rank-revealing fallback at this size: a pivot at or below PIVOT_TOL times
+// its column's original diagonal entry (tested after the factorisation on dinv = 1 / L_jj, a NaN dinv -- a non-positive
+// pivot -- failing too) makes the whole x NaN and counts in g_wide_singular_count, so a singular system never returns a
+// finite solution.  The original diagonal is kept in sm.b1, which no caller uses across a solve.
 __device__ __noinline__ void chol_panel_major(double *Sg, int lds, int mm, double *x, const FitSmem &sm_, PhaseTimer &pt,
                                               bool preloaded = false)
 {
@@ -1212,6 +1219,7 @@ __device__ __noinline__ void chol_panel_major(double *Sg, int lds, int mm, doubl
     double *L = as_shared(sm.tile) + 64;
     double *dg = as_shared(sm.dg);
     double *red = as_shared(sm.red);
+    double *diag0 = as_shared(sm.b1);
     x = as_shared(x);
     const int cap = pm_capacity(sm.arena_len);
     int sc0[PM_MAX_STAGES], snp[PM_MAX_STAGES], ns = 0;
@@ -1226,6 +1234,13 @@ __device__ __noinline__ void chol_panel_major(double *Sg, int lds, int mm, doubl
         const int c0 = sc0[s], np = snp[s];
         pm_offsets(poff, mm, c0, np);
         if (!(preloaded && s == 0)) pm_copy<false>(L, poff, Sg, lds, mm, c0, np);  // (reduce_to_panels filled stage 0)
+        if (s == 0) {  // stage 0's columns from its panels, the later ones from Sg before the first Schur update
+            for (int j = threadIdx.x; j < mm; j += FIT_NT) {
+                const int pb = j >> 4, q = j & (PNB - 1);
+                diag0[j] = pb < np ? L[poff[pb] + q * pm_ld(mm + 1 - pb * PNB) + q] : Sg[(size_t)j * lds + j];
+            }
+            __syncthreads();
+        }
         pt.mark(10);
         if (threadIdx.x < 32) pm_diag_factor(L + poff[0], pm_ld(mm + 1 - c0), min(PNB, mm - c0), dg + c0, colbuf);
         __syncthreads();
@@ -1251,6 +1266,14 @@ __device__ __noinline__ void chol_panel_major(double *Sg, int lds, int mm, doubl
             pm_copy<false>(L, poff, Sg, lds, mm, c0, np);
         }
         pm_backsub(L, poff, mm, c0, np, x, red, dg + c0);
+    }
+    // pivot_j = 1 / dinv_j^2 > PIVOT_TOL * diag0_j, written so that a NaN dinv fails
+    bool bad = false;
+    for (int j = threadIdx.x; j < mm; j += FIT_NT) bad |= !(dg[j] * dg[j] * (PIVOT_TOL * diag0[j]) < 1.0);
+    if (__syncthreads_or(bad)) {
+        for (int j = threadIdx.x; j < mm; j += FIT_NT) x[j] = __longlong_as_double(0x7ff8000000000000ll);
+        if (threadIdx.x == 0) atomicAdd(&g_wide_singular_count, 1ull);
+        __syncthreads();
     }
     pt.mark(12);
 }
@@ -1459,16 +1482,26 @@ __device__ __noinline__ bool warp_chol_solve32(const double *S, int lds, int nu,
     return true;
 }
 
-// Rank 0 holds a bordered system (nu unknowns) at S -- its own shared memory (small systems) or the chain's global matrix
-// (large systems, then every CTA of the cluster takes part in the factorisation): solve it and hand the solution to
-// every CTA of the cluster (out: smem).
-__device__ void solve_broadcast(const ChainCtx &cx, Clu &cl, double *S, int lds, int nu, double *out, const FitSmem &sm_,
-                                bool preloaded = false)
+// Which solver finished a normal-equation solve (solve_on_rank0's return value, reported by the solve probe).
+enum {
+    SOLVE_WARP = 1, SOLVE_WARP_LDLT = 2,   // warp_chol_solve32, and its rank-revealing fallback
+    SOLVE_SMEM = 3, SOLVE_SMEM_LDLT = 4,   // block_chol_solve_small, and its rank-revealing fallback
+    SOLVE_PANEL = 10,                      // + the stage count: chol_panel_major in 1 .. PM_MAX_STAGES stages
+    SOLVE_PACKED = 30,                     // chol_packed_smem
+    SOLVE_CLUSTER = 40                     // chol_blocked_cluster (the whole cluster; never from solve_on_rank0)
+};
+// Every solver except chol_blocked_cluster runs on rank 0 alone.
+__device__ __forceinline__ bool solved_on_rank0(const double *S, int nu, const FitSmem &sm)
+{
+    return S == sm.Ssm || (g_dbg_solver == 0 && nu < FIT_NT && pm_stage_count(nu, sm.arena_len) <= PM_MAX_STAGES) ||
+           packed_fits(nu, sm.arena_len);
+}
+// The solve of a bordered system (nu unknowns) at S when solved_on_rank0(): x -> sm.rhs.  Run by every thread of rank 0.
+__device__ __forceinline__ int solve_on_rank0(double *S, int lds, int nu, const FitSmem &sm_, PhaseTimer &pt, bool preloaded)
 {
     const FitSmem sm = sm_shared(sm_);
-    out = as_shared(out);
     if (S == sm.Ssm) {
-        if (cl.rank == 0 && nu <= 31 && g_dbg_solver == 0) {
+        if (nu <= 31 && g_dbg_solver == 0) {
             // one warp, rows in registers; S stays intact unless every pivot passes
             int *okf = reinterpret_cast<int *>(sm.red);
             __syncthreads();
@@ -1482,25 +1515,46 @@ __device__ void solve_broadcast(const ChainCtx &cx, Clu &cl, double *S, int lds,
                 for (int e = threadIdx.x; e < (nu + 1) * lds; e += FIT_NT) S0[e] = S[e];
                 __syncthreads();
                 ldlt_pivoted_small(S, lds, nu, sm.rhs, S0, sm.tile);
+                return SOLVE_WARP_LDLT;
             }
-        } else if (cl.rank == 0) {
-            // pristine copy (the scratch region is free here): the pivot test of the factorisation compares against it,
-            // and a rank-deficient system is solved again from it by the rank-revealing fallback
-            double *S0 = sm.scratch;
-            __syncthreads();
-            for (int e = threadIdx.x; e < (nu + 1) * lds; e += FIT_NT) S0[e] = S[e];
-            __syncthreads();
-            if (!block_chol_solve_small(S, lds, nu, sm.rhs, sm.dg, S0)) {
-                __syncthreads();
-                for (int e = threadIdx.x; e < (nu + 1) * lds; e += FIT_NT) S[e] = S0[e];
-                __syncthreads();
-                ldlt_pivoted_small(S, lds, nu, sm.rhs, S0, sm.tile);
-            }
+            return SOLVE_WARP;
         }
-    } else if (g_dbg_solver == 0 && nu < FIT_NT && pm_stage_count(nu, sm.arena_len) <= PM_MAX_STAGES) {
-        if (cl.rank == 0) chol_panel_major(S, lds, nu, sm.rhs, sm, cl.pt, preloaded);
-    } else if (packed_fits(nu, sm.arena_len)) {
-        if (cl.rank == 0) chol_packed_smem(S, lds, nu, sm.rhs, sm, cl.pt);
+        // pristine copy (the scratch region is free here): the pivot test of the factorisation compares against it,
+        // and a rank-deficient system is solved again from it by the rank-revealing fallback
+        double *S0 = sm.scratch;
+        __syncthreads();
+        for (int e = threadIdx.x; e < (nu + 1) * lds; e += FIT_NT) S0[e] = S[e];
+        __syncthreads();
+        if (!block_chol_solve_small(S, lds, nu, sm.rhs, sm.dg, S0)) {
+            __syncthreads();
+            for (int e = threadIdx.x; e < (nu + 1) * lds; e += FIT_NT) S[e] = S0[e];
+            __syncthreads();
+            ldlt_pivoted_small(S, lds, nu, sm.rhs, S0, sm.tile);
+            return SOLVE_SMEM_LDLT;
+        }
+        return SOLVE_SMEM;
+    }
+    if (g_dbg_solver == 0 && nu < FIT_NT) {
+        const int ns = pm_stage_count(nu, sm.arena_len);
+        if (ns <= PM_MAX_STAGES) {
+            chol_panel_major(S, lds, nu, sm.rhs, sm, pt, preloaded);
+            return SOLVE_PANEL + ns;
+        }
+    }
+    chol_packed_smem(S, lds, nu, sm.rhs, sm, pt);
+    return SOLVE_PACKED;
+}
+
+// Rank 0 holds a bordered system (nu unknowns) at S -- its own shared memory (small systems) or the chain's global matrix
+// (large systems, then every CTA of the cluster takes part in the factorisation): solve it and hand the solution to
+// every CTA of the cluster (out: smem).
+__device__ void solve_broadcast(const ChainCtx &cx, Clu &cl, double *S, int lds, int nu, double *out, const FitSmem &sm_,
+                                bool preloaded = false)
+{
+    const FitSmem sm = sm_shared(sm_);
+    out = as_shared(out);
+    if (solved_on_rank0(S, nu, sm)) {
+        if (cl.rank == 0) solve_on_rank0(S, lds, nu, sm, cl.pt, preloaded);
     } else {
         chol_blocked_cluster(S, lds, nu, sm.rhs, sm, cl);
     }
@@ -2442,13 +2496,112 @@ void debug_gram(const double *V, int ldv, int nrows, int mm, const double *wt, d
     cudaFree(dV); cudaFree(dw); cudaFree(dS); cudaFree(dt);
 }
 
-long long debug_take_rankdef()
+// ---- production-placement probes (tests).  The solve probe places a bordered system where make_ctx puts it for a support
+// cap kcap -- in sm.Ssm at ld FIT_SMEM_MS when it has at most FIT_SMEM_MS rows, else in global memory at ldA = (kcap + 3) & ~1
+// with the arena of fit_smem_doubles(ldA, kcap) -- and solves it with solve_on_rank0, the code a CL = 1 fit runs.
+__global__ void __launch_bounds__(FIT_NT, 1)
+solve_path_probe_kernel(const double *Sin, int ldin, double *Sg, int ldA, int mm, double *xout, int *path, int smem_doubles)
+{
+    extern __shared__ __align__(128) unsigned char smem_raw[];
+    const FitSmem sm = carve_fit_smem(smem_raw, ldA, smem_doubles);
+    const bool small = mm + 1 <= FIT_SMEM_MS;
+    double *S = small ? sm.Ssm : Sg;
+    const int lds = small ? FIT_SMEM_MS : ldA;
+    for (int e = threadIdx.x; e < (mm + 1) * (mm + 1); e += FIT_NT) S[(size_t)(e / (mm + 1)) * lds + e % (mm + 1)] = Sin[(size_t)(e / (mm + 1)) * ldin + e % (mm + 1)];
+    __syncthreads();
+    PhaseTimer pt;
+    pt.start(false);
+    // a fit hands such a system to chol_blocked_cluster, which needs the whole cluster: reported, not solved
+    const bool rank0 = solved_on_rank0(S, mm, sm);
+    const int code = rank0 ? solve_on_rank0(S, lds, mm, sm, pt, false) : SOLVE_CLUSTER;
+    __syncthreads();
+    for (int a = threadIdx.x; a < mm; a += FIT_NT) xout[a] = rank0 ? sm.rhs[a] : __longlong_as_double(0x7ff8000000000000ll);
+    if (threadIdx.x == 0) *path = code;
+}
+static unsigned long long take_counter(const unsigned long long &sym)
 {
     unsigned long long v = 0ull, z = 0ull;
-    CUDA_CHECK(cudaMemcpyFromSymbol(&v, g_rankdef_count, sizeof(v)));
-    if (v) CUDA_CHECK(cudaMemcpyToSymbol(g_rankdef_count, &z, sizeof(z)));
-    return (long long)v;
+    CUDA_CHECK(cudaMemcpyFromSymbol(&v, sym, sizeof(v)));
+    if (v) CUDA_CHECK(cudaMemcpyToSymbol(sym, &z, sizeof(z)));
+    return v;
 }
+void debug_solve_path(const double *S, int lds, int mm, int kcap, double *x_out, int *path_out)
+{
+    const int ldA = (kcap + 3) & ~1;
+    if (mm < 1 || mm >= FIT_NT || mm > kcap + 1 || lds < mm + 1)
+        throw EngineError{"debug_solve_path: need 1 <= mm < 512, mm <= kcap + 1, lds >= mm + 1"};
+    const int smd = fit_smem_doubles(ldA, kcap);
+    double *dS, *dSg, *dx;
+    int *dp;
+    const size_t nb = sizeof(double) * (size_t)(mm + 1) * lds;
+    CUDA_CHECK(cudaMalloc(&dS, nb));
+    CUDA_CHECK(cudaMalloc(&dSg, sizeof(double) * (size_t)(mm + 1) * ldA));
+    CUDA_CHECK(cudaMalloc(&dx, sizeof(double) * mm));
+    CUDA_CHECK(cudaMalloc(&dp, sizeof(int)));
+    CUDA_CHECK(cudaMemcpy(dS, S, nb, cudaMemcpyHostToDevice));
+    const unsigned long long rd0 = take_counter(g_rankdef_count), ws0 = take_counter(g_wide_singular_count);
+    CUDA_CHECK(cudaFuncSetAttribute(solve_path_probe_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smd * 8));
+    solve_path_probe_kernel<<<1, FIT_NT, (size_t)smd * 8>>>(dS, lds, dSg, ldA, mm, dx, dp, smd);
+    CUDA_CHECK(cudaGetLastError());
+    CUDA_CHECK(cudaDeviceSynchronize());
+    CUDA_CHECK(cudaMemcpy(x_out, dx, sizeof(double) * mm, cudaMemcpyDeviceToHost));
+    CUDA_CHECK(cudaMemcpy(path_out, dp, sizeof(int), cudaMemcpyDeviceToHost));
+    path_out[1] = (int)take_counter(g_rankdef_count);
+    path_out[2] = (int)take_counter(g_wide_singular_count);
+    // give back what a fit running before the probe had counted
+    if (rd0) CUDA_CHECK(cudaMemcpyToSymbol(g_rankdef_count, &rd0, sizeof(rd0)));
+    if (ws0) CUDA_CHECK(cudaMemcpyToSymbol(g_wide_singular_count, &ws0, sizeof(ws0)));
+    cudaFree(dS); cudaFree(dSg); cudaFree(dx); cudaFree(dp);
+}
+
+// The Gram probe over the rows [r0, r1) of V (r0 > 0: a cluster's row slice), wt may be null.  The output lands where
+// gram_solve puts it: in sm.Ssm at ld FIT_SMEM_MS when mm <= FIT_SMEM_MS (the DMMA ring then shares the arena with it),
+// else in global memory at ld ldv; the arena is fit_smem_doubles(ldv, kcap).  S_io (ldo x ldo, ldo = FIT_SMEM_MS or ldv)
+// is loaded as the output region's initial contents and read back whole, so stray writes show.
+__global__ void __launch_bounds__(FIT_NT, 1)
+gram_rows_probe_kernel(const double *V, int ldv, int r0, int r1, int mm, const double *wt, double *Sg, int impl, int smem_doubles)
+{
+    extern __shared__ __align__(128) unsigned char smem_raw[];
+    const FitSmem sm = carve_fit_smem(smem_raw, ldv, smem_doubles);
+    const bool small = mm <= FIT_SMEM_MS;
+    double *S = small ? sm.Ssm : Sg;
+    const int lds = small ? FIT_SMEM_MS : ldv;
+    if (small)
+        for (int e = threadIdx.x; e < FIT_SMEM_MS * FIT_SMEM_MS; e += FIT_NT) S[e] = Sg[e];
+    __syncthreads();
+    if (impl == 1) block_syrk(V, ldv, r0, r1, mm, wt, S, lds, sm);
+    else if (impl == 2) block_syrk_dmma(V, ldv, r0, r1, mm, wt, S, lds, sm);
+    else gram(V, ldv, r0, r1, mm, wt, S, lds, sm);
+    __syncthreads();
+    if (small)
+        for (int e = threadIdx.x; e < FIT_SMEM_MS * FIT_SMEM_MS; e += FIT_NT) Sg[e] = S[e];
+}
+void debug_gram_rows(const double *V, int ldv, int r0, int r1, int mm, const double *wt, double *S_io, int kcap, int impl)
+{
+    if (mm < 1 || mm > ldv || (ldv & 1) || r0 < 0 || r1 <= r0 || mm > kcap + 2 || impl < 0 || impl > 2)
+        throw EngineError{"debug_gram_rows: need 1 <= mm <= min(ldv, kcap + 2), even ldv, 0 <= r0 < r1, impl 0..2"};
+    const int smd = fit_smem_doubles(ldv, kcap);
+    const int ldo = mm <= FIT_SMEM_MS ? FIT_SMEM_MS : ldv;
+    double *dV, *dw = nullptr, *dS;
+    CUDA_CHECK(cudaMalloc(&dV, sizeof(double) * (size_t)r1 * ldv));
+    CUDA_CHECK(cudaMalloc(&dS, sizeof(double) * (size_t)ldo * ldo));
+    CUDA_CHECK(cudaMemcpy(dV, V, sizeof(double) * (size_t)r1 * ldv, cudaMemcpyHostToDevice));
+    if (wt) {
+        CUDA_CHECK(cudaMalloc(&dw, sizeof(double) * r1));
+        CUDA_CHECK(cudaMemcpy(dw, wt, sizeof(double) * r1, cudaMemcpyHostToDevice));
+    }
+    CUDA_CHECK(cudaMemcpy(dS, S_io, sizeof(double) * (size_t)ldo * ldo, cudaMemcpyHostToDevice));
+    CUDA_CHECK(cudaFuncSetAttribute(gram_rows_probe_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smd * 8));
+    gram_rows_probe_kernel<<<1, FIT_NT, (size_t)smd * 8>>>(dV, ldv, r0, r1, mm, dw, dS, impl, smd);
+    CUDA_CHECK(cudaGetLastError());
+    CUDA_CHECK(cudaDeviceSynchronize());
+    CUDA_CHECK(cudaMemcpy(S_io, dS, sizeof(double) * (size_t)ldo * ldo, cudaMemcpyDeviceToHost));
+    cudaFree(dV); cudaFree(dS);
+    if (dw) cudaFree(dw);
+}
+
+long long debug_take_rankdef() { return (long long)take_counter(g_rankdef_count); }
+long long take_wide_singular() { return (long long)take_counter(g_wide_singular_count); }
 
 void debug_set(int key, int val)
 {

@@ -867,6 +867,7 @@ void Engine::begin_load(int n, int p, int family)
 {
     Impl &m = *d_;
     if (n < 2 || p < 1) throw EngineError{"load: need n >= 2 and p >= 1"};
+    stats_.max_cluster = 0;
     if (family < 1 || family > 4) throw EngineError{"load: model_type must be 1..4"};
     if (sharded_) {
         long long lo, hi;
@@ -1923,6 +1924,7 @@ int Engine::run_batch_enqueue(int T, const std::vector<int> &chains, bool new_pa
     b.T = T;
     b.new_path_step = new_path_step ? 1 : 0;
     b.CL = chain_cluster_size(d, d.grouped ? std::min(d.kcap, T * d.gmax) : T, m.cl_chains > 0 ? std::max(m.cl_chains, b.nch) : b.nch);
+    stats_.max_cluster = std::max(stats_.max_cluster, b.CL);
     t.cmin = MAXC;
     t.cmax = -1;
     for (int i = 0; i < b.nch; i++) {

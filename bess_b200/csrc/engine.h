@@ -52,6 +52,8 @@ struct EngineStats {
     long long n_fits = 0, n_pdas_iters = 0, n_sweeps = 0, n_batches = 0, n_boundary_ties = 0;
     long long n_suspect_pivots = 0;   // resident path: fits whose Cholesky met a (numerically) dependent column
     long long n_rank_deficient = 0;   // multi-kernel path: normal-equation solves truncated by the rank-revealing fallback
+    long long n_wide_singular = 0;    // multi-kernel path: singular systems of more than 63 unknowns (no truncating solver)
+    int max_cluster = 0;              // largest cluster size of a chain_fit_kernel launch since load
     double sweep_bytes = 0.0;     // algorithmic bytes of the PDAS dual sweeps (8*n*p per launch + vectors)
     double big_sweep_bytes = 0.0; // algorithmic bytes of the screening sweep(s) over the raw design (8*n*p each)
     double norm_bytes = 0.0;      // algorithmic bytes of the normalisation / x_j.x_j passes

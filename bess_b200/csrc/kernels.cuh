@@ -202,9 +202,14 @@ void debug_set(int key, int val);
 void debug_get(unsigned long long *out32);
 // truncated (rank-deficient) normal-equation solves of the chain kernels since the last call (synchronises the device)
 long long debug_take_rankdef();
+// singular normal-equation systems of more than 63 unknowns (solution returned as NaN) since the last call
+long long take_wide_singular();
 void debug_solve(const double *S, int lds, int mm, double *x_out, int impl, int reps, double *ticks_out);
 void debug_gram(const double *V, int ldv, int nrows, int mm, const double *wt, double *S_out, int impl, int reps,
                 double *ticks_out);
+// path_out[0] = solver that finished (chain_fit.cu SOLVE_*), [1] = truncated solves, [2] = wide singular solves
+void debug_solve_path(const double *S, int lds, int mm, int kcap, double *x_out, int *path_out);
+void debug_gram_rows(const double *V, int ldv, int r0, int r1, int mm, const double *wt, double *S_io, int kcap, int impl);
 
 
 }  // namespace bess

@@ -902,6 +902,7 @@ static void bess_run_once(const BessArgs &a, BessResult &out, bool tie_exact)
         for (int &j : A) j = orig(j);
     out.stats = eng.stats();
     out.stats.n_rank_deficient += debug_take_rankdef();
+    out.stats.n_wide_singular += take_wide_singular();
     eng.profile(out.prof_ms, out.prof_n);
     out.sweep_splits = eng.sweep_splits();
     eng.resident_counters(out.resident);
@@ -924,9 +925,18 @@ void bess_run(const BessArgs &a, BessResult &out)
     // start): the resident kernel flags it (its plain Cholesky has no answer), and a non-finite result says the same of a
     // wide system.  The exact mode runs on the multi-kernel path, whose small-system solver falls back to a rank-revealing
     // LDL^T that truncates like the reference's colPivHouseholderQr / pivoted ldlt (chain_fit.cu: ldlt_pivoted_small).
-    bool finite = std::isfinite(out.train_loss) && std::isfinite(out.ic) && std::isfinite(out.coef0);
-    for (double v : out.beta_val) finite = finite && std::isfinite(v);
-    const bool suspect = out.stats.n_suspect_pivots > 0 || !finite;
+    // Its wide-system solver (more than 63 unknowns, e.g. a sparsity level above the number of training rows) has no such
+    // fallback: it returns NaN and counts the system, and any level of the path -- chosen or not -- may carry it.
+    auto all_finite = [](const std::vector<double> &v) {
+        for (double x : v)
+            if (!std::isfinite(x)) return false;
+        return true;
+    };
+    auto finite_result = [&](const BessResult &r) {
+        bool f = std::isfinite(r.train_loss) && std::isfinite(r.ic) && std::isfinite(r.coef0);
+        return f && all_finite(r.beta_val) && all_finite(r.ic_all) && all_finite(r.train_loss_all);
+    };
+    const bool suspect = out.stats.n_suspect_pivots > 0 || out.stats.n_wide_singular > 0 || !finite_result(out);
     if (redo && (out.stats.n_boundary_ties > 0 || suspect) && a.world <= 1) {
         const bool ties = out.stats.n_boundary_ties > 0;
         BessResult exact;
@@ -935,6 +945,11 @@ void bess_run(const BessArgs &a, BessResult &out)
         out.tie_exact_pass = ties;
         out.robust_pass = suspect;
     }
+    if (out.stats.n_wide_singular > 0)
+        throw EngineError{"rank-deficient wide system: the normal equations of a support with more than 63 unknowns are "
+                          "singular (is the sparsity level above the number of training rows?); only systems of up to 63 "
+                          "unknowns are solved rank-revealingly"};
+    if (!finite_result(out)) throw EngineError{"non-finite criterion, loss or coefficient on the path"};
 }
 
 }  // namespace bess

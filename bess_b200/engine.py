@@ -145,7 +145,8 @@ class GpuEngine:
         o = np.zeros(8)
         _lib.check(self._lib.bessgpu_stats(self._h, _d(o)))
         return dict(n_fits=int(o[0]), n_pdas_iters=int(o[1]), n_sweeps=int(o[2]), n_batches=int(o[3]),
-                    n_boundary_ties=int(o[4]), sweep_bytes=float(o[5]), kernel_launches=int(o[6]))
+                    n_boundary_ties=int(o[4]), sweep_bytes=float(o[5]), kernel_launches=int(o[6]),
+                    max_cluster=int(o[7]))
 
 
 def topk(vals, k):
