@@ -68,6 +68,7 @@ def load():
     lib.bessgpu_gather_columns.argtypes = [C.c_void_p, ip, ip, C.c_int, C.c_void_p, C.c_longlong]
     lib.bessgpu_normalize.argtypes = [C.c_void_p, C.c_int, C.c_int]
     lib.bessgpu_get_norm.argtypes = [C.c_void_p, dp, dp, dp]
+    lib.bessgpu_design.argtypes = [C.c_void_p, dp]
     lib.bessgpu_set_groups.argtypes = [C.c_void_p, ip, C.c_int]
     lib.bessgpu_run_batch_groups.argtypes = [C.c_void_p, C.c_int, ip, C.c_int, C.c_int, C.c_double, ip, dp, ip, ip, dp,
                                              C.c_int]
@@ -77,6 +78,7 @@ def load():
     lib.bessgpu_time_dual_sweep.argtypes = [C.c_void_p, C.c_int, C.POINTER(C.c_float), dp]
     lib.bessgpu_stats.argtypes = [C.c_void_p, dp]
     lib.bessgpu_topk.argtypes = [dp, C.c_int, C.c_int, ip, ip]
+    lib.bessgpu_screen_select.argtypes = [dp, C.c_int, C.c_int, ip, ip]
     lib.bess_b200_shard_range.restype = None
     lib.bess_b200_shard_range.argtypes = [C.c_longlong, C.c_int, C.c_int, C.POINTER(C.c_longlong),
                                           C.POINTER(C.c_longlong)]

@@ -373,6 +373,10 @@ int bessgpu_normalize(bessgpu_handle *h, int data_type, int is_normal)
 {
     return guarded([&] { h->eng->normalize(data_type, is_normal != 0); });
 }
+int bessgpu_design(bessgpu_handle *h, double *x_out)
+{
+    return guarded([&] { h->eng->copy_design(x_out); });
+}
 int bessgpu_get_norm(bessgpu_handle *h, double *xm, double *xn, double *ym)
 {
     return guarded([&] {
@@ -466,6 +470,31 @@ int bessgpu_topk(const double *vals, int n, int k, int *idx_out, int *tie_out)
         ck(cudaMemcpy(idx_out, dout, (size_t)k * 4, cudaMemcpyDeviceToHost));
         if (tie_out) ck(cudaMemcpy(tie_out, dtie, 4, cudaMemcpyDeviceToHost));
         cudaFree(dv); cudaFree(ck0); cudaFree(ck1); cudaFree(ci0); cudaFree(ci1); cudaFree(dout); cudaFree(dtie);
+    });
+}
+
+int bessgpu_screen_select(const double *vals, int n, int k, int *idx_out, int *tie_out)
+{
+    return guarded([&] {
+        if (k < 1 || k > n) throw EngineError{"screen_select: need 1 <= k <= n"};
+        auto ck = [](cudaError_t e) { if (e != cudaSuccess) throw EngineError{cudaGetErrorString(e)}; };
+        configure_kernels();
+        double *dv = nullptr, *ck0 = nullptr, *ck1 = nullptr;
+        int *ci0 = nullptr, *ci1 = nullptr, *dout = nullptr, *dtie = nullptr;
+        void *scratch = nullptr;
+        const long long cs = std::max<long long>(2LL * k + 16, ((long long)n / 8192 + 2) * std::min(k, TOPK_LMAX));
+        ck(cudaMalloc(&dv, (size_t)n * 8));
+        ck(cudaMalloc(&ck0, (size_t)cs * 8)); ck(cudaMalloc(&ck1, (size_t)cs * 8));
+        ck(cudaMalloc(&ci0, (size_t)cs * 4)); ck(cudaMalloc(&ci1, (size_t)cs * 4));
+        ck(cudaMalloc(&dout, (size_t)k * 4)); ck(cudaMalloc(&dtie, 4));
+        ck(cudaMalloc(&scratch, screen_select_scratch_bytes(n)));
+        ck(cudaMemcpy(dv, vals, (size_t)n * 8, cudaMemcpyHostToDevice));
+        ck(cudaMemset(dtie, 0, 4));
+        launch_screen_select(dv, n, k, dout, dtie, scratch, ck0, ci0, ck1, ci1, cs, 0);
+        ck(cudaMemcpy(idx_out, dout, (size_t)k * 4, cudaMemcpyDeviceToHost));
+        if (tie_out) ck(cudaMemcpy(tie_out, dtie, 4, cudaMemcpyDeviceToHost));
+        cudaFree(dv); cudaFree(ck0); cudaFree(ck1); cudaFree(ci0); cudaFree(ci1); cudaFree(dout); cudaFree(dtie);
+        cudaFree(scratch);
     });
 }
 

@@ -483,6 +483,20 @@ struct Engine::Impl {
     int *h_sel_tie = nullptr;
     int sel_count = 0;
     bool sel_pending = false;
+    // screening's gather of the kept columns (dense, unsharded), deferred so that normalize() can fuse it into its one
+    // launch: X (the screened design, allocated but not yet written) <- gsrc[:, gsel].  gsel is the arena list of
+    // screen_select, alive until the next config_sweep; gsrc is the raw design, freed with the gather when owned.
+    const int *gsel = nullptr;
+    double *gsrc = nullptr;
+    long long gsrc_ld = 0;
+    bool gsrc_owned = false;
+    void drop_gather_source()
+    {
+        if (gsrc_owned) dfree(st, gsrc);
+        gsel = nullptr;
+        gsrc = nullptr;
+        gsrc_owned = false;
+    }
     double *h_mean = nullptr, *h_norm = nullptr;  // pinned: column statistics of the last normalisation
     bool stats_pending = false;
     bool stats_have_mean = false;
@@ -629,6 +643,7 @@ Engine::~Engine()
     for (cudaEvent_t e : m.pool) cudaEventDestroy(e);
     m.free_chain_buffers();
     m.free_sweep_buffers();
+    m.drop_gather_source();
     if (m.x_owned) dfree(m.st, m.X);
     m.free_csc();
     dfree(m.st, m.gidx); dfree(m.st, m.gsz); dfree(m.st, m.glist);
@@ -876,6 +891,7 @@ void Engine::begin_load(int n, int p, int family)
     }
     m.free_chain_buffers();
     m.free_sweep_buffers();
+    m.drop_gather_source();
     if (m.x_owned) dfree(m.st, m.X);
     m.free_csc();
     m.X = nullptr;
@@ -997,6 +1013,17 @@ void Engine::densify()
 static int *screen_select(Engine::Impl &m, EngineStats &st, int family, int size, const std::vector<int> &always_select,
                           std::vector<double> *vals_out, std::vector<int> *sel_out, bool to_pinned);
 
+// The deferred gather of screen_enqueue, for every reader of X other than normalize()'s fused launch
+static void materialise_gather(Engine::Impl &m, EngineStats &st)
+{
+    if (!m.gsel) return;
+    const int sp = m.span_begin(5);
+    launch_gather_cols(m.gsrc, m.gsrc_ld, m.n, m.gsel, m.p, m.X, m.ldx, m.st);
+    m.span_end(sp);
+    st.kernel_launches += 1;
+    m.drop_gather_source();
+}
+
 std::vector<int> Engine::screen(int size, const std::vector<int> &always_select)
 {
     screen_enqueue(size, always_select);
@@ -1020,6 +1047,7 @@ void Engine::screen_enqueue(int size, const std::vector<int> &always_select)
 {
     Impl &m = *d_;
     if (size < 1 || size > p_model()) throw EngineError{"screening_size must be in [1, p]"};
+    materialise_gather(m, stats_);  // a second screening reads the first one's kept columns
     const long long ldn = (size + 1) & ~1LL;
     double *Xn = dalloc<double>(m.st, (size_t)m.n * ldn);
     if (ldn != size || m.csc) CUDA_CHECK(cudaMemsetAsync(Xn, 0, (size_t)m.n * ldn * 8, m.st));
@@ -1029,12 +1057,20 @@ void Engine::screen_enqueue(int size, const std::vector<int> &always_select)
     m.sel_count = size;
     if (!sharded_) {
         const int *d_sel = screen_select(m, stats_, family_, size, always_select, nullptr, nullptr, /*to_pinned=*/true);
-        // X <- X[:, sel]  (screening.cpp:83-88)
-        const int spk = m.span_begin(5);
-        if (m.csc) launch_csc_densify(m.cp, m.ri, m.cv, d_sel, size, Xn, ldn, m.st);
-        else launch_gather_cols(m.X, m.ldx, m.n, d_sel, size, Xn, ldn, m.st);
-        m.span_end(spk);
-        stats_.kernel_launches += 1;
+        // X <- X[:, sel]  (screening.cpp:83-88).  A dense design's gather waits for normalize(), which fuses it into its
+        // one launch, or for the first other reader of X (materialise_gather).
+        if (m.csc) {
+            const int spk = m.span_begin(5);
+            launch_csc_densify(m.cp, m.ri, m.cv, d_sel, size, Xn, ldn, m.st);
+            m.span_end(spk);
+            stats_.kernel_launches += 1;
+        } else {
+            m.gsel = d_sel;
+            m.gsrc = m.X;
+            m.gsrc_ld = m.ldx;
+            m.gsrc_owned = m.x_owned;
+            m.x_owned = false;  // ownership of the raw design moved to the pending gather
+        }
         m.sel_pending = true;  // the index list and the tie flag are on their way to the pinned block
     } else {
         // Column-sharded screening (SURVEY 8e axis B): marginal utilities of the local columns, exact local top-`size`,
@@ -1093,6 +1129,7 @@ void Engine::screen_local(int size, const std::vector<int> &always_select, std::
 {
     Impl &m = *d_;
     size = std::min(size, m.p);
+    materialise_gather(m, stats_);
     screen_select(m, stats_, family_, size, always_select, &vals, &idx, /*to_pinned=*/false);
     m.free_sweep_buffers();
 }
@@ -1103,6 +1140,7 @@ void Engine::gather_columns(const int *cols, const int *pos, int mcols, double *
     Impl &m = *d_;
     if (m.csc) throw EngineError{"gather_columns: the design is sparse"};
     if (mcols <= 0) return;
+    materialise_gather(m, stats_);
     int *d_cols = dalloc<int>(m.st, mcols), *d_pos = dalloc<int>(m.st, mcols);
     CUDA_CHECK(cudaMemcpyAsync(d_cols, cols, (size_t)mcols * 4, cudaMemcpyHostToDevice, m.st));
     CUDA_CHECK(cudaMemcpyAsync(d_pos, pos, (size_t)mcols * 4, cudaMemcpyHostToDevice, m.st));
@@ -1168,10 +1206,10 @@ static int *screen_select(Engine::Impl &m, EngineStats &stats_, int family_, int
     double *ck0 = ar.alloc<double>((size_t)cstride), *ck1 = ar.alloc<double>((size_t)cstride);
     int *ci0 = ar.alloc<int>((size_t)cstride), *ci1 = ar.alloc<int>((size_t)cstride);
     int *d_tie = ar.alloc<int>(1);
+    void *scratch = ar.alloc<unsigned char>(screen_select_scratch_bytes(m.p));
     const int spk = m.span_begin(3);
-    launch_topk(m.d.bd, m.d.pstride, m.p, size, 1, d_sel, size, d_tie, ck0, ci0, ck1, ci1, cstride, m.st);
+    stats_.kernel_launches += launch_screen_select(m.d.bd, m.p, size, d_sel, d_tie, scratch, ck0, ci0, ck1, ci1, cstride, m.st);
     m.span_end(spk);
-    stats_.kernel_launches += 2;
     if (m.tie_exact && !m.d.sharded) {
         int tie = 0;
         CUDA_CHECK(cudaMemcpyAsync(&tie, d_tie, 4, cudaMemcpyDeviceToHost, m.st));
@@ -1208,12 +1246,32 @@ static int *screen_select(Engine::Impl &m, EngineStats &stats_, int family_, int
     return d_sel;
 }
 
+void Engine::copy_design(double *host_out)
+{
+    Impl &m = *d_;
+    if (m.csc) throw EngineError{"copy_design: the design is sparse"};
+    if (!m.X) throw EngineError{"copy_design: no design is loaded"};
+    materialise_gather(m, stats_);
+    CUDA_CHECK(cudaMemcpy2DAsync(host_out, (size_t)m.p * 8, m.X, (size_t)m.ldx * 8, (size_t)m.p * 8, m.n,
+                                 cudaMemcpyDeviceToHost, m.st));
+    CUDA_CHECK(cudaStreamSynchronize(m.st));
+}
+
 // Data ctor (Data.h:41-68) + normalize.cpp + add_weight (Data.h:70-77, bess.cpp:97)
 void Engine::normalize(int data_type, bool is_normal)
 {
     Impl &m = *d_;
     if (m.csc) throw EngineError{"normalize: a sparse design must be screened or densified first"};
     const int n = m.n, p = m.p;
+    // ---- a design that fits L2 (after screening: config 5's 40 MB): the whole normalisation is ONE launch, which also
+    // gathers the kept columns of a pending screening when their n x 8 slabs fit shared memory
+    static const bool one_launch = [] {
+        const char *e = std::getenv("BESS_B200_NORM_FUSED");
+        return !(e && e[0] == '0');
+    }();
+    const bool resident = one_launch && is_normal && !sharded_ && (size_t)n * m.ldx * 8 <= ((size_t)64 << 20);
+    const bool fuse_gather = resident && m.gsel && n <= NR_SLAB_ROWS;
+    if (!fuse_gather) materialise_gather(m, stats_);
     if (!m.x_owned) {  // normalisation is in place: take a private copy of a borrowed design
         double *Xc = dalloc<double>(m.st, (size_t)n * m.ldx);
         CUDA_CHECK(cudaMemcpyAsync(Xc, m.X, (size_t)n * m.ldx * 8, cudaMemcpyDeviceToDevice, m.st));
@@ -1223,12 +1281,7 @@ void Engine::normalize(int data_type, bool is_normal)
     DevArena &ar = m.ctx->ar;
     m.stats_have_mean = false;
     m.stats_pending = false;
-    // ---- a design that fits L2 (after screening: config 5's 40 MB): the whole normalisation is ONE launch
-    static const bool one_launch = [] {
-        const char *e = std::getenv("BESS_B200_NORM_FUSED");
-        return !(e && e[0] == '0');
-    }();
-    if (one_launch && is_normal && !sharded_ && (size_t)n * m.ldx * 8 <= ((size_t)64 << 20)) {
+    if (resident) {
         const int sp = m.span_begin(6);
         m.h_mean = m.ctx->rb.alloc<double>((size_t)p);
         m.h_norm = m.ctx->rb.alloc<double>((size_t)p);
@@ -1254,14 +1307,21 @@ void Engine::normalize(int data_type, bool is_normal)
         m.y = m.stage_vec(m.hy.data(), (size_t)n, (size_t)m.npad);  // the response as the fits see it
         m.ctx->mir.flush(m.st);
         double *d_mean = ar.alloc<double>((size_t)p + 2), *d_norm = ar.alloc<double>((size_t)p + 2);
-        launch_normalize_resident(m.X, m.ldx, n, p, d_g, d_w, d_rm, std::sqrt((double)n), d_mean, d_norm, m.st);
+        if (fuse_gather) {
+            launch_gather_normalize(m.gsrc, m.gsrc_ld, m.gsel, m.X, m.ldx, n, p, d_g, d_w, d_rm, std::sqrt((double)n), d_mean,
+                                    d_norm, m.st);
+            m.drop_gather_source();  // stream-ordered: an owned raw design lives until the launch above is done
+            stats_.norm_bytes += 16.0 * n * p;  // one read of the kept elements (each its own sector) and one write
+        } else {
+            launch_normalize_resident(m.X, m.ldx, n, p, d_g, d_w, d_rm, std::sqrt((double)n), d_mean, d_norm, m.st);
+            stats_.norm_bytes += 32.0 * n * p;  // three reads and one write of X
+        }
         if (centre) CUDA_CHECK(cudaMemcpyAsync(m.h_mean, d_mean, (size_t)p * 8, cudaMemcpyDeviceToHost, m.st));
         CUDA_CHECK(cudaMemcpyAsync(m.h_norm, d_norm, (size_t)p * 8, cudaMemcpyDeviceToHost, m.st));
         m.stats_have_mean = centre;
         m.stats_pending = true;
         m.span_end(sp);
         stats_.kernel_launches += 1;
-        stats_.norm_bytes += 32.0 * n * p;  // three reads and one write of X
         h_xmean_.clear();
         h_xnorm_.clear();
         return;
@@ -1438,6 +1498,7 @@ void Engine::setup_chains(int K, const int *fold_of_row, int kcap, int max_iter,
     m.K = K;
     m.nchains = 1 + K;
     const int C = m.nchains;
+    materialise_gather(m, stats_);
     m.config_sweep(pick_fs(C));
     DevArena &ar = m.ctx->ar;
     MirrorArena &mir = m.ctx->mir;

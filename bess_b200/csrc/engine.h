@@ -131,6 +131,8 @@ public:
 
     // ---- Data ctor normalisation (Data.h:41-68, normalize.cpp) + add_weight for gaussian (Data.h:70-77).
     void normalize(int data_type, bool is_normal);
+    // the current dense design (n x p_model(), row-major, without the row padding) -> host; waits for the device
+    void copy_design(double *host_out);
 
     // ---- group selection (R: group.index, Python: GroupPdas*).  g_index: first column of every group, ascending from 0
     // (Data.h:53-61); call after normalize() and before setup_chains().  From then on sparsity levels, top-k results and

@@ -419,20 +419,17 @@ __device__ __forceinline__ unsigned long long topk_key(double v)
     return u;
 }
 
-// Select + ordered compaction over `len` keys already in shared memory (block-synchronised by the caller's first barrier
-// inside).  Outputs as in topk_slices_kernel.
-__device__ __forceinline__ void topk_body(unsigned long long *keys, int len, int k, int slice_len, const int *iin, int b0, int s,
-                                          int f, double *keys_out, int *idx_out, long long out_stride, int *final_out,
-                                          int final_ld, int *tie)
+// The select half of topk_body over `len` keys already in shared memory (block-synchronised by its first barrier):
+// every key > thr is taken, plus the first krem keys equal to thr; neq keys equal thr (a boundary tie when neq > krem).
+// Block-wide: every thread returns the same values.  blockDim = TOPK_NT.
+__device__ __forceinline__ void topk_threshold(const unsigned long long *keys, int len, int kk, unsigned long long &thr_out,
+                                               int &krem_out, int &neq_out)
 {
     __shared__ int hist[256];
     __shared__ unsigned long long sh_prefix;
     __shared__ int sh_krem, sh_neq, sh_cnt;
-    __shared__ unsigned long long scan_sh[34];
     __shared__ unsigned long long small_bin[32];
     const int tid = threadIdx.x;
-    const int kk = min(k, len);
-    const int out_per_slice = min(k, slice_len);
     unsigned long long thr = 0ull;
     int krem = kk, neq = len;
     if (kk < len) {
@@ -531,6 +528,24 @@ __device__ __forceinline__ void topk_body(unsigned long long *keys, int len, int
     } else {
         __syncthreads();
     }
+    thr_out = thr;
+    krem_out = krem;
+    neq_out = neq;
+}
+
+// Select + ordered compaction over `len` keys already in shared memory (block-synchronised by the caller's first barrier
+// inside).  Outputs as in topk_slices_kernel.
+__device__ __forceinline__ void topk_body(unsigned long long *keys, int len, int k, int slice_len, const int *iin, int b0, int s,
+                                          int f, double *keys_out, int *idx_out, long long out_stride, int *final_out,
+                                          int final_ld, int *tie)
+{
+    __shared__ unsigned long long scan_sh[34];
+    const int tid = threadIdx.x;
+    const int kk = min(k, len);
+    const int out_per_slice = min(k, slice_len);
+    unsigned long long thr;
+    int krem, neq;
+    topk_threshold(keys, len, kk, thr, krem, neq);
     // ordered compaction.  thread owns a contiguous chunk.
     const int per = (len + TOPK_NT - 1) / TOPK_NT;
     const int cb = min(len, tid * per), ce = min(len, cb + per);
@@ -671,9 +686,9 @@ void launch_topk_fused(const Dev &d, int mode, int epi, int cmin, int nspan, int
     CUDA_CHECK(cudaGetLastError());
 }
 
-void launch_topk(const double *vals, long long stride, int n_in, int k, int nch, int *out_idx, int out_ld, int *tie,
-                 double *ck0, int *ci0, double *ck1, int *ci1, long long cstride, cudaStream_t st, const int *gate,
-                 const int *idx0)
+int launch_topk(const double *vals, long long stride, int n_in, int k, int nch, int *out_idx, int out_ld, int *tie,
+                double *ck0, int *ci0, double *ck1, int *ci1, long long cstride, cudaStream_t st, const int *gate,
+                const int *idx0)
 {
     if (k > n_in) throw EngineError{"top-k: k > number of candidates"};
     const double *kin = vals;
@@ -688,7 +703,7 @@ void launch_topk(const double *vals, long long stride, int n_in, int k, int nch,
             topk_slices_kernel<<<grid, TOPK_NT, smem, st>>>(kin, iin, in_stride, cur_n, k, cur_n, nullptr, nullptr, 0,
                                                             out_idx, out_ld, tie, gate);
             CUDA_CHECK(cudaGetLastError());
-            return;
+            return guard + 1;
         }
         // slice length: keep >= ~600 CTAs busy but never so short that nothing is filtered
         int slice = 8192;
@@ -717,6 +732,252 @@ void launch_topk(const double *vals, long long stride, int n_in, int k, int nch,
         pp ^= 1;
     }
     throw EngineError{"top-k: did not converge"};
+}
+
+// =====================================================================================================
+// device-wide exact select of the screening list (p > TOPK_LMAX): the same list, order and tie flag as launch_topk
+// =====================================================================================================
+// launch_topk at p = 500 000, k = 5000 is four dependent stages of 31, 10, 4 and 1 CTAs, each an 8-pass radix select in one
+// CTA's shared memory: latency-bound with most SMs idle.  Here every pass spreads over the machine:
+//   ss_hist_kernel (pass 0)  histogram of the top 12 key bits (sign + exponent); the last CTA finds the boundary bin
+//   ss_hist_kernel (pass 1)  histogram of the next 12 bits inside that bin; the last CTA finds the boundary sub-bin
+//   ss_collect_kernel        the keys of the boundary sub-bin -> scratch (at most TOPK_LMAX, else the fallback flag)
+//   ss_resolve_kernel        one CTA: topk_threshold over them -> thr, krem (keys == thr taken), the tie flag
+//   ss_count_kernel          per-chunk counts of (key > thr, key == thr)
+//   ss_write_kernel          chunk base by summing the counts before it, block scan, ordered compaction (ascending)
+// A boundary sub-bin larger than TOPK_LMAX (all-zero or massively tied utilities) sets the fallback flag: the kernels above
+// stop and launch_topk, enqueued behind them and gated on that flag, decides -- no host round trip.
+constexpr int SS_NT = 512;
+constexpr int SS_BINS = 4096;        // 12-bit digits
+constexpr int SS_CHUNK = SS_NT * 8;  // keys per CTA of the ordered compaction
+struct SsState {                     // zeroed before every select
+    int hist[2][SS_BINS];
+    int done[2];
+    int bin[2];    // boundary digit of pass 0 / pass 1
+    int above[2];  // keys above the boundary bin / sub-bin
+    int fallback;
+    int ncand;
+    int krem, neq;
+    unsigned long long thr;
+};
+
+__global__ void __launch_bounds__(SS_NT) ss_hist_kernel(const double *__restrict__ vals, int p, int k, int pass, SsState *s)
+{
+    __shared__ int h[SS_BINS];
+    __shared__ int suf[SS_NT];
+    __shared__ bool last;
+    const int tid = threadIdx.x;
+    for (int i = tid; i < SS_BINS; i += SS_NT) h[i] = 0;
+    __syncthreads();
+    const int b0 = pass ? s->bin[0] : 0;
+    for (long long i = (long long)blockIdx.x * SS_NT + tid; i < p; i += (long long)gridDim.x * SS_NT) {
+        const unsigned long long u = topk_key(vals[i]);
+        if (pass == 0) atomicAdd(&h[(int)(u >> 52)], 1);
+        else if ((int)(u >> 52) == b0) atomicAdd(&h[(int)((u >> 40) & (SS_BINS - 1))], 1);
+    }
+    __syncthreads();
+    for (int i = tid; i < SS_BINS; i += SS_NT)
+        if (h[i]) atomicAdd(&s->hist[pass][i], h[i]);
+    __threadfence();
+    __syncthreads();
+    if (tid == 0) last = atomicAdd(&s->done[pass], 1) == (int)gridDim.x - 1;
+    __syncthreads();
+    if (!last) return;
+    __threadfence();
+    // the last CTA: the digit at which the count from the top reaches krem (thread t owns bins [8t, 8t + 8))
+    const int above0 = pass ? __ldcg(&s->above[0]) : 0;
+    const int krem = k - above0;
+    int loc[8], tot = 0;
+#pragma unroll
+    for (int q = 0; q < 8; q++) {
+        loc[q] = __ldcg(&s->hist[pass][tid * 8 + q]);
+        tot += loc[q];
+    }
+    suf[tid] = tot;
+    __syncthreads();
+    for (int o = 1; o < SS_NT; o <<= 1) {
+        const int v = tid + o < SS_NT ? suf[tid + o] : 0;
+        __syncthreads();
+        suf[tid] += v;
+        __syncthreads();
+    }
+    int acc = suf[tid] - tot;  // keys in the bins of higher threads
+    if (acc < krem && suf[tid] >= krem) {
+        for (int q = 7; q >= 0; q--) {
+            if (acc + loc[q] >= krem) {
+                s->bin[pass] = tid * 8 + q;
+                s->above[pass] = above0 + acc;
+                if (pass == 1) s->fallback = loc[q] > TOPK_LMAX;
+                break;
+            }
+            acc += loc[q];
+        }
+    }
+}
+
+__global__ void __launch_bounds__(SS_NT) ss_collect_kernel(const double *__restrict__ vals, int p, SsState *s,
+                                                           unsigned long long *cand)
+{
+    if (s->fallback) return;
+    const unsigned long long pb = ((unsigned long long)s->bin[0] << 12) | (unsigned long long)s->bin[1];  // key >> 40
+    for (long long i = (long long)blockIdx.x * SS_NT + threadIdx.x; i < p; i += (long long)gridDim.x * SS_NT) {
+        const unsigned long long u = topk_key(vals[i]);
+        if ((u >> 40) == pb) cand[atomicAdd(&s->ncand, 1)] = u;
+    }
+}
+
+__global__ void __launch_bounds__(TOPK_NT) ss_resolve_kernel(int k, SsState *s, const unsigned long long *cand, int *tie)
+{
+    extern __shared__ __align__(128) unsigned char smem_raw[];
+    unsigned long long *keys = reinterpret_cast<unsigned long long *>(smem_raw);
+    __shared__ unsigned long long mn;
+    __shared__ int cmin;
+    if (s->fallback) return;
+    const int tid = threadIdx.x;
+    const int nb = s->ncand;
+    const int krem = k - s->above[1];  // 1 <= krem <= nb
+    for (int i = tid; i < nb; i += TOPK_NT) keys[i] = cand[i];
+    unsigned long long thr;
+    int kr, neq;
+    if (krem < nb) {
+        topk_threshold(keys, nb, krem, thr, kr, neq);
+    } else {  // the whole sub-bin is taken: the threshold is its smallest key, and every copy of it is taken
+        if (tid == 0) { mn = ~0ull; cmin = 0; }
+        __syncthreads();
+        for (int i = tid; i < nb; i += TOPK_NT) atomicMin(&mn, keys[i]);
+        __syncthreads();
+        for (int i = tid; i < nb; i += TOPK_NT)
+            if (keys[i] == mn) atomicAdd(&cmin, 1);
+        __syncthreads();
+        thr = mn;
+        kr = neq = cmin;
+    }
+    if (tid == 0) {
+        s->thr = thr;
+        s->krem = kr;
+        s->neq = neq;
+        *tie = neq > kr ? 1 : 0;
+    }
+}
+
+// (key > thr, key == thr) packed as (gt << 32) | eq
+__device__ __forceinline__ unsigned long long ss_block_sum(unsigned long long v, unsigned long long *red)
+{
+    const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
+    if (lane == 0) red[wid] = v;
+    __syncthreads();
+    unsigned long long t = 0;
+    if (wid == 0) {
+        t = lane < SS_NT / 32 ? red[lane] : 0ull;
+#pragma unroll
+        for (int o = 16; o > 0; o >>= 1) t += __shfl_xor_sync(0xffffffffu, t, o);
+    }
+    return t;  // valid on thread 0
+}
+
+__global__ void __launch_bounds__(SS_NT) ss_count_kernel(const double *__restrict__ vals, int p, const SsState *s,
+                                                         unsigned long long *cnt)
+{
+    __shared__ unsigned long long red[SS_NT / 32];
+    if (s->fallback) return;
+    const unsigned long long thr = s->thr;
+    const long long c0 = (long long)blockIdx.x * SS_CHUNK;
+    unsigned long long c = 0;
+#pragma unroll
+    for (int q = 0; q < 8; q++) {
+        const long long i = c0 + q * SS_NT + threadIdx.x;
+        if (i < p) {
+            const unsigned long long u = topk_key(vals[i]);
+            c += (u > thr ? (1ull << 32) : 0ull) + (u == thr ? 1ull : 0ull);
+        }
+    }
+    const unsigned long long t = ss_block_sum(c, red);
+    if (threadIdx.x == 0) cnt[blockIdx.x] = t;
+}
+
+__global__ void __launch_bounds__(SS_NT) ss_write_kernel(const double *__restrict__ vals, int p, const SsState *s,
+                                                         const unsigned long long *cnt, int *out_idx)
+{
+    __shared__ unsigned long long red[SS_NT / 32];
+    __shared__ unsigned long long base_sh;
+    __shared__ unsigned long long scan_sh[SS_NT / 32];
+    if (s->fallback) return;
+    const unsigned long long thr = s->thr;
+    const int krem = s->krem;
+    const int tid = threadIdx.x, lane = tid & 31, wid = tid >> 5;
+    // counts of the chunks before this one
+    unsigned long long b = 0;
+    for (int q = tid; q < (int)blockIdx.x; q += SS_NT) b += cnt[q];
+    b = ss_block_sum(b, red);
+    if (tid == 0) base_sh = b;
+    // this thread's 8 contiguous keys
+    const long long i0 = (long long)blockIdx.x * SS_CHUNK + (long long)tid * 8;
+    unsigned long long u[8];
+    unsigned long long v = 0;
+#pragma unroll
+    for (int q = 0; q < 8; q++) {
+        u[q] = i0 + q < p ? topk_key(vals[i0 + q]) : 0ull;
+        if (i0 + q < p) v += (u[q] > thr ? (1ull << 32) : 0ull) + (u[q] == thr ? 1ull : 0ull);
+    }
+    // exclusive block scan of v
+    unsigned long long inc = v;
+#pragma unroll
+    for (int o = 1; o < 32; o <<= 1) {
+        const unsigned long long t = __shfl_up_sync(0xffffffffu, inc, o);
+        if (lane >= o) inc += t;
+    }
+    if (lane == 31) scan_sh[wid] = inc;
+    __syncthreads();
+    if (wid == 0) {
+        const unsigned long long w = lane < SS_NT / 32 ? scan_sh[lane] : 0ull;
+        unsigned long long winc = w;
+#pragma unroll
+        for (int o = 1; o < 32; o <<= 1) {
+            const unsigned long long t = __shfl_up_sync(0xffffffffu, winc, o);
+            if (lane >= o) winc += t;
+        }
+        if (lane < SS_NT / 32) scan_sh[lane] = winc - w;
+    }
+    __syncthreads();
+    const unsigned long long ex = base_sh + scan_sh[wid] + (inc - v);
+    int gt_before = (int)(ex >> 32), eq_before = (int)(ex & 0xffffffffull);
+#pragma unroll
+    for (int q = 0; q < 8; q++) {
+        if (i0 + q >= p) break;
+        const bool sel = u[q] > thr || (u[q] == thr && eq_before < krem);
+        if (sel) out_idx[gt_before + min(eq_before, krem)] = (int)(i0 + q);
+        gt_before += u[q] > thr;
+        eq_before += u[q] == thr;
+    }
+}
+
+size_t screen_select_scratch_bytes(int p)
+{
+    return sizeof(SsState) + (size_t)TOPK_LMAX * 8 + (size_t)((p + SS_CHUNK - 1) / SS_CHUNK) * 8;
+}
+
+int launch_screen_select(const double *vals, int p, int k, int *out_idx, int *tie, void *scratch, double *ck0, int *ci0,
+                         double *ck1, int *ci1, long long cstride, cudaStream_t st)
+{
+    if (k < 1 || k > p) throw EngineError{"screen select: need 1 <= k <= p"};
+    // one CTA holds every key (p <= TOPK_LMAX), or a k the fallback could not take: launch_topk as it is
+    if (p <= TOPK_LMAX || 2LL * k > TOPK_LMAX) return launch_topk(vals, p, p, k, 1, out_idx, k, tie, ck0, ci0, ck1, ci1, cstride, st);
+    SsState *s = static_cast<SsState *>(scratch);
+    unsigned long long *cand = reinterpret_cast<unsigned long long *>(s + 1);
+    unsigned long long *cnt = cand + TOPK_LMAX;
+    CUDA_CHECK(cudaMemsetAsync(s, 0, sizeof(SsState), st));
+    const int gh = (int)std::min<long long>(1184, ((long long)p + SS_NT * 8 - 1) / (SS_NT * 8));
+    const int nchunk = (p + SS_CHUNK - 1) / SS_CHUNK;
+    ss_hist_kernel<<<gh, SS_NT, 0, st>>>(vals, p, k, 0, s);
+    ss_hist_kernel<<<gh, SS_NT, 0, st>>>(vals, p, k, 1, s);
+    ss_collect_kernel<<<gh, SS_NT, 0, st>>>(vals, p, s, cand);
+    ss_resolve_kernel<<<1, TOPK_NT, (size_t)TOPK_LMAX * 8, st>>>(k, s, cand, tie);
+    ss_count_kernel<<<nchunk, SS_NT, 0, st>>>(vals, p, s, cnt);
+    ss_write_kernel<<<nchunk, SS_NT, 0, st>>>(vals, p, s, cnt, out_idx);
+    CUDA_CHECK(cudaGetLastError());
+    return 6 + launch_topk(vals, p, p, k, 1, out_idx, k, tie, ck0, ci0, ck1, ci1, cstride, st, &s->fallback);
 }
 
 // =====================================================================================================
@@ -803,9 +1064,15 @@ void launch_gather_owned_cols(const double *X, long long ldx, int n, int p_local
     CUDA_CHECK(cudaGetLastError());
 }
 
+__global__ void gather_normalize_kernel(const double *__restrict__ X, long long ldx, const int *__restrict__ cols, double *Xn,
+                                        long long ldn, int n, int p, const double *gmean, const double *wnorm,
+                                        const double *rowmul, double sn, double *mean_out, double *norm_out);
+
 void configure_kernels()
 {
     CUDA_CHECK(cudaFuncSetAttribute(topk_slices_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, TOPK_LMAX * 8));
+    CUDA_CHECK(cudaFuncSetAttribute(ss_resolve_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, TOPK_LMAX * 8));
+    CUDA_CHECK(cudaFuncSetAttribute(gather_normalize_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, NR_SLAB_ROWS * NR_TC * 8));
 }
 
 // =====================================================================================================
@@ -939,10 +1206,13 @@ void launch_norm_factors(const double *h, int p, double sn, double *norm_out, do
 // only the summation order of the two column sums differs from the sweep kernels (fixed: rows warp-strided, warps added
 // in order).  Replaces 7 launches and 6 passes over X by 1 launch and 4.
 constexpr int NR_NT = 256;
-constexpr int NR_TC = 8;  // columns per CTA: a warp load covers 4 rows x 64 bytes; p / 8 CTAs keep every SM streaming
-__global__ void __launch_bounds__(NR_NT) normalize_resident_kernel(double *X, long long ldx, int n, int p, const double *gmean,
-                                                                   const double *wnorm, const double *rowmul, double sn,
-                                                                   double *mean_out, double *norm_out)
+// The three passes over one tile of NR_TC columns; ld(i) reads element i of this thread's column (only called for live
+// columns and rows < n), st(i, v) writes it.  Shared by the in-place kernel (ld / st on X itself) and the gather-fused
+// kernel (ld from a shared-memory slab, st to Xn): the rows each thread sums, the shuffles, the order in which warps are
+// added and the per-element arithmetic are the same for both, so they agree bit for bit.
+template <class Ld, class St>
+__device__ __forceinline__ void normalize_tile(Ld ld, St st, int n, int p, const double *gmean, const double *wnorm,
+                                               const double *rowmul, double sn, double *mean_out, double *norm_out)
 {
     __shared__ double red[NR_NT / 32][NR_TC];
     __shared__ double cmean[NR_TC], cmul[NR_TC];
@@ -951,7 +1221,6 @@ __global__ void __launch_bounds__(NR_NT) normalize_resident_kernel(double *X, lo
     const int c = lane & (NR_TC - 1), rg = lane >> 3;
     const long long j = (long long)blockIdx.x * NR_TC + c;
     const bool live = j < p;
-    double *col = X + (live ? j : 0);
     const int ifirst = wid * 4 + rg;
     // column sum of f(x_i, i) over this thread's rows, 8 loads in flight; then lanes of the same column, then warps
     auto column_sum = [&](auto f) {
@@ -959,7 +1228,7 @@ __global__ void __launch_bounds__(NR_NT) normalize_resident_kernel(double *X, lo
         for (int i0 = ifirst; i0 < n; i0 += 8 * RS) {
             double v[8];
 #pragma unroll
-            for (int u = 0; u < 8; u++) v[u] = (live && i0 + u * RS < n) ? col[(size_t)(i0 + u * RS) * ldx] : 0.0;
+            for (int u = 0; u < 8; u++) v[u] = (live && i0 + u * RS < n) ? ld(i0 + u * RS) : 0.0;
 #pragma unroll
             for (int u = 0; u < 8; u++)
                 if (i0 + u * RS < n) s = f(v[u], i0 + u * RS, s);
@@ -1005,19 +1274,77 @@ __global__ void __launch_bounds__(NR_NT) normalize_resident_kernel(double *X, lo
     for (int i0 = ifirst; i0 < n; i0 += 8 * RS) {
         double v[8];
 #pragma unroll
-        for (int u = 0; u < 8; u++) v[u] = (live && i0 + u * RS < n) ? col[(size_t)(i0 + u * RS) * ldx] : 0.0;
+        for (int u = 0; u < 8; u++) v[u] = (live && i0 + u * RS < n) ? ld(i0 + u * RS) : 0.0;
 #pragma unroll
         for (int u = 0; u < 8; u++)
             if (live && i0 + u * RS < n) {
                 const double rm = rowmul ? rowmul[i0 + u * RS] : 1.0;
-                col[(size_t)(i0 + u * RS) * ldx] = (v[u] - mean) * mul * rm;
+                st(i0 + u * RS, (v[u] - mean) * mul * rm);
             }
     }
+}
+__global__ void __launch_bounds__(NR_NT) normalize_resident_kernel(double *X, long long ldx, int n, int p, const double *gmean,
+                                                                   const double *wnorm, const double *rowmul, double sn,
+                                                                   double *mean_out, double *norm_out)
+{
+    const long long j = (long long)blockIdx.x * NR_TC + (threadIdx.x & (NR_TC - 1));
+    double *col = X + (j < p ? j : 0);
+    normalize_tile([&](int i) { return col[(size_t)i * ldx]; }, [&](int i, double v) { col[(size_t)i * ldx] = v; }, n, p,
+                   gmean, wnorm, rowmul, sn, mean_out, norm_out);
 }
 void launch_normalize_resident(double *X, long long ldx, int n, int p, const double *gmean, const double *wnorm,
                                const double *rowmul, double sn, double *mean_out, double *norm_out, cudaStream_t st)
 {
     normalize_resident_kernel<<<(p + NR_TC - 1) / NR_TC, NR_NT, 0, st>>>(X, ldx, n, p, gmean, wnorm, rowmul, sn, mean_out, norm_out);
+    CUDA_CHECK(cudaGetLastError());
+}
+
+// Screening's gather fused into the one-launch normalisation: the CTA of tile b copies the n x NR_TC slab of its kept
+// columns cols[8b .. 8b+8) from the RAW design into shared memory, runs the three passes over the slab and writes Xn
+// once.  Every element is its own 32-byte sector of a multi-GB design, so the copy is latency-bound: it goes global ->
+// shared by cp.async, with no register round trip, and all n x 8 copies of the CTA are in flight at once.  The raw
+// sectors are read with an L2 evict-first policy so that they do not push the screened design, which the path reads
+// next, out of L2.  Replaces gather_cols (one write of Xn) + normalize_resident (three reads and one write of Xn).
+__global__ void __launch_bounds__(NR_NT) gather_normalize_kernel(const double *__restrict__ X, long long ldx,
+                                                                 const int *__restrict__ cols, double *Xn, long long ldn,
+                                                                 int n, int p, const double *gmean, const double *wnorm,
+                                                                 const double *rowmul, double sn, double *mean_out,
+                                                                 double *norm_out)
+{
+    extern __shared__ __align__(16) double slab[];  // [n][NR_TC]
+    {
+        constexpr int RR = NR_NT / NR_TC;  // rows per round of the copy
+        const int tc = threadIdx.x & (NR_TC - 1), tr = threadIdx.x / NR_TC;
+        const long long jt = (long long)blockIdx.x * NR_TC + tc;
+        if (jt < p) {
+            const double *src = X + cols[jt];
+            unsigned long long pol;
+            asm volatile("createpolicy.fractional.L2::evict_first.b64 %0, 1.0;" : "=l"(pol));
+            for (int i = tr; i < n; i += RR) {
+                const unsigned dst = (unsigned)__cvta_generic_to_shared(slab + i * NR_TC + tc);
+                asm volatile("cp.async.ca.shared.global.L2::cache_hint [%0], [%1], 8, %2;" ::"r"(dst),
+                             "l"(src + (size_t)i * ldx), "l"(pol)
+                             : "memory");
+            }
+            asm volatile("cp.async.wait_all;" ::: "memory");
+        } else {
+            for (int i = tr; i < n; i += RR) slab[i * NR_TC + tc] = 0.0;
+        }
+        __syncthreads();
+    }
+    const int c = threadIdx.x & (NR_TC - 1);
+    const long long j = (long long)blockIdx.x * NR_TC + c;
+    double *out = Xn + (j < p ? j : 0);
+    normalize_tile([&](int i) { return slab[i * NR_TC + c]; }, [&](int i, double v) { out[(size_t)i * ldn] = v; }, n, p,
+                   gmean, wnorm, rowmul, sn, mean_out, norm_out);
+}
+void launch_gather_normalize(const double *X, long long ldx, const int *cols, double *Xn, long long ldn, int n, int p,
+                             const double *gmean, const double *wnorm, const double *rowmul, double sn, double *mean_out,
+                             double *norm_out, cudaStream_t st)
+{
+    if (n > NR_SLAB_ROWS) throw EngineError{"gather_normalize: the n x 8 slab does not fit shared memory"};
+    gather_normalize_kernel<<<(p + NR_TC - 1) / NR_TC, NR_NT, (size_t)n * NR_TC * 8, st>>>(X, ldx, cols, Xn, ldn, n, p, gmean,
+                                                                                         wnorm, rowmul, sn, mean_out, norm_out);
     CUDA_CHECK(cudaGetLastError());
 }
 

@@ -12,6 +12,10 @@ constexpr int SWEEP_RC = 64;     // rows per TMA-staged chunk of the gradient ve
 constexpr int FIT_NT = 512;      // threads per chain_fit CTA (one CTA per chain)
 constexpr int TOPK_NT = 1024;
 constexpr int TOPK_LMAX = 16384; // keys per top-k slice held in shared memory (128 KB)
+// one-launch normalisation: columns per CTA (a warp load covers 4 rows x 64 bytes; p / 8 CTAs keep every SM streaming), and
+// the most rows whose n x NR_TC slab the gather-fused variant stages in shared memory (227 KB less 1 KB for its static arrays)
+constexpr int NR_TC = 8;
+constexpr int NR_SLAB_ROWS = (227 * 1024 - 1024) / (NR_TC * 8);
 constexpr int CLMAX = 16;        // max thread-block cluster size of chain_fit_kernel (8 = the portable limit; 16-CTA
                                  // clusters, one per GPC, are used when a batch has few chains: single-chain paths, fold shards)
 
@@ -122,9 +126,15 @@ void launch_pin(const Dev &d, double *vals, long long stride, int nch, const int
 // `gate`: see Dev::gate
 // exact top-k of `vals` ([nch][stride], first n_in of each row) -> out_idx [nch][out_ld] ascending; uses ping-pong scratch
 // idx0: optional explicit index of every input key ([nch][stride], ascending inside each row); default = position
-void launch_topk(const double *vals, long long stride, int n_in, int k, int nch, int *out_idx, int out_ld, int *tie,
-                 double *ck0, int *ci0, double *ck1, int *ci1, long long cstride, cudaStream_t st,
-                 const int *gate = nullptr, const int *idx0 = nullptr);
+int launch_topk(const double *vals, long long stride, int n_in, int k, int nch, int *out_idx, int out_ld, int *tie,
+                double *ck0, int *ci0, double *ck1, int *ci1, long long cstride, cudaStream_t st,
+                const int *gate = nullptr, const int *idx0 = nullptr);
+// the exact top-k of the screening (ascending indices, larger key first then lower index, the tie flag of launch_topk) by a
+// device-wide radix select when p > TOPK_LMAX; otherwise, or when the boundary bin is too large, launch_topk.  scratch:
+// screen_select_scratch_bytes(p) device bytes; ck*/ci*/cstride as for launch_topk.  Returns the number of launches.
+size_t screen_select_scratch_bytes(int p);
+int launch_screen_select(const double *vals, int p, int k, int *out_idx, int *tie, void *scratch, double *ck0, int *ci0,
+                         double *ck1, int *ci1, long long cstride, cudaStream_t st);
 // finish + pin + top-k in one kernel (p <= TOPK_LMAX): reads the sweep partials, writes d.Anew / d.tie for chains
 // cmin .. cmin + nspan - 1 that have not met the stopping rule
 void launch_topk_fused(const Dev &d, int mode, int epi, int cmin, int nspan, int k, const int *always, int n_always,
@@ -169,6 +179,10 @@ void launch_norm_factors(const double *h, int p, double sn, double *norm_out, do
 // one-launch normalisation of an L2-resident design (gmean = w / n or nullptr for no centring, wnorm = w, rowmul or nullptr)
 void launch_normalize_resident(double *X, long long ldx, int n, int p, const double *gmean, const double *wnorm,
                                const double *rowmul, double sn, double *mean_out, double *norm_out, cudaStream_t st);
+// the same with screening's gather of the kept columns fused in: Xn[:, q] <- normalised X[:, cols[q]], q < p (n <= NR_SLAB_ROWS)
+void launch_gather_normalize(const double *X, long long ldx, const int *cols, double *Xn, long long ldn, int n, int p,
+                             const double *gmean, const double *wnorm, const double *rowmul, double sn, double *mean_out,
+                             double *norm_out, cudaStream_t st);
 void launch_center_scale(double *X, long long ldx, int n, int p, const double *sub, const double *mul,
                          const double *rowmul, cudaStream_t st);
 void launch_gather_cols(const double *X, long long ldx, int n, const int *cols, int pnew, double *Xn, long long ldn,

@@ -92,6 +92,13 @@ class GpuEngine:
         _lib.check(self._lib.bessgpu_get_norm(self._h, _d(xm), _d(xn), C.byref(ym)))
         return xm, xn, ym.value
 
+    def design(self):
+        """A host copy of the engine's current dense design (n x p): the kept columns after ``screen``, normalised after
+        ``normalize``."""
+        x = np.zeros((self.n, self.p))
+        _lib.check(self._lib.bessgpu_design(self._h, _d(x)))
+        return x
+
     def set_groups(self, g_index):
         """Group selection: g_index = first column of every group; levels / kcap / always_select then count groups."""
         g = np.ascontiguousarray(g_index, dtype=np.int32)
@@ -156,4 +163,15 @@ def topk(vals, k):
     out = np.zeros(k, dtype=np.int32)
     tie = C.c_int(0)
     _lib.check(lib.bessgpu_topk(_d(v), v.size, k, _i(out), C.byref(tie)))
+    return out, tie.value
+
+
+def screen_select(vals, k):
+    """``topk`` by the screening's select (device-wide when there are more than 16384 values): same result."""
+    lib = _lib.load()
+    _lib.require_gpu()
+    v = np.ascontiguousarray(vals, dtype=np.float64)
+    out = np.zeros(k, dtype=np.int32)
+    tie = C.c_int(0)
+    _lib.check(lib.bessgpu_screen_select(_d(v), v.size, k, _i(out), C.byref(tie)))
     return out, tie.value

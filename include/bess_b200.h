@@ -189,6 +189,9 @@ int bessgpu_normalize(bessgpu_handle *h, int data_type, int is_normal);
  * count groups (Algorithm.h:1097-1129, 1206-1263, 1324-1367, 1497-1568; utilities.cpp:113-177). */
 int bessgpu_set_groups(bessgpu_handle *h, const int *g_index, int n_groups);
 int bessgpu_get_norm(bessgpu_handle *h, double *x_mean_out, double *x_norm_out, double *y_mean_out);
+/* the engine's current dense design (after screening: the kept columns; after normalize: normalised), row-major
+ * n x p into host memory */
+int bessgpu_design(bessgpu_handle *h, double *x_out);
 /* Metric.h:49-129 (fold row lists, per-fold x_j.x_j) + workspace for supports up to kcap */
 int bessgpu_setup_chains(bessgpu_handle *h, int K, const int *fold_of_row, int kcap, int max_iter, int warm_start,
                          const int *always_select, int n_always);
@@ -207,6 +210,8 @@ int bessgpu_stats(bessgpu_handle *h, double *out8);
 /* stand-alone exact top-k (utilities.cpp:179-188 max_k): host vals[n] -> ascending indices; tie_out = 1 when keys equal to
  * the k-th straddle the boundary */
 int bessgpu_topk(const double *vals, int n, int k, int *idx_out, int *tie_out);
+/* the same by the screening's select (a device-wide radix select when n > 16384): same indices, order and tie flag */
+int bessgpu_screen_select(const double *vals, int n, int k, int *idx_out, int *tie_out);
 
 /* pgs_path geometry (path.cpp:414-577, pure host code): the points where the search line p + t*u leaves the box
  * [s_min, s_max] x [log_lambda_min, log_lambda_max]; a2_out / b2_out receive the first two in the reference's edge order.
