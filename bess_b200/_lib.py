@@ -77,6 +77,7 @@ def load():
     lib.bessgpu_losses.argtypes = [C.c_void_p, ip, ip, ip, C.c_int, dp]
     lib.bessgpu_time_dual_sweep.argtypes = [C.c_void_p, C.c_int, C.POINTER(C.c_float), dp]
     lib.bessgpu_stats.argtypes = [C.c_void_p, dp]
+    lib.bessgpu_sacrifice.argtypes = [C.c_void_p, ip, C.c_int, C.c_double, dp, ip]
     lib.bessgpu_topk.argtypes = [dp, C.c_int, C.c_int, ip, ip]
     lib.bessgpu_screen_select.argtypes = [dp, C.c_int, C.c_int, ip, ip]
     lib.bess_b200_shard_range.restype = None

@@ -442,6 +442,14 @@ int bessgpu_time_dual_sweep(bessgpu_handle *h, int reps, float *ms_out, double *
         if (bytes_out) *bytes_out = 8.0 * (double)h->eng->n() * (double)h->eng->p();
     });
 }
+int bessgpu_sacrifice(bessgpu_handle *h, const int *chains, int nch, double lambda, double *bd_out, int *info_out)
+{
+    return guarded([&] {
+        std::vector<double> bd;
+        h->eng->debug_sacrifice(std::vector<int>(chains, chains + nch), lambda, bd, info_out);
+        std::copy(bd.begin(), bd.end(), bd_out);
+    });
+}
 int bessgpu_stats(bessgpu_handle *h, double *o)
 {
     return guarded([&] {

@@ -2401,6 +2401,32 @@ __global__ void __launch_bounds__(256) chain_state_gather_kernel(const Dev d, in
     if (off)
         for (int r = blockIdx.x * blockDim.x + threadIdx.x; r < nt; r += gridDim.x * blockDim.x) XA[(size_t)r * d.ldA] = 1.0;
 }
+// A chain that meets the stopping rule returns from chain_fit_kernel before chain_gradient, so the vectors it last published
+// belong to the beta before its last fit; this kernel publishes them for the stored (A, beta_A, coef0) (kernels.cuh).
+__global__ void __launch_bounds__(FIT_NT, 1) chain_gradient_kernel(const Dev d, const BatchDesc b)
+{
+    extern __shared__ __align__(128) unsigned char smem_raw[];
+    const FitSmem sm = carve_fit_smem(smem_raw, d.ldA, d.fit_smem_doubles);
+    const int c = b.chain[blockIdx.x];
+    const int ks = d.ks[c];
+    for (int a = threadIdx.x; a < ks; a += FIT_NT) sm.b0[a] = d.bA[(size_t)c * d.kcap + a];
+    __syncthreads();
+    Clu cl = make_clu(sm, 1);
+    ChainCtx cx = make_ctx(d, c, ks, cl, sm);
+    chain_gradient(d, cx, cl, sm.b0, ks, d.coef0[c], sm);
+}
+void launch_chain_gradient(const Dev &d, const BatchDesc &b, cudaStream_t st)
+{
+    for (int i = 0; i < b.nch; i++) {
+        chain_state_gather_kernel<<<148, 256, 0, st>>>(d, b.chain[i]);
+        CUDA_CHECK(cudaGetLastError());
+    }
+    const size_t smem = fit_smem_bytes(d);
+    CUDA_CHECK(cudaFuncSetAttribute(chain_gradient_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    chain_gradient_kernel<<<b.nch, FIT_NT, smem, st>>>(d, b);
+    CUDA_CHECK(cudaGetLastError());
+}
+
 void launch_chain_state(const Dev &d, int chain, int op, int slot_beta, int slot_coef0, const StateSlots &s, cudaStream_t st)
 {
     chain_state_kernel<<<1, FIT_NT, 0, st>>>(d, chain, op, slot_beta, slot_coef0, s);

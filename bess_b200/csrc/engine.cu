@@ -2306,20 +2306,53 @@ float Engine::time_dual_sweep(int nch, int reps)
     return ms / (float)reps;
 }
 
-// Recompute the sacrifice of `chain` for its CURRENT beta (test hook for the sweep + finish kernels).
-void Engine::debug_sacrifice(int chain, std::vector<double> &bd_out)
+// Test hook: recompute the sacrifice of every chain of `chains` for the state the last batch returned, through the
+// dispatch a fit of this batch uses.  The gradient vectors are published again from the stored (A, beta_A, coef0) first
+// (see launch_chain_gradient); the launches run on a copy of the descriptor without gate, at ridge level `lambda`, with
+// every chain marked as iterating (the group kernels skip chains that are done).
+void Engine::debug_sacrifice(const std::vector<int> &chains, double lambda, std::vector<double> &bd_out, int *info_out)
 {
     Impl &m = *d_;
-    Dev &d = m.d;
+    if (!m.chains_ready) throw EngineError{"debug_sacrifice before setup_chains"};
+    if (sharded_) throw EngineError{"debug_sacrifice is not available in column-sharded mode"};
+    if (m.tk[0].pending || m.tk[1].pending) throw EngineError{"debug_sacrifice: a batch is still pending"};
+    if (chains.empty() || (int)chains.size() > m.nchains) throw EngineError{"bad chain set"};
+    if (!(lambda >= 0.0)) throw EngineError{"lambda must be >= 0"};
+    Dev d = m.d;
+    d.gate = nullptr;
+    d.prev_active = nullptr;
+    d.lambda = lambda;
     BatchDesc b{};
-    b.nch = 1;
-    b.chain[0] = chain;
+    b.nch = (int)chains.size();
+    b.CL = 1;
+    for (int i = 0; i < b.nch; i++) {
+        if (chains[i] < 0 || chains[i] >= m.nchains) throw EngineError{"chain id out of range"};
+        b.chain[i] = chains[i];
+    }
+    int *done0 = dalloc<int>(m.st, MAXC);
+    CUDA_CHECK(cudaMemsetAsync(done0, 0, MAXC * sizeof(int), m.st));
+    d.done = done0;
+    launch_chain_gradient(d, b, m.st);
     const int mode = sweep_mode(family_), epi = sweep_epi(family_);
-    launch_dual_sweep(d, mode, m.st);
-    launch_finish(d, mode, epi, b, nullptr, m.st);
-    bd_out.resize(d.p);
-    CUDA_CHECK(cudaMemcpyAsync(bd_out.data(), d.bd + (size_t)chain * d.pstride, (size_t)d.p * 8, cudaMemcpyDeviceToHost,
-                               m.st));
+    for (int q = 0; q < 8; q++) info_out[q] = 0;
+    info_out[1] = d.FS;
+    if (d.grouped) {
+        info_out[0] = 3;
+        info_out[5] = launch_group_sacrifice(d, b, m.st);
+    } else {
+        info_out[0] = sweep_uses_tma(d) ? 2 : 1;
+        info_out[2] = sweep_cpt(d, mode);
+        info_out[3] = d.S;
+        info_out[4] = d.rows_per_split;
+        launch_dual_sweep(d, mode, m.st);
+        launch_finish(d, mode, epi, b, nullptr, m.st);
+    }
+    const int N = d.grouped ? d.N : d.p;
+    bd_out.resize((size_t)b.nch * N);
+    for (int i = 0; i < b.nch; i++)
+        CUDA_CHECK(cudaMemcpyAsync(bd_out.data() + (size_t)i * N, d.bd + (size_t)b.chain[i] * d.pstride, (size_t)N * 8,
+                                   cudaMemcpyDeviceToHost, m.st));
+    dfree(m.st, done0);
     CUDA_CHECK(cudaStreamSynchronize(m.st));
 }
 

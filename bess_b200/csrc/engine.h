@@ -190,7 +190,9 @@ public:
     // ---- primitives exposed for tests / roofline benchmarking through the C-ABI
     // Dual sweep + sacrifice for `nch` chains (chain slots f0..f0+nch) -> bd on device; returns kernel ms if timed.
     float time_dual_sweep(int nch, int reps);
-    void debug_sacrifice(int chain, std::vector<double> &bd_out);   // after run_batch: recompute bd for chain's current beta
+    // after run_batch: bd of `chains` for their current model ([nch][p], or [nch][n_groups]); info_out[8] as
+    // bessgpu_sacrifice (include/bess_b200.h)
+    void debug_sacrifice(const std::vector<int> &chains, double lambda, std::vector<double> &bd_out, int *info_out);
 
     int n() const { return n_; }
     int p() const { return p_; }

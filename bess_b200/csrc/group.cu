@@ -449,8 +449,9 @@ __global__ void group_expand_kernel(const Dev d, const BatchDesc b)
     d.Tc[c] = cnt;
 }
 
-void launch_group_sacrifice(const Dev &d, const BatchDesc &b, cudaStream_t st)
+int launch_group_sacrifice(const Dev &d, const BatchDesc &b, cudaStream_t st)
 {
+    int ran = 0;
     static const bool serial = [] {
         const char *e = std::getenv("BESS_B200_GROUP_SERIAL");
         return e && e[0] == '1';
@@ -459,6 +460,7 @@ void launch_group_sacrifice(const Dev &d, const BatchDesc &b, cudaStream_t st)
         const dim3 grid((unsigned)((d.N + GS_NT - 1) / GS_NT), (unsigned)b.nch);
         if (d.family == FAM_COX) group_sacrifice_kernel<true><<<grid, GS_NT, 0, st>>>(d, b);
         else group_sacrifice_kernel<false><<<grid, GS_NT, 0, st>>>(d, b);
+        ran |= GSAC_SERIAL;
     } else {
         static const bool per_chain = [] {
             const char *e = std::getenv("BESS_B200_GROUP_PER_CHAIN");
@@ -468,6 +470,7 @@ void launch_group_sacrifice(const Dev &d, const BatchDesc &b, cudaStream_t st)
             const int wpb = GS_NT / 32;
             const dim3 grid((unsigned)((d.N + wpb - 1) / wpb), (unsigned)b.nch);
             group_sacrifice_warp_kernel<<<grid, GS_NT, 0, st>>>(d, b);
+            ran |= GSAC_WARP;
         } else {
             const int wpb = GB_NT / 32;
             for (int k = 0; k < 3; k++) {  // one instantiation per width class of the narrow groups
@@ -477,6 +480,7 @@ void launch_group_sacrifice(const Dev &d, const BatchDesc &b, cudaStream_t st)
                 if (k == 0) group_sacrifice_batched_kernel<2><<<grid, GB_NT, 0, st>>>(d, b, lo, hi);
                 else if (k == 1) group_sacrifice_batched_kernel<4><<<grid, GB_NT, 0, st>>>(d, b, lo, hi);
                 else group_sacrifice_batched_kernel<GMAX><<<grid, GB_NT, 0, st>>>(d, b, lo, hi);
+                ran |= GSAC_BATCHED2 << k;
             }
         }
     }
@@ -492,7 +496,9 @@ void launch_group_sacrifice(const Dev &d, const BatchDesc &b, cudaStream_t st)
             group_sacrifice_wide_kernel<false><<<grid, GW_NT, smem, st>>>(d, b);
         }
         CUDA_CHECK(cudaGetLastError());
+        ran |= GSAC_WIDE;
     }
+    return ran;
 }
 void launch_group_expand(const Dev &d, const BatchDesc &b, cudaStream_t st)
 {

@@ -239,22 +239,32 @@ static void launch_sweep_t(const Dev &d, cudaStream_t st)
     CUDA_CHECK(cudaGetLastError());
 }
 
+// columns per thread of dual_sweep_kernel: 2 (16-byte loads) unless the accumulator set would not fit in registers
+constexpr int stream_cpt(int FT, int MODE)
+{
+    return FT <= 2 ? 2 : (FT <= 6 ? (MODE == MODE_COX ? 1 : 2) : (FT <= 12 ? (MODE == MODE_D ? 2 : 1) : 1));
+}
+
 template <int MODE>
 static void launch_sweep_m(const Dev &d, cudaStream_t st)
 {
-    // columns per thread: 2 (16-byte loads) unless the accumulator set would not fit in registers
     switch (d.FS) {
-        case 1: launch_sweep_t<1, MODE, 2>(d, st); break;
-        case 2: launch_sweep_t<2, MODE, 2>(d, st); break;
-        case 4: launch_sweep_t<4, MODE, MODE == MODE_COX ? 1 : 2>(d, st); break;
-        case 6: launch_sweep_t<6, MODE, MODE == MODE_COX ? 1 : 2>(d, st); break;
-        case 8: launch_sweep_t<8, MODE, MODE == MODE_D ? 2 : 1>(d, st); break;
-        case 12: launch_sweep_t<12, MODE, MODE == MODE_D ? 2 : 1>(d, st); break;
-        case 16: launch_sweep_t<16, MODE, 1>(d, st); break;
-        case 24: launch_sweep_t<24, MODE, 1>(d, st); break;
-        case 32: launch_sweep_t<32, MODE, 1>(d, st); break;
+        case 1: launch_sweep_t<1, MODE, stream_cpt(1, MODE)>(d, st); break;
+        case 2: launch_sweep_t<2, MODE, stream_cpt(2, MODE)>(d, st); break;
+        case 4: launch_sweep_t<4, MODE, stream_cpt(4, MODE)>(d, st); break;
+        case 6: launch_sweep_t<6, MODE, stream_cpt(6, MODE)>(d, st); break;
+        case 8: launch_sweep_t<8, MODE, stream_cpt(8, MODE)>(d, st); break;
+        case 12: launch_sweep_t<12, MODE, stream_cpt(12, MODE)>(d, st); break;
+        case 16: launch_sweep_t<16, MODE, stream_cpt(16, MODE)>(d, st); break;
+        case 24: launch_sweep_t<24, MODE, stream_cpt(24, MODE)>(d, st); break;
+        case 32: launch_sweep_t<32, MODE, stream_cpt(32, MODE)>(d, st); break;
         default: throw EngineError{"dual sweep: unsupported chain tile FS=" + std::to_string(d.FS)};
     }
+}
+
+int sweep_cpt(const Dev &d, int mode)
+{
+    return sweep_uses_tma(d) ? sweep_tma_cpt(d.FS, mode) : stream_cpt(d.FS, mode);
 }
 
 void launch_dual_sweep(const Dev &d, int mode, cudaStream_t st)

@@ -121,6 +121,9 @@ void launch_dual_sweep(const Dev &d, int mode, cudaStream_t st);
 // bulk-TMA pipelined variant for batched chains (sweep_tma.cu); launch_dual_sweep dispatches to it when FS >= 2
 bool sweep_uses_tma(const Dev &d);
 void launch_dual_sweep_tma(const Dev &d, int mode, cudaStream_t st);
+// columns per thread of the sweep launch_dual_sweep runs for d.FS and `mode` (sweep_tma_cpt: of the bulk-TMA kernel)
+int sweep_cpt(const Dev &d, int mode);
+int sweep_tma_cpt(int FS, int mode);
 void launch_finish(const Dev &d, int mode, int epi, const BatchDesc &b, double *raw_out, cudaStream_t st);
 void launch_pin(const Dev &d, double *vals, long long stride, int nch, const int *idx, int nidx, cudaStream_t st);
 // `gate`: see Dev::gate
@@ -157,7 +160,9 @@ void launch_gather_owned_cols(const double *X, long long ldx, int n, int p_local
                               double *Xn, long long ldn, cudaStream_t st);
 void launch_chain_begin(const Dev &d, const BatchDesc &b, cudaStream_t st);
 // ---- group selection (group.cu): sweep + group sacrifice in one kernel -> d.bd[chain][group]; selected groups -> columns
-void launch_group_sacrifice(const Dev &d, const BatchDesc &b, cudaStream_t st);
+// returns the GSAC_* bits of the kernels it launched
+enum { GSAC_SERIAL = 1, GSAC_WARP = 2, GSAC_BATCHED2 = 4, GSAC_BATCHED4 = 8, GSAC_BATCHED8 = 16, GSAC_WIDE = 32 };
+int launch_group_sacrifice(const Dev &d, const BatchDesc &b, cudaStream_t st);
 void launch_group_expand(const Dev &d, const BatchDesc &b, cudaStream_t st);
 // ---- explicit warm-start state of a chain.  pgs_path re-seeds Algorithm::beta_init / coef0_init by hand (zeros at the
 // start of every line search, path.cpp:590-592; the snapshot after the first fit for the backward walk of seq_search,
@@ -173,6 +178,9 @@ struct StateSlots {
 // and re-gathers X_A).  ZERO: beta = 0, coef0 = 0.  A negative slot leaves that half untouched.
 void launch_chain_state(const Dev &d, int chain, int op, int slot_beta, int slot_coef0, const StateSlots &s, cudaStream_t st);
 void launch_chain_fit(const Dev &d, const BatchDesc &b, cudaStream_t st);
+// test hook: the gradient vectors (G, W, TH, C2) of every chain of the batch from its stored state (A, beta_A, coef0), X_A
+// re-gathered first -- what chain_begin_kernel publishes, without touching the chains' iteration state
+void launch_chain_gradient(const Dev &d, const BatchDesc &b, cudaStream_t st);
 void launch_losses(const Dev &d, const LossDesc &jobs, const int *testrows, const int *ntest, const double *y,
                    const double *w, const double *lfact, double *scratch, double *out, cudaStream_t st);
 void launch_norm_factors(const double *h, int p, double sn, double *norm_out, double *mul_out, cudaStream_t st);

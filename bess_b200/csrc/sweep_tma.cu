@@ -251,19 +251,24 @@ void launch_tma_t(const Dev &d, cudaStream_t st)
     CUDA_CHECK(cudaGetLastError());
 }
 
+// columns per thread: 2 (16-byte shared loads) unless the accumulator set would not fit in registers
+constexpr int tma_cpt(int FT, int MODE)
+{
+    return FT <= 6 ? 2 : (FT <= 12 ? (MODE == MODE_COX ? 1 : 2) : (FT == 16 ? (MODE == MODE_D ? 2 : 1) : 1));
+}
+
 template <int MODE>
 void launch_tma_m(const Dev &d, cudaStream_t st)
 {
-    // columns per thread: 2 (16-byte shared loads) unless the accumulator set would not fit in registers
     switch (d.FS) {
-        case 2: launch_tma_t<2, MODE, 2>(d, st); break;
-        case 4: launch_tma_t<4, MODE, 2>(d, st); break;
-        case 6: launch_tma_t<6, MODE, 2>(d, st); break;
-        case 8: launch_tma_t<8, MODE, MODE == MODE_COX ? 1 : 2>(d, st); break;
-        case 12: launch_tma_t<12, MODE, MODE == MODE_COX ? 1 : 2>(d, st); break;
-        case 16: launch_tma_t<16, MODE, MODE == MODE_D ? 2 : 1>(d, st); break;
-        case 24: launch_tma_t<24, MODE, 1>(d, st); break;
-        case 32: launch_tma_t<32, MODE, 1>(d, st); break;
+        case 2: launch_tma_t<2, MODE, tma_cpt(2, MODE)>(d, st); break;
+        case 4: launch_tma_t<4, MODE, tma_cpt(4, MODE)>(d, st); break;
+        case 6: launch_tma_t<6, MODE, tma_cpt(6, MODE)>(d, st); break;
+        case 8: launch_tma_t<8, MODE, tma_cpt(8, MODE)>(d, st); break;
+        case 12: launch_tma_t<12, MODE, tma_cpt(12, MODE)>(d, st); break;
+        case 16: launch_tma_t<16, MODE, tma_cpt(16, MODE)>(d, st); break;
+        case 24: launch_tma_t<24, MODE, tma_cpt(24, MODE)>(d, st); break;
+        case 32: launch_tma_t<32, MODE, tma_cpt(32, MODE)>(d, st); break;
         default: throw EngineError{"dual sweep: unsupported chain tile FS=" + std::to_string(d.FS)};
     }
 }
@@ -278,6 +283,11 @@ bool sweep_uses_tma(const Dev &d)
         force = (e && std::string(e) == "stream") ? 0 : 1;
     }
     return force == 1 && d.FS >= 2;
+}
+
+int sweep_tma_cpt(int FS, int mode)
+{
+    return tma_cpt(FS, mode);
 }
 
 void launch_dual_sweep_tma(const Dev &d, int mode, cudaStream_t st)

@@ -148,6 +148,18 @@ class GpuEngine:
         _lib.check(self._lib.bessgpu_time_dual_sweep(self._h, reps, C.byref(ms), C.byref(by)))
         return ms.value, by.value
 
+    def sacrifice(self, chains, lam=0.0):
+        """Test probe after a batch: the sacrifice of every chain in ``chains`` for its current model, recomputed through
+        the kernels a fit of this batch runs -> (bd [nch][p] or [nch][n_groups], dict of what ran)."""
+        ch = np.ascontiguousarray(chains, dtype=np.int32)
+        N = len(self._group_sizes) if hasattr(self, "_group_sizes") else self.p
+        bd = np.zeros((ch.size, N))
+        info = np.zeros(8, dtype=np.int32)
+        _lib.check(self._lib.bessgpu_sacrifice(self._h, _i(ch), ch.size, float(lam), _d(bd), _i(info)))
+        kind = {1: "stream", 2: "tma", 3: "group"}[int(info[0])]
+        return bd, dict(kernel=kind, FS=int(info[1]), CPT=int(info[2]), S=int(info[3]), rows_per_split=int(info[4]),
+                        groups=int(info[5]))
+
     def stats(self):
         o = np.zeros(8)
         _lib.check(self._lib.bessgpu_stats(self._h, _d(o)))

@@ -206,6 +206,13 @@ int bessgpu_run_batch_groups(bessgpu_handle *h, int T, const int *chains, int nc
 int bessgpu_losses(bessgpu_handle *h, const int *chain, const int *kind, const int *fold, int njobs, double *out);
 /* roofline probe: mean device time (ms) of one dual-sweep launch over all chain slots and its algorithmic bytes */
 int bessgpu_time_dual_sweep(bessgpu_handle *h, int reps, float *ms_out, double *bytes_out);
+/* test probe, after a batch returned: the sacrifice of every chain of `chains` for its current model (gradient vectors
+ * published again from the chain's support, coefficients and intercept), through the dispatch a fit of this batch uses,
+ * at ridge level `lambda`.  bd_out: [nch][p], or [nch][number of groups] with groups.  info_out[8]: [0] what ran (1
+ * streaming column sweep, 2 bulk-TMA column sweep, 3 group kernels), [1] chain slots FS, [2] columns per thread, [3] row
+ * splits, [4] rows per split, [5] group kernels launched (bits: 1 serial, 2 warp, 4 / 8 / 16 batched for widths <= 2 /
+ * 4 / 8, 32 wide) */
+int bessgpu_sacrifice(bessgpu_handle *h, const int *chains, int nch, double lambda, double *bd_out, int *info_out);
 int bessgpu_stats(bessgpu_handle *h, double *out8);
 /* stand-alone exact top-k (utilities.cpp:179-188 max_k): host vals[n] -> ascending indices; tie_out = 1 when keys equal to
  * the k-th straddle the boundary */
