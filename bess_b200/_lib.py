@@ -31,7 +31,7 @@ class Ext(C.Structure):
                 ("world", C.c_int), ("rank", C.c_int), ("col_lo", C.c_longlong), ("p_total", C.c_longlong),
                 ("nccl_unique_id", C.c_void_p), ("chosen_lambda_out", dp), ("beta_out_zeroed", C.c_int), ("cv_reduce_over_ranks", C.c_int),
                 ("cv_seed_set", C.c_int), ("tie_exact_out", ip), ("resident_out", dp), ("fold_shard", C.c_int),
-                ("x_csc", C.POINTER(Csc))]
+                ("x_csc", C.POINTER(Csc)), ("sparse_sweeps_out", ip)]
 
 
 _PYWRAP_ARGS = [dp, C.c_int, C.c_int, dp, C.c_int, C.c_int, dp, C.c_int, C.c_bool, C.c_int, C.c_int, C.c_int, C.c_int,

@@ -210,6 +210,8 @@ def fit(x, y, data_type, weight, is_normal, algorithm_type, model_type, max_iter
     tie_exact = C.c_int(0)
     ext.tie_exact_out = C.pointer(tie_exact)
     ext.resident_out = _d(resident)
+    sparse_sweeps = C.c_int(0)
+    ext.sparse_sweeps_out = C.pointer(sparse_sweeps)
     ext.profile = 1 if profile else 0
     ext.beta_out_zeroed = 1  # `beta` comes from np.zeros (calloc): untouched pages stay untouched
     ext.cv_reduce_over_ranks = 1 if (cv_reduce_over_ranks and sharded) else 0
@@ -230,6 +232,7 @@ def fit(x, y, data_type, weight, is_normal, algorithm_type, model_type, max_iter
                           host_ms=dict(zip(("load", "screen", "normalize", "setup_chains", "path"), stats[27:32].tolist())),
                           resident=resident.tolist(), tie_exact_pass=bool(tie_exact.value & 1),
                           robust_pass=bool(tie_exact.value & 2), rank_deficient=bool(tie_exact.value & 4),
+                          sparse_sweeps=int(sparse_sweeps.value),
                           prof_ms=dict(zip(PROF_CATS, stats[8:16].tolist())),
                           prof_launches=dict(zip(PROF_CATS, [int(v) for v in stats[16:24]]))))
     if is_screening:

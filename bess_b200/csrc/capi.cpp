@@ -125,6 +125,7 @@ int bess_b200_fit_impl(double *x, int x_row, int x_col, double *y, int y_len, in
             if (ext->screening_A_out && !r.screening_A.empty())
                 std::copy(r.screening_A.begin(), r.screening_A.end(), ext->screening_A_out);
             if (ext->chosen_s_out) *ext->chosen_s_out = r.chosen_s;
+            if (ext->sparse_sweeps_out) *ext->sparse_sweeps_out = r.sparse_sweeps ? 1 : 0;
             if (ext->chosen_lambda_out) *ext->chosen_lambda_out = r.lambda;
             if (ext->resident_out) std::copy(r.resident, r.resident + 24 + 4 * MAXC, ext->resident_out);
             if (ext->tie_exact_out)
@@ -439,7 +440,7 @@ int bessgpu_time_dual_sweep(bessgpu_handle *h, int reps, float *ms_out, double *
 {
     return guarded([&] {
         *ms_out = h->eng->time_dual_sweep(0, reps);
-        if (bytes_out) *bytes_out = 8.0 * (double)h->eng->n() * (double)h->eng->p();
+        if (bytes_out) *bytes_out = h->eng->dual_sweep_bytes();
     });
 }
 int bessgpu_sacrifice(bessgpu_handle *h, const int *chains, int nch, double lambda, double *bd_out, int *info_out)

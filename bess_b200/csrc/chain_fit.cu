@@ -2261,7 +2261,7 @@ __global__ void __launch_bounds__(FIT_NT, 1) chain_fit_kernel(const Dev d, const
                 const int it = it0 + q * FIT_NT;
                 if (it < tot) {
                     const int r = it / T, a = it - r * T;
-                    val[q] = d.sharded ? d.AXr[((size_t)c * d.n + rows[cx.rb + r]) * d.ldXr + a]
+                    val[q] = d.ax_ext ? d.AXr[((size_t)c * d.n + rows[cx.rb + r]) * d.ldXr + a]
                                        : __ldg(d.X + (size_t)rows[cx.rb + r] * d.ldx + Anew[a]);
                 }
             }
@@ -2276,7 +2276,7 @@ __global__ void __launch_bounds__(FIT_NT, 1) chain_fit_kernel(const Dev d, const
         }
         if (cx.off)
             for (int r = cx.rb + threadIdx.x; r < cx.re; r += FIT_NT) cx.XA[(size_t)r * ldA] = 1.0;
-        if (d.sharded) {  // keep the all-row columns of this support for the loss kernel
+        if (d.ax_ext) {  // keep the all-row columns of this support for the loss kernel
             const double *src = d.AXr + (size_t)c * d.n * d.ldXr;
             double *dst = d.AXk + (size_t)c * d.n * d.ldXk;
             for (int e = cl.rank * FIT_NT + threadIdx.x; e < d.n * T; e += cl.CL * FIT_NT) {
@@ -2396,7 +2396,8 @@ __global__ void __launch_bounds__(256) chain_state_gather_kernel(const Dev d, in
     const long long tot = (long long)nt * ks;
     for (long long e = (long long)blockIdx.x * blockDim.x + threadIdx.x; e < tot; e += (long long)gridDim.x * blockDim.x) {
         const int r = (int)(e / ks), a = (int)(e - (long long)r * ks);
-        XA[(size_t)r * d.ldA + off + a] = __ldg(d.X + (size_t)rows[r] * d.ldx + A[a]);
+        XA[(size_t)r * d.ldA + off + a] = d.ax_ext ? d.AXk[((size_t)c * d.n + rows[r]) * d.ldXk + a]
+                                                   : __ldg(d.X + (size_t)rows[r] * d.ldx + A[a]);
     }
     if (off)
         for (int r = blockIdx.x * blockDim.x + threadIdx.x; r < nt; r += gridDim.x * blockDim.x) XA[(size_t)r * d.ldA] = 1.0;
@@ -2417,6 +2418,7 @@ __global__ void __launch_bounds__(FIT_NT, 1) chain_gradient_kernel(const Dev d, 
 }
 void launch_chain_gradient(const Dev &d, const BatchDesc &b, cudaStream_t st)
 {
+    if (d.ccp) launch_csc_gather(d, b, 1, st);  // AXk <- the stored supports, re-expanded from the CSC arrays
     for (int i = 0; i < b.nch; i++) {
         chain_state_gather_kernel<<<148, 256, 0, st>>>(d, b.chain[i]);
         CUDA_CHECK(cudaGetLastError());
@@ -2432,6 +2434,12 @@ void launch_chain_state(const Dev &d, int chain, int op, int slot_beta, int slot
     chain_state_kernel<<<1, FIT_NT, 0, st>>>(d, chain, op, slot_beta, slot_coef0, s);
     CUDA_CHECK(cudaGetLastError());
     if (op == STATE_LOAD && slot_beta >= 0) {
+        if (d.ccp) {  // AXk (losses) <- the restored support from the CSC arrays; XA's train rows follow from it
+            BatchDesc b{};
+            b.nch = 1;
+            b.chain[0] = chain;
+            launch_csc_gather(d, b, 1, st);
+        }
         chain_state_gather_kernel<<<148, 256, 0, st>>>(d, chain);
         CUDA_CHECK(cudaGetLastError());
     }

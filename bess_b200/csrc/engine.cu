@@ -347,6 +347,10 @@ struct Engine::Impl {
     int *ri = nullptr;
     double *cv = nullptr;
     long long nnz = 0;
+    // a sparse design normalised in place of densifying it (normalize of a CSC engine): the path sweeps the CSC arrays and
+    // sees x~_ij = ((x_ij - cmean[j]) * cmul[j]) * crm[i] (Dev::ccp)
+    bool csc_norm = false;
+    double *cmean = nullptr, *cmul = nullptr, *crm = nullptr;
     void free_csc()
     {
         if (csc_owned) {
@@ -354,8 +358,11 @@ struct Engine::Impl {
             dfree(st, ri);
             dfree(st, cv);
         }
+        dfree(st, cmean);
+        dfree(st, cmul);
+        dfree(st, crm);
         cp = nullptr; ri = nullptr; cv = nullptr;
-        csc = csc_owned = false;
+        csc = csc_owned = csc_norm = false;
         nnz = 0;
     }
     int n = 0, p = 0, npad = 0;
@@ -567,6 +574,7 @@ struct Engine::Impl {
                 }
             }
         }
+        if (csc_norm) S = 1;  // the CSC sweep reduces each column over all rows itself
         int rps = (int)((n + S - 1) / S);
         rps = (rps + 1) & ~1;
         d.rows_per_split = rps;
@@ -579,6 +587,31 @@ struct Engine::Impl {
         d.c2sum = ctx->ar.alloc<double>((size_t)d.S * FS);
         d.bd = ctx->ar.alloc<double>((size_t)FS * d.pstride);
         raw = ctx->ar.alloc<double>((size_t)2 * FS * d.pstride);
+        d.ccp = nullptr; d.cri = nullptr; d.ccv = nullptr;
+        d.clong = nullptr; d.nlong = 0;
+        d.cmean = d.cmul = d.crm = nullptr;
+        d.csum = d.cpre = nullptr;
+        if (csc_norm) {
+            d.ccp = cp; d.cri = ri; d.ccv = cv;
+            d.cmean = cmean; d.cmul = cmul; d.crm = crm;
+            d.csum = ctx->ar.alloc<double>((size_t)2 * FS);
+            d.cpre = d.family == FAM_COX ? ctx->ar.alloc<double>((size_t)npad * FS) : nullptr;
+            const double mean_len = (double)nnz / (double)p;
+            d.csc_g = mean_len < 4.0 ? 2 : (mean_len < 16.0 ? 8 : 32);
+            d.csc_nnz = nnz;
+            // a column longer than 16 steps of its G lanes (the frequent terms of a power-law design) is swept by a CTA of
+            // its own, so that it does not hold the rest of the grid up
+            d.clong_thr = 16LL * d.csc_g;
+            int *list = ctx->ar.alloc<int>((size_t)p);
+            int *cnt = ctx->ar.alloc<int>(1);
+            int *h_cnt = ctx->rb.alloc<int>(1);
+            CUDA_CHECK(cudaMemsetAsync(cnt, 0, sizeof(int), st));
+            launch_csc_long_list(cp, p, d.clong_thr, list, cnt, st);
+            CUDA_CHECK(cudaMemcpyAsync(h_cnt, cnt, sizeof(int), cudaMemcpyDeviceToHost, st));
+            CUDA_CHECK(cudaStreamSynchronize(st));
+            d.clong = list;
+            d.nlong = *h_cnt;
+        }
         mk_sweep_end = ctx->ar.mark();
         have_sweep = true;
     }
@@ -1249,7 +1282,17 @@ static int *screen_select(Engine::Impl &m, EngineStats &stats_, int family_, int
 void Engine::copy_design(double *host_out)
 {
     Impl &m = *d_;
-    if (m.csc) throw EngineError{"copy_design: the design is sparse"};
+    if (m.csc && !m.csc_norm) throw EngineError{"copy_design: the design is sparse (normalise it first)"};
+    if (m.csc) {  // the normalised design, expanded on the device
+        if (!m.have_sweep) m.config_sweep(1);
+        double *buf = dalloc<double>(m.st, (size_t)m.n * m.p);
+        launch_csc_expand(m.d, buf, m.p, m.st);
+        CUDA_CHECK(cudaMemcpyAsync(host_out, buf, (size_t)m.n * m.p * 8, cudaMemcpyDeviceToHost, m.st));
+        dfree(m.st, buf);
+        CUDA_CHECK(cudaStreamSynchronize(m.st));
+        stats_.kernel_launches += 1;
+        return;
+    }
     if (!m.X) throw EngineError{"copy_design: no design is loaded"};
     materialise_gather(m, stats_);
     CUDA_CHECK(cudaMemcpy2DAsync(host_out, (size_t)m.p * 8, m.X, (size_t)m.ldx * 8, (size_t)m.p * 8, m.n,
@@ -1261,7 +1304,10 @@ void Engine::copy_design(double *host_out)
 void Engine::normalize(int data_type, bool is_normal)
 {
     Impl &m = *d_;
-    if (m.csc) throw EngineError{"normalize: a sparse design must be screened or densified first"};
+    if (m.csc) {
+        normalize_csc(data_type, is_normal);
+        return;
+    }
     const int n = m.n, p = m.p;
     // ---- a design that fits L2 (after screening: config 5's 40 MB): the whole normalisation is ONE launch, which also
     // gathers the kept columns of a pending screening when their n x 8 slabs fit shared memory
@@ -1421,6 +1467,78 @@ void Engine::normalize(int data_type, bool is_normal)
     }
 }
 
+// normalize() of a sparse design: the arrays stay as they are and only the column statistics and the row factors are
+// computed (normalize.cpp:20-86, add_weight of Data.h:70-77); the design the path sees is the implicit
+// x~_ij = ((x_ij - mean_j) * mul_j) * rowmul_i, swept on its non-zeros.  Equal to the dense statistics up to summation order.
+void Engine::normalize_csc(int data_type, bool is_normal)
+{
+    Impl &m = *d_;
+    if (m.csc_norm) throw EngineError{"normalize: the sparse design is already normalised"};
+    const int n = m.n, p = m.p;
+    const int sp = m.span_begin(6);
+    const bool centre = is_normal && (data_type == 1 || data_type == 2);
+    m.free_sweep_buffers();
+    m.cmean = dalloc<double>(m.st, (size_t)p);
+    m.cmul = dalloc<double>(m.st, (size_t)p);
+    m.stats_have_mean = false;
+    m.stats_pending = false;
+    if (is_normal) {
+        std::vector<double> g(n);
+        double sumw = 0.0;
+        for (int i = 0; i < n; i++) {
+            g[i] = m.hw[i] / (double)n;  // meanx_j = w.x_j / n (normalize.cpp:25-28, 52-55)
+            sumw += m.hw[i];
+        }
+        double *d_g = centre ? m.stage_vec(g.data(), (size_t)n, (size_t)n) : nullptr;
+        m.ctx->mir.flush(m.st);
+        m.h_mean = m.ctx->rb.alloc<double>((size_t)p);
+        m.h_norm = m.ctx->rb.alloc<double>((size_t)p);
+        double *d_norm = m.ctx->ar.alloc<double>((size_t)p);
+        launch_csc_stats(m.cp, m.ri, m.cv, p, d_g, m.w, sumw, std::sqrt((double)n), m.cmean, d_norm, m.cmul, m.st);
+        if (centre) CUDA_CHECK(cudaMemcpyAsync(m.h_mean, m.cmean, (size_t)p * 8, cudaMemcpyDeviceToHost, m.st));
+        CUDA_CHECK(cudaMemcpyAsync(m.h_norm, d_norm, (size_t)p * 8, cudaMemcpyDeviceToHost, m.st));
+        m.stats_have_mean = centre;
+        m.stats_pending = true;
+        stats_.kernel_launches += 1;
+        stats_.norm_bytes += 2.0 * (12.0 * (double)m.nnz + 8.0 * ((double)p + 1)) + 16.0 * n + 24.0 * p;
+    } else {
+        std::vector<double> zero((size_t)p, 0.0), one((size_t)p, 1.0);
+        CUDA_CHECK(cudaMemcpyAsync(m.cmean, zero.data(), (size_t)p * 8, cudaMemcpyHostToDevice, m.st));
+        CUDA_CHECK(cudaMemcpyAsync(m.cmul, one.data(), (size_t)p * 8, cudaMemcpyHostToDevice, m.st));
+        CUDA_CHECK(cudaStreamSynchronize(m.st));  // the host vectors die here
+    }
+    if (data_type == 1 && is_normal) {
+        double s = 0.0;
+        for (int i = 0; i < n; i++) s += m.hy[i] * m.hw[i];  // normalize.cpp:29
+        y_mean_ = s / (double)n;
+        for (int i = 0; i < n; i++) m.hy[i] -= y_mean_;
+    }
+    if (family_ == FAM_LM) {  // add_weight: rows scaled by sqrt(w) (Data.h:70-77)
+        std::vector<double> rm(n);
+        for (int i = 0; i < n; i++) {
+            rm[i] = std::sqrt(m.hw[i]);
+            m.hy[i] *= rm[i];
+        }
+        m.crm = dalloc<double>(m.st, (size_t)n);
+        CUDA_CHECK(cudaMemcpyAsync(m.crm, rm.data(), (size_t)n * 8, cudaMemcpyHostToDevice, m.st));
+        CUDA_CHECK(cudaStreamSynchronize(m.st));
+    }
+    m.y = m.stage_vec(m.hy.data(), (size_t)n, (size_t)m.npad);  // the response as the fits see it
+    m.ctx->mir.flush(m.st);
+    m.csc_norm = true;
+    m.span_end(sp);
+    h_xmean_.clear();
+    h_xnorm_.clear();
+}
+
+bool Engine::sparse_sweeps() const { return d_->csc_norm; }
+size_t Engine::device_total_bytes() const
+{
+    size_t free_b = 0, total_b = 0;
+    CUDA_CHECK(cudaMemGetInfo(&free_b, &total_b));
+    return total_b;
+}
+
 // The column statistics of the last normalize() on the host (h_xmean_, h_xnorm_): waits for the device only here.
 void Engine::ensure_stats() const
 {
@@ -1441,6 +1559,7 @@ void Engine::set_groups(const std::vector<int> &g_index)
 {
     Impl &m = *d_;
     if (sharded_) throw EngineError{"group selection is not available in column-sharded mode"};
+    if (m.csc) throw EngineError{"group selection needs a dense design (densify or screen the sparse one)"};
     const int p = m.p, N = (int)g_index.size();
     if (N < 1 || N > p) throw EngineError{"g_index must hold between 1 and p group starts"};
     if (g_index[0] != 0) throw EngineError{"g_index must start at column 0"};
@@ -1480,6 +1599,7 @@ void Engine::setup_chains(int K, const int *fold_of_row, int kcap, int max_iter,
     Impl &m = *d_;
     const int n = m.n, p = m.p;
     if (K < 0 || K > MAXC - 1) throw EngineError{"K (nfolds) must be in [0, 31]"};
+    if (m.csc && !m.csc_norm) throw EngineError{"setup_chains: a sparse design must be normalised (or densified) first"};
     if (max_iter < 1 || max_iter > MAX_ITER_CAP) throw EngineError{"max_iter must be in [1, 100000]"};
     const bool grp = grouped();
     if (kcap < 1 || kcap > (grp ? n_groups_ : p_model())) throw EngineError{"support size must be in [1, p]"};
@@ -1510,6 +1630,7 @@ void Engine::setup_chains(int K, const int *fold_of_row, int kcap, int max_iter,
     d.warm = warm_start ? 1 : 0;
     d.sharded = sharded_ ? 1 : 0;
     d.col_lo = sharded_ ? (int)col_lo_ : 0;
+    d.ax_ext = (sharded_ || m.csc_norm) ? 1 : 0;
     d.nmat = family_ == FAM_COX ? 2 : 1;
     d.grouped = grp ? 1 : 0;
     d.N = n_groups_;
@@ -1587,7 +1708,11 @@ void Engine::setup_chains(int K, const int *fold_of_row, int kcap, int max_iter,
         std::memset(h_ind, 0, vsz * 8);
         for (int c = 0; c < C; c++) {
             const double v = grp ? 1.0 / (double)h_ntrain[c] : 1.0;
-            for (int r = 0; r < h_ntrain[c]; r++) h_ind[(size_t)h_rows[(size_t)c * n + r] * d.FS + c] = v;
+            for (int r = 0; r < h_ntrain[c]; r++) {
+                const int i = h_rows[(size_t)c * n + r];
+                // the sparse sweep sees the raw column: the row factors of add_weight enter as rowmul^2
+                h_ind[(size_t)i * d.FS + c] = m.csc_norm ? std::sqrt(m.hw[i]) * std::sqrt(m.hw[i]) : v;
+            }
         }
     }
     // resident path (lm_path.cu): one cooperative launch per path segment when the problem fits
@@ -1694,7 +1819,8 @@ void Engine::setup_chains(int K, const int *fold_of_row, int kcap, int max_iter,
         b.nch = C;
         for (int c = 0; c < C; c++) b.chain[c] = c;
         const int spx = m.span_begin(6);
-        launch_dual_sweep(d, MODE_DH, m.st);
+        if (m.csc_norm) launch_csc_sweep(d, MODE_DH, m.st);
+        else launch_dual_sweep(d, MODE_DH, m.st);
         launch_finish(d, MODE_DH, EPI_RAW, b, m.raw, m.st);
         m.span_end(spx);
         d.W = Wkeep;
@@ -1702,8 +1828,14 @@ void Engine::setup_chains(int K, const int *fold_of_row, int kcap, int max_iter,
         // these chains live)
         d.xtx = m.raw + (size_t)d.FS * d.pstride;
         stats_.n_sweeps++;
-        stats_.norm_bytes += 8.0 * n * p;
-        stats_.kernel_launches += 2;
+        stats_.norm_bytes += m.csc_norm ? 12.0 * (double)m.nnz + 8.0 * ((double)p + 1) + 16.0 * n * d.FS : 8.0 * n * p;
+        stats_.kernel_launches += m.csc_norm ? 3 + (d.nlong ? 1 : 0) : 2;
+    }
+    if (m.csc_norm) {  // the active columns are expanded from the CSC arrays into AXr every iteration (launch_csc_gather)
+        d.AXr = dalloc<double>(m.st, (size_t)C * n * kcap);
+        d.ldXk = kcap;
+        d.AXk = dalloc<double>(m.st, (size_t)C * n * d.ldXk);
+        CUDA_CHECK(cudaMemsetAsync(d.AXk, 0, (size_t)C * n * d.ldXk * 8, m.st));
     }
     if (sharded_) {
         m.cand_s = dalloc<Cand>(m.st, (size_t)C * kcap);
@@ -1904,6 +2036,14 @@ void Engine::run_steps(const std::vector<PathStep> &steps, const std::vector<int
     m.collect_spans();
 }
 
+// Algorithmic bytes of one CSC sweep (launch_csc_sweep): the three CSC arrays, the statistics of every column, the
+// n-vectors of every chain slot (read by the sums kernel and, for cox, the prefix written and read), the partials written.
+static double csc_sweep_bytes(const Dev &d, int mode)
+{
+    const int nv = mode == MODE_D ? 1 : (mode == MODE_DH ? 2 : 4), nq = mode == MODE_D ? 1 : (mode == MODE_DH ? 2 : 5);
+    return 12.0 * (double)d.csc_nnz + 8.0 * ((double)d.p + 1) + 16.0 * d.p + 8.0 * d.n * d.FS * (nv + (mode == MODE_COX ? 2 : 0)) +
+           8.0 * (double)d.p * d.FS * nq;
+}
 static inline int sweep_mode(int family) { return family == FAM_LM ? MODE_D : (family == FAM_COX ? MODE_COX : MODE_DH); }
 static inline int sweep_epi(int family)
 {
@@ -1941,7 +2081,8 @@ static void run_batch_exact(Engine::Impl &m, Engine::Impl::Ticket &t, EngineStat
         if (d.grouped) {
             launch_group_sacrifice(d, b, m.st);
         } else {
-            launch_dual_sweep(d, mode, m.st);
+            if (d.ccp) launch_csc_sweep(d, mode, m.st);
+            else launch_dual_sweep(d, mode, m.st);
             launch_finish(d, mode, epi, b, nullptr, m.st);
         }
         if (m.n_always) launch_pin(d, d.bd + (size_t)cmin * d.pstride, d.pstride, nspan, m.always, m.n_always, m.st);
@@ -1960,9 +2101,10 @@ static void run_batch_exact(Engine::Impl &m, Engine::Impl::Ticket &t, EngineStat
             CUDA_CHECK(cudaStreamSynchronize(m.st));  // hsel is reused
         }
         if (d.grouped) launch_group_expand(d, b, m.st);
+        if (d.ccp) launch_csc_gather(d, b, 0, m.st);
         launch_chain_fit(d, b, m.st);
         t.enq++;
-        stats.kernel_launches += d.grouped ? 4 : 5;
+        stats.kernel_launches += d.grouped ? 4 : (d.ccp ? 7 + (d.nlong ? 1 : 0) : 5);
     }
     enqueue_results(m, t);
 }
@@ -2090,7 +2232,8 @@ static void enqueue_iterations(Engine::Impl &m, Engine::Impl::Ticket &t, int cou
             continue;
         }
         sp = m.span_begin(1);
-        launch_dual_sweep(d, mode, m.st);
+        if (d.ccp) launch_csc_sweep(d, mode, m.st);
+        else launch_dual_sweep(d, mode, m.st);
         m.span_end(sp);
         if (!t.fused) {
             sp = m.span_begin(2);
@@ -2128,6 +2271,7 @@ static void enqueue_iterations(Engine::Impl &m, Engine::Impl::Ticket &t, int cou
         }
         m.span_end(sp);
         sp = m.span_begin(4);
+        if (d.ccp) launch_csc_gather(d, b, 0, m.st);
         launch_chain_fit(d, b, m.st);
         m.span_end(sp);
     }
@@ -2219,9 +2363,9 @@ bool Engine::run_batch_collect(int ticket, BatchResult &out, std::vector<double>
     const int mode = sweep_mode(family_);
     const double vec_bytes = 8.0 * d.n * b.nch * (mode == MODE_D ? 1 : (mode == MODE_DH ? 2 : 4)) + 8.0 * d.p * b.nch;
     const long long per_iter = d.grouped ? 4 + (m.n_always ? 1 : 0)
-                                         : (t.fused ? 3 : 4 + (m.n_always ? 1 : 0) + (sharded_ ? 4 : 0));
+                                         : (t.fused ? 3 : 4 + (m.n_always ? 1 : 0) + (sharded_ ? 4 : 0)) + (d.ccp ? 2 + (d.nlong ? 1 : 0) : 0);
     stats_.n_sweeps += executed;
-    stats_.sweep_bytes += executed * (8.0 * d.n * d.p * (d.grouped ? b.nch : 1) + vec_bytes);
+    stats_.sweep_bytes += executed * (d.ccp ? csc_sweep_bytes(d, mode) : 8.0 * d.n * d.p * (d.grouped ? b.nch : 1) + vec_bytes);
     stats_.kernel_launches += 1 + (long long)executed * per_iter + (t.has_jobs ? 1 : 0);  // gated no-op launches are not counted
     stats_.n_fits += b.nch;
     stats_.n_batches++;
@@ -2293,17 +2437,27 @@ float Engine::time_dual_sweep(int nch, int reps)
     cudaEvent_t e0, e1;
     CUDA_CHECK(cudaEventCreate(&e0));
     CUDA_CHECK(cudaEventCreate(&e1));
-    launch_dual_sweep(m.d, mode, m.st);
+    auto sweep = [&] {
+        if (m.d.ccp) launch_csc_sweep(m.d, mode, m.st);
+        else launch_dual_sweep(m.d, mode, m.st);
+    };
+    sweep();
     CUDA_CHECK(cudaEventRecord(e0, m.st));
-    for (int r = 0; r < reps; r++) launch_dual_sweep(m.d, mode, m.st);
+    for (int r = 0; r < reps; r++) sweep();
     CUDA_CHECK(cudaEventRecord(e1, m.st));
     CUDA_CHECK(cudaStreamSynchronize(m.st));
     float ms = 0.f;
     CUDA_CHECK(cudaEventElapsedTime(&ms, e0, e1));
     cudaEventDestroy(e0);
     cudaEventDestroy(e1);
-    stats_.kernel_launches += reps + 1;
+    stats_.kernel_launches += (long long)(reps + 1) * (m.d.ccp ? 2 + (m.d.nlong ? 1 : 0) : 1);
     return ms / (float)reps;
+}
+
+double Engine::dual_sweep_bytes() const
+{
+    const Dev &d = d_->d;
+    return d.ccp ? csc_sweep_bytes(d, sweep_mode(family_)) : 8.0 * (double)n_ * (double)p_;
 }
 
 // Test hook: recompute the sacrifice of every chain of `chains` for the state the last batch returned, through the
@@ -2339,6 +2493,14 @@ void Engine::debug_sacrifice(const std::vector<int> &chains, double lambda, std:
     if (d.grouped) {
         info_out[0] = 3;
         info_out[5] = launch_group_sacrifice(d, b, m.st);
+    } else if (d.ccp) {
+        info_out[0] = 4;  // the sweep over the CSC arrays
+        info_out[2] = d.csc_g;
+        info_out[5] = d.nlong;  // columns swept by a CTA each
+        info_out[3] = d.S;
+        info_out[4] = d.rows_per_split;
+        launch_csc_sweep(d, mode, m.st);
+        launch_finish(d, mode, epi, b, nullptr, m.st);
     } else {
         info_out[0] = sweep_uses_tma(d) ? 2 : 1;
         info_out[2] = sweep_cpt(d, mode);

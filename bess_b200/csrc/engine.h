@@ -112,6 +112,9 @@ public:
     // the whole CSC design -> the dense row-major n x ldx design a load() of the same matrix holds
     void densify();
     bool sparse() const;
+    // normalize() kept the design sparse: the PDAS sweeps run on the CSC arrays (DESIGN 3.12, "without screening")
+    bool sparse_sweeps() const;
+    size_t device_total_bytes() const;  // cudaDeviceProp::totalGlobalMem of the engine's device
     // per-category device time (CUDA events on the engine's stream): 0 screening sweep (the pass over the raw design),
     // 1 PDAS dual sweeps, 2 finish, 3 top-k, 4 chain kernels, 5 other, 6 normalisation / x_j.x_j passes, 7 host->device upload
     void set_profiling(bool on);
@@ -131,7 +134,8 @@ public:
 
     // ---- Data ctor normalisation (Data.h:41-68, normalize.cpp) + add_weight for gaussian (Data.h:70-77).
     void normalize(int data_type, bool is_normal);
-    // the current dense design (n x p_model(), row-major, without the row padding) -> host; waits for the device
+    // the current dense design (n x p_model(), row-major, without the row padding) -> host; waits for the device.  A sparse
+    // design normalised in place of densifying is expanded to its normalised dense form.
     void copy_design(double *host_out);
 
     // ---- group selection (R: group.index, Python: GroupPdas*).  g_index: first column of every group, ascending from 0
@@ -190,6 +194,8 @@ public:
     // ---- primitives exposed for tests / roofline benchmarking through the C-ABI
     // Dual sweep + sacrifice for `nch` chains (chain slots f0..f0+nch) -> bd on device; returns kernel ms if timed.
     float time_dual_sweep(int nch, int reps);
+    // algorithmic bytes of one such sweep: 8np, or for a sparse design swept on its non-zeros those of launch_csc_sweep
+    double dual_sweep_bytes() const;
     // after run_batch: bd of `chains` for their current model ([nch][p], or [nch][n_groups]); info_out[8] as
     // bessgpu_sacrifice (include/bess_b200.h)
     void debug_sacrifice(const std::vector<int> &chains, double lambda, std::vector<double> &bd_out, int *info_out);
@@ -209,6 +215,7 @@ public:
     struct Impl;
 private:
     void begin_load(int n, int p, int family);
+    void normalize_csc(int data_type, bool is_normal);
     void end_load(const double *y, const double *weight, int family);
     Impl *d_ = nullptr;
     int n_ = 0, p_ = 0, family_ = 0;

@@ -1113,7 +1113,7 @@ __global__ void __launch_bounds__(FIT_NT) loss_kernel(const Dev d, const LossDes
     for (int r = threadIdx.x; r < nr; r += FIT_NT) {
         const int i = rl ? rl[r] : r;
         double eta = d.family == FAM_LM || d.family == FAM_COX ? 0.0 : coef0;
-        if (d.sharded) {
+        if (d.ax_ext) {
             const double *row = d.AXk + ((size_t)c * d.n + i) * d.ldXk;
             for (int a = 0; a < ks; a++) eta = fma(row[a], bsl[a], eta);
         } else {
@@ -1730,6 +1730,397 @@ void launch_screen_csc_lm(const long long *colptr, const int *rowidx, const doub
         case 16: screen_csc_lm_kernel<16><<<grid, 256, 0, st>>>(colptr, rowidx, values, p, y, util); break;
         default: screen_csc_lm_kernel<32><<<grid, 256, 0, st>>>(colptr, rowidx, values, p, y, util); break;
     }
+    CUDA_CHECK(cudaGetLastError());
+}
+
+// ---- sparse design swept on its non-zeros (Dev::ccp).  The design stays in CSC form; the centring and scaling of
+// normalize.cpp are applied implicitly, with the unstored rows' terms summed in closed form.  Every sum is a per-lane
+// sequential sum followed by a fixed shuffle tree: a call is bitwise reproducible.
+
+// mask of the G-lane group of this thread inside its warp (sub-warp shuffles of groups that loop independently)
+template <int G>
+__device__ __forceinline__ unsigned group_mask()
+{
+    if constexpr (G == 32) return 0xffffffffu;
+    else return ((1u << G) - 1u) << ((threadIdx.x & 31) & ~(G - 1));
+}
+template <int G>
+__device__ __forceinline__ double group_sum(double v, unsigned mask)
+{
+#pragma unroll
+    for (int o = G / 2; o > 0; o >>= 1) v += __shfl_xor_sync(mask, v, o, G);
+    return v;
+}
+
+__global__ void __launch_bounds__(256) csc_stats_kernel(const long long *__restrict__ colptr, const int *__restrict__ rowidx,
+                                                        const double *__restrict__ values, int p, const double *g,
+                                                        const double *w, double sumw, double sn, double *mean_out,
+                                                        double *norm_out, double *mul_out)
+{
+    const int lane = threadIdx.x & 31;
+    const long long nw = ((long long)gridDim.x * blockDim.x) >> 5;
+    for (long long j = ((long long)blockIdx.x * blockDim.x + threadIdx.x) >> 5; j < p; j += nw) {
+        const long long b = __ldg(colptr + j), e = __ldg(colptr + j + 1);
+        double m = 0.0;
+        if (g) {
+            for (long long k = b + lane; k < e; k += 32) m = fma(__ldg(values + k), __ldg(g + __ldg(rowidx + k)), m);
+            m = warp_sum(m);
+        }
+        double h = 0.0, ws = 0.0;
+        for (long long k = b + lane; k < e; k += 32) {
+            const double wi = __ldg(w + __ldg(rowidx + k));
+            const double xc = __ldg(values + k) - m;
+            h = fma(xc * xc, wi, h);
+            ws += wi;
+        }
+        h = warp_sum(h);
+        ws = warp_sum(ws);
+        h += m * m * (sumw - ws);
+        if (lane == 0) {
+            const double nx = sqrt(h);
+            mean_out[j] = m;
+            norm_out[j] = nx;
+            mul_out[j] = sn / nx;
+        }
+    }
+}
+void launch_csc_stats(const long long *colptr, const int *rowidx, const double *values, int p, const double *g,
+                      const double *w, double sumw, double sn, double *mean_out, double *norm_out, double *mul_out,
+                      cudaStream_t st)
+{
+    csc_stats_kernel<<<csc_grid(8, p), 256, 0, st>>>(colptr, rowidx, values, p, g, w, sumw, sn, mean_out, norm_out, mul_out);
+    CUDA_CHECK(cudaGetLastError());
+}
+
+// The per-iteration sums the implicit centring needs, one CTA per chain slot: csum[0][f] = sum_i G'_i[f], csum[1][f] =
+// sum_i W_i[f] (gaussian / GLM); cox (no centring): cpre[i][f] = sum_{k <= i} C2_k[f], c2sum[f] = its total.  Each thread
+// owns a contiguous row chunk, so the order of every sum is fixed.
+constexpr int CSUM_NT = 512;
+__global__ void __launch_bounds__(CSUM_NT) csc_sums_kernel(const Dev d, int mode)
+{
+    __shared__ double red[40];
+    if (d.gate && *d.gate == 0) return;
+    const int f = blockIdx.x, FS = d.FS, n = d.n;
+    const int per = (n + CSUM_NT - 1) / CSUM_NT;
+    const int r0 = min(n, (int)threadIdx.x * per), r1 = min(n, r0 + per);
+    if (mode == MODE_COX) {
+        double s = 0.0;
+        for (int i = r0; i < r1; i++) s += d.C2[(size_t)i * FS + f];
+        double tot;
+        double run = block_excl_scan<CSUM_NT>(s, red, &tot);
+        for (int i = r0; i < r1; i++) {
+            run += d.C2[(size_t)i * FS + f];
+            d.cpre[(size_t)i * FS + f] = run;
+        }
+        if (threadIdx.x == 0) d.c2sum[f] = tot;
+        return;
+    }
+    const double *rm = mode == MODE_D ? d.crm : nullptr;
+    double sg = 0.0, sw = 0.0;
+    for (int i = r0; i < r1; i++) {
+        const double gi = d.G[(size_t)i * FS + f];
+        sg += rm ? rm[i] * gi : gi;
+        if (mode == MODE_DH) sw += d.W[(size_t)i * FS + f];
+    }
+    sg = block_sum<CSUM_NT>(sg, red);
+    sw = block_sum<CSUM_NT>(sw, red);
+    if (threadIdx.x == 0) {
+        d.csum[f] = sg;
+        d.csum[FS + f] = sw;
+    }
+}
+
+// The dual sweep over the CSC arrays.  With x~ = (x - m) mul rm and G' = rm o G, per column j and chain slot f:
+//   MODE_D   d = mul (sum_stored x G' - m sum_i G'_i)
+//   MODE_DH  d as in MODE_D (rm = 1), h = mul^2 (sum_stored (x - m)^2 W + m^2 (sum_i W_i - sum_stored W))
+//   MODE_COX (m = 0) d, h as above; s1 = mul sum_stored TH x; R = mul^2 sum_t (P_{i_t} - P_{i_{t-1}}) S_t^2 with S_t the
+//            suffix of TH x over the column's entries from t and P the row prefix of C2 (s1_k is constant between stored
+//            rows); B = mul sum_t (P_{i_t} - P_{i_{t-1}}) S_t
+// The partials land where dual_sweep_kernel writes them with S = 1: part[(q * FT + f) * pstride + j].
+// Work split: columns of at most Dev::clong_thr entries are walked by G lanes each (csc_sweep_kernel, G from the mean
+// column length); longer ones -- the frequent terms of a power-law design -- by a whole CTA each (csc_sweep_long_kernel),
+// its warps owning fixed consecutive segments whose sums are combined in a fixed order.
+template <int FT, int MODE>
+__host__ __device__ constexpr int csc_fc() { return MODE == MODE_COX ? (FT < 4 ? FT : 4) : (FT < 8 ? FT : 8); }
+
+// The sums of the entries [k0, k1) of a column that starts at entry b (the Cox dP of entry k reads row k - 1 when k > b),
+// for chain slots fb .. fb + FC - 1, by the G lanes of `mask`.  Cox: the entries are walked in chunks of G from k1 down,
+// carry[f] enters as the suffix of the entries after k1 and leaves as the suffix from k0.  Per-lane partials: the caller
+// reduces them.
+template <int FT, int MODE, int G>
+__device__ __forceinline__ void csc_range(const Dev &d, long long b, long long k0, long long k1, int fb, double mj, int lane,
+                                          unsigned mask, double (&ad)[csc_fc<FT, MODE>()], double (&ah)[csc_fc<FT, MODE>()],
+                                          double (&aw)[csc_fc<FT, MODE>()], double (&aR)[csc_fc<FT, MODE>()],
+                                          double (&aB)[csc_fc<FT, MODE>()], double (&carry)[csc_fc<FT, MODE>()])
+{
+    constexpr int FC = csc_fc<FT, MODE>();
+    const double *rm = MODE == MODE_D ? d.crm : nullptr;
+    if constexpr (MODE != MODE_COX) {
+        for (long long k = k0 + lane; k < k1; k += G) {
+            const int i = __ldg(d.cri + k);
+            const double x = __ldg(d.ccv + k);
+            const double r = rm ? __ldg(rm + i) : 1.0;
+            const double xc = x - mj;
+#pragma unroll
+            for (int f = 0; f < FC; f++) {
+                if (fb + f < FT) {
+                    const double gi = __ldg(d.G + (size_t)i * FT + fb + f);
+                    ad[f] = fma(x, rm ? r * gi : gi, ad[f]);
+                    if constexpr (MODE == MODE_DH) {
+                        const double wi = __ldg(d.W + (size_t)i * FT + fb + f);
+                        ah[f] = fma(xc * xc, wi, ah[f]);
+                        aw[f] += wi;
+                    }
+                }
+            }
+        }
+    } else {
+        const long long nck = (k1 - k0 + G - 1) / G;
+        for (long long q = nck - 1; q >= 0; q--) {
+            const long long k = k0 + q * G + lane;
+            const bool valid = k < k1;
+            const int i = valid ? __ldg(d.cri + k) : 0;
+            const int ip = (valid && k > b) ? __ldg(d.cri + k - 1) : -1;
+            const double x = valid ? __ldg(d.ccv + k) : 0.0;
+#pragma unroll
+            for (int f = 0; f < FC; f++) {
+                if (fb + f < FT) {
+                    const size_t o = (size_t)i * FT + fb + f;
+                    const double v = valid ? x * __ldg(d.TH + o) : 0.0;
+                    double s = v;
+#pragma unroll
+                    for (int sh = 1; sh < G; sh <<= 1) {
+                        const double t = __shfl_down_sync(mask, s, sh, G);
+                        if (lane + sh < G) s += t;
+                    }
+                    const double S = s + carry[f];
+                    carry[f] += __shfl_sync(mask, s, 0, G);
+                    if (valid) {
+                        const double dP = d.cpre[o] - (ip >= 0 ? d.cpre[(size_t)ip * FT + fb + f] : 0.0);
+                        aR[f] = fma(dP * S, S, aR[f]);
+                        aB[f] = fma(dP, S, aB[f]);
+                        ad[f] = fma(x, __ldg(d.G + o), ad[f]);
+                        ah[f] = fma(x * x, __ldg(d.W + o), ah[f]);
+                    }
+                }
+            }
+        }
+    }
+}
+
+// the partials of column j, slot ff from its reduced sums
+template <int FT, int MODE>
+__device__ __forceinline__ void csc_put(const Dev &d, long long j, int ff, double mj, double mu, double ad, double ah,
+                                        double aw, double aR, double aB, double s1)
+{
+    auto put = [&](int qq, double v) { d.part[((size_t)qq * FT + ff) * d.pstride + j] = v; };
+    if constexpr (MODE == MODE_COX) {
+        put(0, mu * ad);
+        put(1, mu * mu * ah);
+        put(2, mu * s1);
+        put(3, mu * mu * aR);
+        put(4, mu * aB);
+    } else {
+        put(0, mu * (ad - mj * d.csum[ff]));
+        if constexpr (MODE == MODE_DH) put(1, mu * mu * (ah + mj * mj * (d.csum[FT + ff] - aw)));
+    }
+}
+
+template <int FT, int MODE, int G>
+__global__ void __launch_bounds__(256, 1) csc_sweep_kernel(const Dev d)
+{
+    constexpr int FC = csc_fc<FT, MODE>();
+    if (d.gate && *d.gate == 0) return;
+    const int lane = threadIdx.x & (G - 1);
+    const unsigned mask = group_mask<G>();
+    const long long per_pass = ((long long)gridDim.x * blockDim.x) / G;
+    for (long long j = ((long long)blockIdx.x * blockDim.x + threadIdx.x) / G; j < d.p; j += per_pass) {
+        const long long b = __ldg(d.ccp + j), e = __ldg(d.ccp + j + 1);
+        if (e - b > d.clong_thr) continue;  // csc_sweep_long_kernel's column
+        const double mj = MODE == MODE_COX ? 0.0 : d.cmean[j];
+        const double mu = d.cmul[j];
+#pragma unroll 1
+        for (int fb = 0; fb < FT; fb += FC) {
+            double ad[FC], ah[FC], aw[FC], aR[FC], aB[FC], carry[FC];
+#pragma unroll
+            for (int f = 0; f < FC; f++) ad[f] = ah[f] = aw[f] = aR[f] = aB[f] = carry[f] = 0.0;
+            csc_range<FT, MODE, G>(d, b, b, e, fb, mj, lane, mask, ad, ah, aw, aR, aB, carry);
+#pragma unroll
+            for (int f = 0; f < FC; f++) {
+                if (fb + f >= FT) continue;
+                ad[f] = group_sum<G>(ad[f], mask);
+                if constexpr (MODE >= MODE_DH) ah[f] = group_sum<G>(ah[f], mask);
+                if constexpr (MODE == MODE_DH) aw[f] = group_sum<G>(aw[f], mask);
+                if constexpr (MODE == MODE_COX) {
+                    aR[f] = group_sum<G>(aR[f], mask);
+                    aB[f] = group_sum<G>(aB[f], mask);
+                }
+                if (lane == 0) csc_put<FT, MODE>(d, j, fb + f, mj, mu, ad[f], ah[f], aw[f], aR[f], aB[f], carry[f]);
+            }
+        }
+    }
+}
+
+// One CTA per long column (Dev::clong): warp w owns the entries [b + w seg, b + (w + 1) seg).  The warps' sums are added
+// in warp order; for Cox a first pass gives every segment's suffix total, so that each warp starts its scan with the
+// suffix of the segments after it (added from the last segment down).
+constexpr int CSC_LONG_NT = 256;
+template <int FT, int MODE>
+__global__ void __launch_bounds__(CSC_LONG_NT, 1) csc_sweep_long_kernel(const Dev d)
+{
+    constexpr int FC = csc_fc<FT, MODE>();
+    constexpr int NW = CSC_LONG_NT / 32;
+    __shared__ double red[4][FC][NW];
+    __shared__ double cin[FC][NW];
+    if (d.gate && *d.gate == 0) return;
+    const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
+    const long long j = d.clong[blockIdx.x];
+    const long long b = __ldg(d.ccp + j), e = __ldg(d.ccp + j + 1);
+    const long long seg = (e - b + NW - 1) / NW;
+    const long long k0 = min(e, b + wid * seg), k1 = min(e, k0 + seg);
+    const double mj = MODE == MODE_COX ? 0.0 : d.cmean[j];
+    const double mu = d.cmul[j];
+#pragma unroll 1
+    for (int fb = 0; fb < FT; fb += FC) {
+        double ad[FC], ah[FC], aw[FC], aR[FC], aB[FC], carry[FC];
+#pragma unroll
+        for (int f = 0; f < FC; f++) ad[f] = ah[f] = aw[f] = aR[f] = aB[f] = carry[f] = 0.0;
+        if constexpr (MODE == MODE_COX) {
+            // pass 1: the segment's own suffix total
+            csc_range<FT, MODE, 32>(d, b, k0, k1, fb, mj, lane, 0xffffffffu, ad, ah, aw, aR, aB, carry);
+            if (lane == 0)
+#pragma unroll
+                for (int f = 0; f < FC; f++) cin[f][wid] = carry[f];
+            __syncthreads();
+#pragma unroll
+            for (int f = 0; f < FC; f++) {
+                double c = 0.0;
+                for (int w2 = NW - 1; w2 > wid; w2--) c += cin[f][w2];
+                ad[f] = ah[f] = aR[f] = aB[f] = 0.0;
+                carry[f] = c;
+            }
+            __syncthreads();
+        }
+        csc_range<FT, MODE, 32>(d, b, k0, k1, fb, mj, lane, 0xffffffffu, ad, ah, aw, aR, aB, carry);
+#pragma unroll
+        for (int f = 0; f < FC; f++) {
+            if (fb + f >= FT) continue;
+            const double v[4] = {warp_sum(ad[f]), warp_sum(ah[f]), warp_sum(MODE == MODE_COX ? aR[f] : aw[f]),
+                                 warp_sum(aB[f])};
+            if (lane == 0)
+#pragma unroll
+                for (int q = 0; q < 4; q++) red[q][f][wid] = v[q];
+            if (MODE == MODE_COX && wid == 0 && lane == 0) cin[f][0] = carry[f];  // suffix from the column's first entry
+        }
+        __syncthreads();
+        if (threadIdx.x < FC && fb + (int)threadIdx.x < FT) {
+            const int f = threadIdx.x;
+            double t[4] = {0.0, 0.0, 0.0, 0.0};
+            for (int w2 = 0; w2 < NW; w2++)
+#pragma unroll
+                for (int q = 0; q < 4; q++) t[q] += red[q][f][w2];
+            if constexpr (MODE == MODE_COX) csc_put<FT, MODE>(d, j, fb + f, mj, mu, t[0], t[1], 0.0, t[2], t[3], cin[f][0]);
+            else csc_put<FT, MODE>(d, j, fb + f, mj, mu, t[0], t[1], t[2], 0.0, 0.0, 0.0);
+        }
+        __syncthreads();
+    }
+}
+
+template <int FT, int MODE>
+static void launch_csc_sweep_t(const Dev &d, cudaStream_t st)
+{
+    switch (d.csc_g) {
+        case 2: csc_sweep_kernel<FT, MODE, 2><<<csc_grid(128, d.p), 256, 0, st>>>(d); break;
+        case 8: csc_sweep_kernel<FT, MODE, 8><<<csc_grid(32, d.p), 256, 0, st>>>(d); break;
+        default: csc_sweep_kernel<FT, MODE, 32><<<csc_grid(8, d.p), 256, 0, st>>>(d); break;
+    }
+    if (d.nlong > 0) csc_sweep_long_kernel<FT, MODE><<<d.nlong, CSC_LONG_NT, 0, st>>>(d);
+}
+template <int MODE>
+static void launch_csc_sweep_m(const Dev &d, cudaStream_t st)
+{
+    switch (d.FS) {
+        case 1: launch_csc_sweep_t<1, MODE>(d, st); break;
+        case 2: launch_csc_sweep_t<2, MODE>(d, st); break;
+        case 4: launch_csc_sweep_t<4, MODE>(d, st); break;
+        case 6: launch_csc_sweep_t<6, MODE>(d, st); break;
+        case 8: launch_csc_sweep_t<8, MODE>(d, st); break;
+        case 12: launch_csc_sweep_t<12, MODE>(d, st); break;
+        case 16: launch_csc_sweep_t<16, MODE>(d, st); break;
+        case 24: launch_csc_sweep_t<24, MODE>(d, st); break;
+        case 32: launch_csc_sweep_t<32, MODE>(d, st); break;
+        default: throw EngineError{"csc sweep: unsupported chain tile FS=" + std::to_string(d.FS)};
+    }
+}
+void launch_csc_sweep(const Dev &d, int mode, cudaStream_t st)
+{
+    csc_sums_kernel<<<d.FS, CSUM_NT, 0, st>>>(d, mode);
+    CUDA_CHECK(cudaGetLastError());
+    if (mode == MODE_D) launch_csc_sweep_m<MODE_D>(d, st);
+    else if (mode == MODE_DH) launch_csc_sweep_m<MODE_DH>(d, st);
+    else launch_csc_sweep_m<MODE_COX>(d, st);
+    CUDA_CHECK(cudaGetLastError());
+}
+
+// the columns with more than thr entries (their order does not matter: each is summed by its own CTA)
+__global__ void __launch_bounds__(256) csc_long_list_kernel(const long long *__restrict__ colptr, int p, long long thr,
+                                                            int *list, int *count)
+{
+    for (long long j = (long long)blockIdx.x * blockDim.x + threadIdx.x; j < p; j += (long long)gridDim.x * blockDim.x)
+        if (__ldg(colptr + j + 1) - __ldg(colptr + j) > thr) list[atomicAdd(count, 1)] = (int)j;
+}
+void launch_csc_long_list(const long long *colptr, int p, long long thr, int *list, int *count, cudaStream_t st)
+{
+    csc_long_list_kernel<<<csc_grid(256, p), 256, 0, st>>>(colptr, p, thr, list, count);
+    CUDA_CHECK(cudaGetLastError());
+}
+
+// column j of the implicit normalised design into out[i * ld] for all n rows: every row first gets the value of an unstored
+// entry, then the stored rows theirs; per element the expression of center_scale_kernel's two passes, ((x - m) mul) rm
+__device__ __forceinline__ void csc_column_out(const Dev &d, int j, double *out, long long ld, int lane)
+{
+    const double mj = d.cmean[j], mu = d.cmul[j];
+    const double z = (0.0 - mj) * mu;
+    for (int i = lane; i < d.n; i += 32) out[(size_t)i * ld] = z * (d.crm ? d.crm[i] : 1.0);
+    __syncwarp();
+    const long long b = __ldg(d.ccp + j), e = __ldg(d.ccp + j + 1);
+    for (long long k = b + lane; k < e; k += 32) {
+        const int i = __ldg(d.cri + k);
+        out[(size_t)i * ld] = ((__ldg(d.ccv + k) - mj) * mu) * (d.crm ? d.crm[i] : 1.0);
+    }
+}
+__global__ void __launch_bounds__(256) csc_gather_kernel(const Dev d, const BatchDesc b, int which)
+{
+    const int c = b.chain[blockIdx.y];
+    if (which == 0) {
+        if (d.gate && *d.gate == 0) return;
+        if (d.done[c]) return;
+    }
+    const int cnt = which == 0 ? b.T : d.ks[c];
+    const int a = blockIdx.x * 8 + (threadIdx.x >> 5);
+    if (a >= cnt) return;
+    const int j = (which == 0 ? d.Anew : d.A)[(size_t)c * d.kcap + a];
+    const long long ld = which == 0 ? d.ldXr : d.ldXk;
+    double *out = (which == 0 ? d.AXr : d.AXk) + (size_t)c * d.n * ld + a;
+    csc_column_out(d, j, out, ld, threadIdx.x & 31);
+}
+void launch_csc_gather(const Dev &d, const BatchDesc &b, int which, cudaStream_t st)
+{
+    const int cols = which == 0 ? b.T : d.kcap;
+    if (cols <= 0) return;
+    dim3 grid((unsigned)((cols + 7) / 8), (unsigned)b.nch);
+    csc_gather_kernel<<<grid, 256, 0, st>>>(d, b, which);
+    CUDA_CHECK(cudaGetLastError());
+}
+__global__ void __launch_bounds__(256) csc_expand_kernel(const Dev d, double *out, long long ld)
+{
+    const long long nw = ((long long)gridDim.x * blockDim.x) >> 5;
+    for (long long j = ((long long)blockIdx.x * blockDim.x + threadIdx.x) >> 5; j < d.p; j += nw)
+        csc_column_out(d, (int)j, out + j, ld, threadIdx.x & 31);
+}
+void launch_csc_expand(const Dev &d, double *out, long long ld, cudaStream_t st)
+{
+    csc_expand_kernel<<<csc_grid(8, d.p), 256, 0, st>>>(d, out, ld);
     CUDA_CHECK(cudaGetLastError());
 }
 

@@ -83,6 +83,21 @@ struct Dev {
     int *AnewCols;      // [MAXC][kcap] those columns (find_ind, utilities.cpp:113-130)
     int sharded;
     int col_lo;
+    int ax_ext;         // X_A comes from AXr (column-sharded mode, sparse design): chain_fit gathers its train rows from
+                        // there and keeps AXk; the loss kernel reads AXk
+    // sparse design swept on its non-zeros (ccp != nullptr; X unused): the design the fits see is the implicit
+    // x~_ij = ((x_ij - cmean[j]) * cmul[j]) * crm[i] (crm == nullptr: 1), an unstored x_ij reading 0
+    const long long *ccp;
+    const int *cri;
+    const double *ccv;
+    const double *cmean, *cmul, *crm;
+    double *csum;       // [2][FS] per-iteration sums of the CSC sweep: 0 = sum_i G'_i (G' = crm o G in MODE_D), 1 = sum_i W_i
+    double *cpre;       // [n][FS] cox: prefix sums of C2 over the rows (inclusive)
+    int csc_g;          // lanes per column of the CSC sweep (2, 8 or 32)
+    long long clong_thr;// columns with more entries are swept by a CTA each ...
+    const int *clong;   // ... these [nlong]
+    int nlong;
+    long long csc_nnz;
     double *AXr;        // [MAXC][n][ldXr] active columns of this iteration for ALL rows, summed over ranks (ldXr = T)
     double *AXk;        // [MAXC][n][ldXk] all-row active columns of each chain's CURRENT support (losses)
     int ldXr, ldXk;
@@ -212,6 +227,21 @@ void launch_screen_csc_lm(const long long *colptr, const int *rowidx, const doub
 // screen_glm_kernel with a CSC column reader (absent rows read as 0.0): the same arithmetic in the same order
 void launch_screen_glm_csc(const long long *colptr, const int *rowidx, const double *values, int n, int p, const double *y,
                            const double *w, int family, double *util, cudaStream_t st);
+// ---- sparse design swept on its non-zeros (Dev::ccp; DESIGN 3.12 "without screening")
+// column statistics of normalize.cpp:20-86 over the stored entries: mean_j = sum_stored x g (g = w / n; nullptr: no centring,
+// mean 0), norm_j = sqrt(sum_stored w (x - m)^2 + m^2 (sumw - sum_stored w)), mul_j = sn / norm_j
+void launch_csc_stats(const long long *colptr, const int *rowidx, const double *values, int p, const double *g,
+                      const double *w, double sumw, double sn, double *mean_out, double *norm_out, double *mul_out,
+                      cudaStream_t st);
+// the sums of the sweep vectors (Dev::csum, Dev::cpre) and the sweep itself: the partials of dual_sweep_kernel with S = 1
+void launch_csc_sweep(const Dev &d, int mode, cudaStream_t st);
+// list[0, *count) <- the columns with more than thr entries (any order); *count must be zero on entry
+void launch_csc_long_list(const long long *colptr, int p, long long thr, int *list, int *count, cudaStream_t st);
+// which 0: AXr[c] <- x~ of the columns Anew[c][0, T) for all rows (gated; chains that are done skip);
+// which 1: AXk[c] <- x~ of the columns A[c][0, ks[c]) (the chain's stored support)
+void launch_csc_gather(const Dev &d, const BatchDesc &b, int which, cudaStream_t st);
+// out[i * ld + q] = x~_{i, q} for every column q < p (the normalised dense design)
+void launch_csc_expand(const Dev &d, double *out, long long ld, cudaStream_t st);
 // device-side gen.data design (gen_design.cu): X[i][j], row-major n x p with leading dimension ld
 void launch_gen_design(double *X, long long ld, int n, long long p, double rho, unsigned long long seed, cudaStream_t st);
 void launch_gen_design_cortype(double *X, long long ld, int n, long long p, double rho, unsigned long long seed, int cortype,

@@ -1528,6 +1528,7 @@ bool lm_path_eligible(const Dev &d, int max_iter, int sm_count, std::string *why
     if (d.family != FAM_LM) return no("family is not gaussian");
     if (d.grouped) return no("group selection");
     if (d.sharded) return no("column-sharded mode");
+    if (d.ccp) return no("sparse design (swept on its non-zeros)");
     if (d.kcap > LP_KMAX) return no("support larger than 64");
     if (d.kcap > d.p) return no("support larger than p");
     if (sm_count < MAXC + 8) return no("too few SMs");

@@ -766,6 +766,20 @@ void fold_shard_chains(int K, int world, int rank, bool last_fold_everywhere, st
     }
 }
 
+// Where a sparse design without screening is swept: on its CSC arrays (the dual sweep reads 12 bytes per stored entry, the
+// fits read the active columns expanded from them) or densified (8 bytes per entry, stored or not, read by every sweep).
+// Small designs stay dense: every one up to 1 GiB, which includes every design of the resident path (64 MB).  Larger
+// ones keep the CSC form when it is at most 1 / KEEP_SPARSE_RATIO of the dense bytes -- the crossover measured in
+// DESIGN 3.12 -- or when the dense form could not fit the device at all.  The device's total memory decides, not its
+// free memory, so that a call's numerics never depend on what other jobs hold.
+constexpr double KEEP_SPARSE_RATIO = 24.0;
+bool keep_sparse(long long n, long long p, long long nnz, size_t device_total)
+{
+    const double dense = 8.0 * (double)n * (double)(((p + 1) & ~1LL));
+    const double sparse = 12.0 * (double)nnz + 8.0 * ((double)p + 1);
+    return (dense > (double)(1LL << 30) && sparse * KEEP_SPARSE_RATIO <= dense) || dense > (double)device_total;
+}
+
 static void bess_run_once(const BessArgs &a, BessResult &out, bool tie_exact)
 {
     // ---- argument validation (the reference validates in its R/Python front-ends and dereferences null otherwise,
@@ -825,7 +839,9 @@ static void bess_run_once(const BessArgs &a, BessResult &out, bool tie_exact)
     else if (a.fold_shard && a.world > 1 && a.is_cv) eng.init_comm(a.world, a.rank, a.nccl_id);
     if (a.csc) {
         eng.load_csc(a.csc_colptr, a.csc_rowidx, a.csc_values, a.n, a.p, a.csc_nnz, a.x_on_device, a.y, a.weight, a.model_type);
-        if (!a.is_screening) eng.densify();  // screening densifies only the columns it keeps
+        // screening densifies only the columns it keeps; without it the design is densified unless the sweeps run on the
+        // CSC arrays (keep_sparse)
+        if (!a.is_screening && (grouped || !keep_sparse(a.n, a.p, a.csc_nnz, eng.device_total_bytes()))) eng.densify();
     } else {
         eng.load(a.x, a.n, a.p, a.x_on_device, a.y, a.weight, a.model_type, /*borrow=*/a.is_screening);
     }
@@ -900,6 +916,7 @@ static void bess_run_once(const BessArgs &a, BessResult &out, bool tie_exact)
     }
     for (auto &A : out.A_all)
         for (int &j : A) j = orig(j);
+    out.sparse_sweeps = eng.sparse_sweeps();
     out.stats = eng.stats();
     out.stats.n_rank_deficient += debug_take_rankdef();
     out.stats.n_wide_singular += take_wide_singular();

@@ -86,6 +86,7 @@ struct BessResult {
     double prof_ms[PROF_NCAT] = {};
     long long prof_n[PROF_NCAT] = {};
     int sweep_splits = 1;
+    bool sparse_sweeps = false;   // the PDAS sweeps ran on the CSC arrays of a sparse design (keep_sparse)
     bool tie_exact_pass = false;  // the call met a boundary tie and was repeated with host-resolved selections
     bool robust_pass = false;     // the fast pass met a dependent active column (or a non-finite result) and the call was
                                   // repeated on the multi-kernel path, whose solver is rank-revealing
@@ -109,5 +110,7 @@ void fold_shard_chains(int K, int world, int rank, bool last_fold_everywhere, st
 
 // throws EngineError
 void bess_run(const BessArgs &a, BessResult &out);
+// a sparse design without screening (and without groups) keeps its CSC form for the PDAS sweeps (DESIGN 3.12)
+bool keep_sparse(long long n, long long p, long long nnz, size_t device_total);
 
 }  // namespace bess

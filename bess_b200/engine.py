@@ -156,9 +156,9 @@ class GpuEngine:
         bd = np.zeros((ch.size, N))
         info = np.zeros(8, dtype=np.int32)
         _lib.check(self._lib.bessgpu_sacrifice(self._h, _i(ch), ch.size, float(lam), _d(bd), _i(info)))
-        kind = {1: "stream", 2: "tma", 3: "group"}[int(info[0])]
+        kind = {1: "stream", 2: "tma", 3: "group", 4: "csc"}[int(info[0])]
         return bd, dict(kernel=kind, FS=int(info[1]), CPT=int(info[2]), S=int(info[3]), rows_per_split=int(info[4]),
-                        groups=int(info[5]))
+                        groups=int(info[5]), long_columns=int(info[5]) if kind == "csc" else 0)
 
     def stats(self):
         o = np.zeros(8)

@@ -75,7 +75,9 @@ typedef struct bess_b200_ext {
     int *screening_A_out;     /* [screening_size] kept columns, ascending (List key "screening_A", bess.cpp:199)     */
     int *chosen_s_out;        /* sparsity level of the returned model                                                 */
     double *stats_out;        /* [32]: 0 n_fits, 1 n_pdas_iters, 2 n_sweeps, 3 n_batches, 4 n_boundary_ties,          */
-                              /*  5 PDAS dual-sweep algorithmic bytes, 6 kernel_launches, 7 trace_len,                */
+                              /*  5 PDAS dual-sweep algorithmic bytes (8np + vectors per sweep; sweeps on the CSC      */
+                              /*  arrays: 12 nnz + 8 (p + 1) + the column statistics + the n-vectors read + the        */
+                              /*  partials written), 6 kernel_launches, 7 trace_len,                                   */
                               /*  8..15 device ms per kernel category (profile != 0): screening sweep, PDAS dual      */
                               /*  sweeps, finish, top-k, chain kernels, other, normalisation passes, H2D upload;      */
                               /*  16..23 launches per category; 24 algorithmic bytes of the screening sweep (8np;     */
@@ -116,9 +118,13 @@ typedef struct bess_b200_ext {
                                 /* returns the same model, bit-identical to the single-GPU call                               */
     const bess_b200_csc *x_csc; /* non-NULL: the design is sparse (see bess_b200_csc); x must then be NULL, x_row / x_col give */
                                 /* n and p, and x_on_device = 1 means the three arrays are device pointers (read in place,   */
-                                /* never written).  Screening densifies only the kept columns; without screening the whole    */
-                                /* design is densified on the device (n * p * 8 bytes must fit).  Single GPU only (world <= 1); */
-                                /* screening together with groups is refused as for dense designs                             */
+                                /* never written).  Screening densifies only the kept columns.  Without screening and groups, */
+                                /* a design whose dense form is over 1 GiB and at least 24 times its CSC bytes (12 nnz +      */
+                                /* 8 (p + 1)), or larger than the device's memory, is swept on its non-zeros and only the     */
+                                /* active columns are expanded; any other is densified on the device (n * p * 8 bytes must    */
+                                /* fit).  Single GPU only (world <= 1); screening together with groups is refused as for      */
+                                /* dense designs                                                                              */
+    int *sparse_sweeps_out;     /* 1 when the call's PDAS sweeps ran on the CSC arrays of x_csc, else 0; may be NULL          */
 } bess_b200_ext;
 
 /* Same arguments and outputs as pywrap_bess, returns 0 on success.  The per-level trace of the call (what the reference's
@@ -209,9 +215,9 @@ int bessgpu_time_dual_sweep(bessgpu_handle *h, int reps, float *ms_out, double *
 /* test probe, after a batch returned: the sacrifice of every chain of `chains` for its current model (gradient vectors
  * published again from the chain's support, coefficients and intercept), through the dispatch a fit of this batch uses,
  * at ridge level `lambda`.  bd_out: [nch][p], or [nch][number of groups] with groups.  info_out[8]: [0] what ran (1
- * streaming column sweep, 2 bulk-TMA column sweep, 3 group kernels), [1] chain slots FS, [2] columns per thread, [3] row
- * splits, [4] rows per split, [5] group kernels launched (bits: 1 serial, 2 warp, 4 / 8 / 16 batched for widths <= 2 /
- * 4 / 8, 32 wide) */
+ * streaming column sweep, 2 bulk-TMA column sweep, 3 group kernels, 4 the sweep over a sparse design's CSC arrays),
+ * [1] chain slots FS, [2] columns per thread (4: lanes per column), [3] row splits, [4] rows per split, [5] group kernels
+ * launched (bits: 1 serial, 2 warp, 4 / 8 / 16 batched for widths <= 2 / 4 / 8, 32 wide; 4: columns swept by a CTA each) */
 int bessgpu_sacrifice(bessgpu_handle *h, const int *chains, int nch, double lambda, double *bd_out, int *info_out);
 int bessgpu_stats(bessgpu_handle *h, double *out8);
 /* stand-alone exact top-k (utilities.cpp:179-188 max_k): host vals[n] -> ascending indices; tie_out = 1 when keys equal to
