@@ -33,6 +33,7 @@
 #include <cfloat>
 #include <cmath>
 #include <cstdlib>
+#include <type_traits>
 
 #include "device_utils.cuh"
 #include "lm_path.cuh"
@@ -123,68 +124,93 @@ __device__ __forceinline__ void fence_acq_rel_gpu() { asm volatile("fence.acq_re
 
 // The CTA's writes so far (ordered before thread 0's release by the block barrier) become visible to whoever acquires
 // the counter afterwards.
-__device__ __forceinline__ void cta_arrive(unsigned *ctr)
+__device__ __forceinline__ void cta_arrive(unsigned *ctr, unsigned add = 1u)
 {
     __syncthreads();
-    if (threadIdx.x == 0) red_release_add_u32(ctr, 1u);
+    if (threadIdx.x == 0) red_release_add_u32(ctr, add);
 }
-// Thread 0 polls up to three counters with RELAXED loads (an acquire load invalidates the L1 on every poll) and fences
-// once when all have reached their targets.  Returns false when the launch was aborted (by this or another CTA's watchdog).
-__device__ __forceinline__ bool cta_wait3(unsigned *sync, int w0, unsigned t0, int w1, unsigned t1, int w2, unsigned t2,
-                                          int *flag_sh)
+// The owner that sets LP_SYNC_TERM adds this flag with its next arrival at B2.  A waiter that reads no flag in the counters
+// of its decision point knows, without reading the termination word, that no phase up to that point has set it.
+constexpr unsigned LP_TERM_FLAG = 1u << 31;
+// Thread 0 polls counters with RELAXED loads (an acquire load invalidates the L1 on every poll) and fences once when all
+// have reached their targets.  The abort word is loaded with the counters, not after them: one L2 round trip per poll.
+// *flags <- LP_TERM_FLAG when a counter carried it.  Returns false when the launch was aborted (by this or another CTA's
+// watchdog).
+__device__ __forceinline__ bool poll_until(unsigned *sync, int w0, unsigned t0, int w1, unsigned t1, unsigned *flags)
 {
-    if (threadIdx.x == 0) {
-        int ok = 1;
-        unsigned spins = 0;
-        unsigned long long ts = 0;
-        for (;;) {
-            const bool r0 = ld_relaxed_u32(sync + w0) >= t0;
-            const bool r1 = w1 < 0 || ld_relaxed_u32(sync + w1) >= t1;
-            const bool r2 = w2 < 0 || ld_relaxed_u32(sync + w2) >= t2;
-            if (r0 && r1 && r2) break;
-            if ((++spins & 0x3ffu) == 0u) {
-                if (ts == 0) ts = lp_globaltimer();
-                if (ld_relaxed_u32(sync + LP_SYNC_ABORT) != 0u || lp_globaltimer() - ts > LP_WATCHDOG_NS) {
-                    atomicExch(sync + LP_SYNC_ABORT, 1u);
-                    ok = 0;
-                    break;
-                }
+    unsigned spins = 0;
+    unsigned long long ts = 0;
+    for (;;) {
+        const unsigned v0 = ld_relaxed_u32(sync + w0);
+        const unsigned v1 = w1 < 0 ? t1 : ld_relaxed_u32(sync + w1);
+        if (ld_relaxed_u32(sync + LP_SYNC_ABORT) != 0u) return false;
+        if ((v0 & ~LP_TERM_FLAG) >= t0 && (v1 & ~LP_TERM_FLAG) >= t1) {
+            *flags = (v0 | v1) & LP_TERM_FLAG;
+            break;
+        }
+        if ((++spins & 0x3ffu) == 0u) {
+            if (ts == 0) ts = lp_globaltimer();
+            if (lp_globaltimer() - ts > LP_WATCHDOG_NS) {
+                atomicExch(sync + LP_SYNC_ABORT, 1u);
+                return false;
             }
         }
-        if (ok && ld_relaxed_u32(sync + LP_SYNC_ABORT) != 0u) ok = 0;
-        fence_acq_rel_gpu();
-        *flag_sh = ok;
+    }
+    fence_acq_rel_gpu();
+    return true;
+}
+// The CTA waits for counters w0 / w1 (w1 < 0: none), then decides: LP_WAIT_TERM when the termination word holds a phase
+// index at or below `decision` (see sweeper_main); else, when wb >= 0, it waits for counter wb as well.  Every phase up to
+// `decision` has arrived on w0 / w1 by then (the owner that sets the word arrives with LP_TERM_FLAG), or on a counter of an
+// earlier decision point of this CTA, at which it would have left; so the word is read only when a counter carries the
+// flag.  Thread 0 does all of it and hands the outcome to the CTA through one block barrier pair.
+enum { LP_WAIT_ABORT = 0, LP_WAIT_GO = 1, LP_WAIT_TERM = 2 };
+__device__ __forceinline__ int cta_wait_term(unsigned *sync, int w0, unsigned t0, int w1, unsigned t1, unsigned decision,
+                                             int wb, unsigned tb, int *flag_sh)
+{
+    if (threadIdx.x == 0) {
+        int res = LP_WAIT_ABORT;
+        unsigned flags = 0u, fb;
+        if (poll_until(sync, w0, t0, w1, t1, &flags)) {
+            const unsigned term = flags ? ld_acquire_u32(sync + LP_SYNC_TERM) : 0u;
+            if (term != 0u && term - 1u <= decision) res = LP_WAIT_TERM;
+            else if (wb < 0 || poll_until(sync, wb, tb, -1, 0u, &fb)) res = LP_WAIT_GO;
+        }
+        *flag_sh = res;
     }
     __syncthreads();
-    const bool ok = *flag_sh != 0;
+    const int res = *flag_sh;
     __syncthreads();
-    return ok;
+    return res;
 }
-__device__ __forceinline__ bool cta_wait(unsigned *sync, int which, unsigned target, int *flag_sh)
-{
-    return cta_wait3(sync, which, target, -1, 0u, -1, 0u, flag_sh);
-}
+
+// Phase-timer and counter width of a kernel instantiation.  Per launch the sums stay far below 2^32 clocks, and 32-bit
+// sums leave registers to the owner's hot code: at FT = 6 the kernel's spills fall from 130 to 64 bytes and the slowest
+// owner phase of a C5 round from 18.7 to 16.5 us.  The widest residual stages keep 64 bits; there the narrower sums only
+// move the spills into the sweep.
+template <int FT>
+using LpTick = typename std::conditional<(FT >= 12), unsigned long long, unsigned>::type;
 
 // Phase timers of ONE thread (clock ticks).  The sums stay in that thread's registers and are flushed to global memory
 // once, when the CTA leaves -- a read-modify-write of global memory per mark stalls the timing warp (and everybody
 // behind the next barrier) for an L2 round trip, which at 13 marks per fit distorted what it measured.
-template <int NSLOT>
+template <int NSLOT, typename Tick>
 struct Timer {
     long long t;
     bool on;
-    unsigned long long acc[NSLOT];
+    Tick acc[NSLOT];
     __device__ __forceinline__ void start(bool enable)
     {
         on = enable;
 #pragma unroll
-        for (int q = 0; q < NSLOT; q++) acc[q] = 0ull;
+        for (int q = 0; q < NSLOT; q++) acc[q] = 0;
         if (on) t = clock64();
     }
     __device__ __forceinline__ void mark(int id)
     {
         if (on) {
             const long long now = clock64();
-            const unsigned long long dt = (unsigned long long)(now - t);
+            const Tick dt = (Tick)(now - t);
 #pragma unroll
             for (int q = 0; q < NSLOT; q++)
                 if (q == id) acc[q] += dt;
@@ -278,7 +304,7 @@ __device__ void sweeper_main(const Dev &d, const LpDesc &L, unsigned char *raw)
         asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
     }
     __syncthreads();
-    Timer<3> tm;
+    Timer<3, LpTick<FT>> tm;
     tm.start(tid == 0 && sidx == 0);
     uint32_t parity = 0;
     // step s sweeps group g = s % ng for the r-th time (r = s / ng + 1) once that group's owners have finished their
@@ -287,11 +313,7 @@ __device__ void sweeper_main(const Dev &d, const LpDesc &L, unsigned char *raw)
     for (unsigned st = 0;; st++) {
         const int g = (int)(st % (unsigned)L.ng);
         const unsigned r = st / (unsigned)L.ng + 1u;
-        if (!cta_wait(L.sync, LP_SYNC_B2 + g, (unsigned)L.gcount[g] * r, sm.flag)) break;
-        {
-            const unsigned term = ld_acquire_u32(L.sync + LP_SYNC_TERM);
-            if (term != 0u && term - 1u <= st) break;
-        }
+        if (cta_wait_term(L.sync, LP_SYNC_B2 + g, (unsigned)L.gcount[g] * r, -1, 0u, st, -1, 0u, sm.flag) != LP_WAIT_GO) break;
         tm.mark(0);
         if (L.trace && tid == 0 && sidx == 0 && st < LP_TRACE) L.trace[((size_t)MAXC * LP_TRACE + st) * 2] = lp_globaltimer();
         const double *Rsrc = L.Rg[g];
@@ -441,7 +463,8 @@ struct OwnSm {
     int *misc;     // [16]
     int ldS;
 };
-enum { MI_FLAG = 0, MI_CNT = 1, MI_NNEW = 2, MI_SEEN = 3, MI_TIE = 4, MI_KREM = 5, MI_NEQ = 6, MI_COUNT = 7, MI_Q = 8, MI_RANKN = 9 };
+enum { MI_FLAG = 0, MI_CNT = 1, MI_NNEW = 2, MI_SEEN = 3, MI_TIE = 4, MI_KREM = 5, MI_NEQ = 6, MI_COUNT = 7, MI_Q = 8, MI_RANKN = 9,
+       MI_B2ADD = 10 };
 
 __host__ __device__ inline size_t owner_smem_bytes(int npad, int kcap, int ns, int hist_rows)
 {
@@ -878,7 +901,6 @@ __device__ void gram_new(const Dev &d, OwnSm &s, int nnew, int ns, int npad)
 //
 // All variants are compact rolled loops: a fully unrolled register version (one lane per row) was tried and lost -- 40 KB
 // of straight-line code executed once per fit by one warp is bound by instruction fetch, not by its dependency chain.
-__device__ unsigned long long g_dbg_chol[8];
 constexpr int CHOL_NR = 4;  // new rows (incl. the right-hand side) the append variant carries in registers
 
 // k <= 32 and k - q + 1 == NR <= CHOL_NR.  Lane c owns COLUMN c of the NR new rows (the last one is the right-hand side).
@@ -985,7 +1007,8 @@ __device__ __forceinline__ void chol_backsub_warp(const double *S, int ldS, cons
     if (lane < k) out[lane] = z;
 }
 
-__device__ void chol_solve(OwnSm &s, int k, int q)
+// chol[0..3] (shared memory, owner 0 only): factor ticks, back-substitution ticks, warp solves, their summed k
+__device__ __forceinline__ void chol_solve(OwnSm &s, int k, int q, unsigned long long *chol)
 {
     const int tid = threadIdx.x, lane = tid & 31, wid = tid >> 5;
     const int ldS = s.ldS;
@@ -1001,11 +1024,11 @@ __device__ void chol_solve(OwnSm &s, int k, int q)
             const long long t1 = clock64();
             chol_backsub_warp(S, ldS, s.dg, s.bage, k);
             const long long t2 = clock64();
-            if (lane == 0 && blockIdx.x == 0) {
-                g_dbg_chol[0] += (unsigned long long)(t1 - t0);
-                g_dbg_chol[1] += (unsigned long long)(t2 - t1);
-                g_dbg_chol[2] += 1ull;
-                g_dbg_chol[3] += (unsigned long long)k;
+            if (tid == 0 && blockIdx.x == 0) {
+                chol[0] += (unsigned long long)(t1 - t0);
+                chol[1] += (unsigned long long)(t2 - t1);
+                chol[2] += 1ull;
+                chol[3] += (unsigned long long)k;
             }
         }
         __syncthreads();
@@ -1045,11 +1068,10 @@ __device__ void chol_solve(OwnSm &s, int k, int q)
 
 // Residual of the next sweep, G[i][c] = (y_i - x_i,A beta_A) / n_train on the chain's train rows, 0 elsewhere
 // (Algorithm.h:1109), and on request the Lm losses of Metric.h:145-148 (all rows, / n) and :190 (held-out rows, / 2 n_t).
-__device__ void residual(const Dev &d, OwnSm &s, int c, double *Rcol, int fh, int ks, int nt, int npad, bool want_loss,
+__device__ void residual(const Dev &d, OwnSm &s, double *Rcol, int fh, int ks, int nt, int npad, bool want_loss,
                          double *loss_all, double *loss_test)
 {
-    // Rcol: this chain's column of its group's residual matrix [npad][fh] (what the sweepers stage); d.G gets the same
-    // values so that the multi-kernel helpers (debug_sacrifice, time_dual_sweep) see the chain's current state
+    // Rcol: this chain's column of its group's residual matrix [npad][fh] (what the sweepers stage)
     const int n = d.n;
     double sa = 0.0, st = 0.0;
     for (int i0 = threadIdx.x; i0 < n; i0 += 2 * LP_NT) {
@@ -1067,7 +1089,6 @@ __device__ void residual(const Dev &d, OwnSm &s, int c, double *Rcol, int fh, in
             const bool train = s.m[i0] != 0.0;
             const double gv = train ? e / (double)nt : 0.0;
             __stcg(Rcol + (size_t)i0 * fh, gv);
-            d.G[(size_t)i0 * d.FS + c] = gv;
             sa += e * e;
             if (!train) st += e * e;
         }
@@ -1076,7 +1097,6 @@ __device__ void residual(const Dev &d, OwnSm &s, int c, double *Rcol, int fh, in
             const bool train = s.m[i1] != 0.0;
             const double gv = train ? e / (double)nt : 0.0;
             __stcg(Rcol + (size_t)i1 * fh, gv);
-            d.G[(size_t)i1 * d.FS + c] = gv;
             sa += e * e;
             if (!train) st += e * e;
         }
@@ -1103,6 +1123,7 @@ __device__ void residual(const Dev &d, OwnSm &s, int c, double *Rcol, int fh, in
     __syncthreads();
 }
 
+template <int FT>
 __device__ void owner_main(const Dev &d, const LpDesc &L, unsigned char *raw)
 {
     const int tid = threadIdx.x, lane = tid & 31, wid = tid >> 5;
@@ -1117,9 +1138,11 @@ __device__ void owner_main(const Dev &d, const LpDesc &L, unsigned char *raw)
     double *Rcol = L.Rg[g] + L.oslot[ci];
     const int *rows = d.rows + (size_t)c * n;
     double *bD = d.betaD + (size_t)c * d.pstride;
-    Timer<13> tm;
+    Timer<13, LpTick<FT>> tm;
     tm.start(tid == 0 && ci == 0);
-    unsigned long long own_busy = 0ull, own_max = 0ull, own_fb = 0ull, own_fits = 0ull;  // thread 0: flushed at exit
+    LpTick<FT> own_busy = 0, own_max = 0, own_fb = 0, own_fits = 0;  // thread 0: flushed at exit
+    // solver timers of owner 0 (chol_solve) in the spare tail of s.red: an array in registers would live on the stack
+    unsigned long long *chol = reinterpret_cast<unsigned long long *>(s.red + 36);
 
     // ---- phase O(0): Algorithm::fit prologue from the chain's stored state (Algorithm.h:141-148)
     for (int i = tid; i < npad; i += LP_NT) {
@@ -1130,6 +1153,8 @@ __device__ void owner_main(const Dev &d, const LpDesc &L, unsigned char *raw)
         s.slot_col[q] = -1;
         s.pos[q] = -1;
     }
+    if (tid < 4) chol[tid] = 0ull;
+    if (tid == 0) s.misc[MI_B2ADD] = 1;  // what this owner's arrivals add to B2 (LP_TERM_FLAG too after it sets the word)
     __syncthreads();
     for (int r = tid; r < nt; r += LP_NT) s.m[rows[r]] = 1.0;
     __syncthreads();
@@ -1154,7 +1179,7 @@ __device__ void owner_main(const Dev &d, const LpDesc &L, unsigned char *raw)
     double lam = L.lam[0], lam_fact = L.lam[0];
     for (int a = tid; a < T; a += LP_NT) s.hist[a] = 0;  // A_list.col(0) = 0 (Algorithm.h:143)
     double la = 0.0, lt = 0.0;
-    residual(d, s, c, Rcol, L.fh, ks, nt, npad, false, &la, &lt);
+    residual(d, s, Rcol, L.fh, ks, nt, npad, false, &la, &lt);
     double tau = L.tau[c];
     if (tid == 0) {
         __stcg(L.pub + 2 * c, tau);
@@ -1168,15 +1193,12 @@ __device__ void owner_main(const Dev &d, const LpDesc &L, unsigned char *raw)
     // seen every owner phase up to its decision index complete (its own group's phase it - 1 and the other group's phase
     // just before it), so the word can no longer change below that index: every CTA leaves at the same point.
     for (unsigned it = 1;; it++) {
-        if (!cta_wait3(L.sync, LP_SYNC_B2 + g, (unsigned)L.gcount[g] * it, L.ng == 2 ? LP_SYNC_B2 + og : -1,
-                       (unsigned)L.gcount[og] * (g == 0 ? it - 1u : it), -1, 0u, &s.misc[MI_FLAG]))
+        // (B1 only after the termination word: once the last chain has finished, the sweepers leave and that counter
+        // never moves again)
+        if (cta_wait_term(L.sync, LP_SYNC_B2 + g, (unsigned)L.gcount[g] * it, L.ng == 2 ? LP_SYNC_B2 + og : -1,
+                          (unsigned)L.gcount[og] * (g == 0 ? it - 1u : it), (unsigned)L.ng * (it - 1u) + (unsigned)g,
+                          LP_SYNC_B1 + g, (unsigned)L.nsweep * it, &s.misc[MI_FLAG]) != LP_WAIT_GO)
             break;
-        {
-            const unsigned term = ld_acquire_u32(L.sync + LP_SYNC_TERM);
-            if (term != 0u && term - 1u <= (unsigned)L.ng * (it - 1u) + (unsigned)g) break;
-        }
-        // (only now: once the last chain has finished, the sweepers leave and this counter never moves again)
-        if (!cta_wait(L.sync, LP_SYNC_B1 + g, (unsigned)L.nsweep * it, &s.misc[MI_FLAG])) break;
         tm.mark(1);
         const long long t_phase = clock64();
         if (L.trace && tid == 0 && it < LP_TRACE) L.trace[((size_t)ci * LP_TRACE + it) * 2] = lp_globaltimer();
@@ -1339,8 +1361,8 @@ __device__ void owner_main(const Dev &d, const LpDesc &L, unsigned char *raw)
                     }
                     __syncthreads();
                     tm.mark(8);
-                    own_fb += (unsigned long long)(k - q) * 1965ull;  // DEBUG: new rows per fit (x1965 so the us conversion shows the count)
-                    chol_solve(s, k, q);
+                    own_fb += (LpTick<FT>)(k - q) * 1965u;  // DEBUG: new rows per fit (x1965 so the us conversion shows the count)
+                    chol_solve(s, k, q, chol);
                     // A pivot at or below 1e-13 of its column's own squared norm (or a NaN) is a numerically dependent
                     // active column (e.g. an exact duplicate): this kernel's plain Cholesky has no answer for it.  Flag
                     // the launch; the host repeats the call on the multi-kernel path, whose solver truncates the way the
@@ -1374,9 +1396,9 @@ __device__ void owner_main(const Dev &d, const LpDesc &L, unsigned char *raw)
                     seen = s.misc[MI_SEEN] != 0;
                     tm.mark(11);
                     // the losses ride along with every residual: a fit that ends on a repeated set needs them without a pass
-                    residual(d, s, c, Rcol, L.fh, ks, nt, npad, true, &la, &lt);
+                    residual(d, s, Rcol, L.fh, ks, nt, npad, true, &la, &lt);
                     tm.mark(6);
-                    own_fits += 1ull;
+                    own_fits += 1;
                 }
                 l += 1;
                 tie_acc += s.misc[MI_TIE];
@@ -1405,6 +1427,9 @@ __device__ void owner_main(const Dev &d, const LpDesc &L, unsigned char *raw)
                             d.A[(size_t)c * kcap + a2] = s.A[a2];
                             d.bA[(size_t)c * kcap + a2] = s.beta[a2];
                         }
+                        // the chain's last residual into d.G, where the multi-kernel helpers (debug_sacrifice,
+                        // time_dual_sweep) read a chain's current state after the launch
+                        for (int i = tid; i < n; i += LP_NT) d.G[(size_t)i * d.FS + c] = __ldcg(Rcol + (size_t)i * L.fh);
                         if (tid == 0) {
                             d.ks[c] = ks;
                             d.l[c] = l_out;
@@ -1415,6 +1440,7 @@ __device__ void owner_main(const Dev &d, const LpDesc &L, unsigned char *raw)
                             const unsigned old = atomicAdd(L.sync + LP_SYNC_NCOMPLETE, 1u);
                             if (old + 1u == (unsigned)L.nch) {
                                 atomicExch(L.sync + LP_SYNC_TERM, (unsigned)L.ng * it + (unsigned)g + 1u);
+                                s.misc[MI_B2ADD] = (int)(1u + LP_TERM_FLAG);
                                 atomicExch(L.sync + LP_SYNC_ITERS, (unsigned)L.ng * (it - 1u) + (unsigned)g + 1u);  // sweeps that fed a fit
                             }
                         }
@@ -1429,7 +1455,7 @@ __device__ void owner_main(const Dev &d, const LpDesc &L, unsigned char *raw)
                         if (!d.warm) {
                             for (int a2 = tid; a2 < ks; a2 += LP_NT) __stcg(bD + s.A[a2], 0.0);
                             ks = 0;  // (the factor stays: its leading columns are reused if the next fit selects them again)
-                            residual(d, s, c, Rcol, L.fh, 0, nt, npad, true, &la, &lt);
+                            residual(d, s, Rcol, L.fh, 0, nt, npad, true, &la, &lt);
                         } else if (same && lam == lam_prev) {
                             again = true;  // the sweep this phase consumed was computed from exactly the state the next step starts in
                             if (tid == 0) atomicAdd(L.sync + LP_SYNC_MERGED, 1u);
@@ -1447,18 +1473,18 @@ __device__ void owner_main(const Dev &d, const LpDesc &L, unsigned char *raw)
             tm.mark(7);
         }
         if (tid == 0) {
-            const unsigned long long dt = (unsigned long long)(clock64() - t_phase);
+            const LpTick<FT> dt = (LpTick<FT>)(clock64() - t_phase);
             own_busy += dt;
             if (dt > own_max) own_max = dt;
             if (L.trace && it < LP_TRACE) L.trace[((size_t)ci * LP_TRACE + it) * 2 + 1] = lp_globaltimer();
         }
-        cta_arrive(L.sync + LP_SYNC_B2 + g);
+        cta_arrive(L.sync + LP_SYNC_B2 + g, (unsigned)s.misc[MI_B2ADD]);
     }
     tm.flush(L.dbg);
     if (tid == 0 && ci == 0) {
-        L.dbg[13] = g_dbg_chol[0];
-        L.dbg[14] = g_dbg_chol[1];
-        L.dbg[15] = g_dbg_chol[3] * 1965ull / (g_dbg_chol[2] ? g_dbg_chol[2] : 1ull);
+        L.dbg[13] += chol[0];
+        L.dbg[14] += chol[1];
+        L.dbg[15] = chol[3] * 1965ull / (chol[2] ? chol[2] : 1ull);
     }
     if (tid == 0) {
         unsigned long long *od = L.dbg + 32 + 4 * ci;
@@ -1473,7 +1499,7 @@ template <int FT>
 __global__ void __launch_bounds__(LP_NT, 1) lm_path_kernel(const Dev d, const LpDesc L)
 {
     extern __shared__ __align__(128) unsigned char lp_smem[];
-    if ((int)blockIdx.x < L.nch) owner_main(d, L, lp_smem);
+    if ((int)blockIdx.x < L.nch) owner_main<FT>(d, L, lp_smem);
     else sweeper_main<FT>(d, L, lp_smem);
 }
 
